@@ -47,7 +47,16 @@ def parse():
     ap.add_argument("--engine", default="auto", choices=["auto", "simt", "tc"])
     ap.add_argument("--cpu-sample", type=int, default=400, help="proteins (pairs) in the cpu_baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step computed as DIR/<name>.npy (rank 0): the GO-term "
+                         "scores of the resident leg; config2: every head's scores from the end-to-end leg; config1: the "
+                         "bit-packed contact maps of the end-to-end leg.  Outputs above 64 MB in all are a fixed, seeded sample")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return args
 
 
 ARGS = parse()
@@ -103,6 +112,33 @@ def ncu_traffic(stage):
     if os.path.exists(p):
         return json.load(open(p)).get(stage)
     return None
+
+
+DUMP_BYTES = 60 << 20          # --dump-outputs: data bytes of all files together (< 64 MB with the .npy headers)
+
+
+def dump_outputs(out_dir, scores=None, maps=None):
+    """--dump-outputs.  `scores`: {name: float32 [n, C]} with a common n, written whole or as the same seeded sample of rows
+    (rows.npy) when larger than DUMP_BYTES.  `maps`: bit-packed uint32 [Lq, words] per pair, a seeded sample of pairs
+    written as float64 (exact for uint32): cmap_words.npy = their words, concatenated; cmap_pairs.npy = (pair, Lq) rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(0)
+    if maps is not None:
+        order = rng.permutation(len(maps))
+        size = np.cumsum([maps[i].size * 8 + 16 for i in order])
+        keep = np.sort(order[size <= DUMP_BYTES])
+        out = {"cmap_words": np.concatenate([maps[i].ravel() for i in keep]).astype(np.float64),
+               "cmap_pairs": np.array([(i, maps[i].shape[0]) for i in keep], np.float64).reshape(-1, 2)}
+    else:
+        n = len(next(iter(scores.values())))
+        row_bytes = sum(s.shape[1] * 4 for s in scores.values())
+        k = min(n, DUMP_BYTES // (row_bytes + 8))
+        rows = np.arange(n) if k == n else np.sort(rng.choice(n, k, replace=False))
+        out = {name: np.ascontiguousarray(s[rows], np.float32) for name, s in scores.items()}
+        if k < n:
+            out["rows"] = rows.astype(np.float64)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def sub(wl, idx):
@@ -645,6 +681,11 @@ def run_b200(args, rank, world, local_rank, inputs):
     }
     if job:
         line["sharded_job"] = job
+    if args.dump_outputs:
+        if maps_only:
+            dump_outputs(args.dump_outputs, maps=maps)
+        else:
+            dump_outputs(args.dump_outputs, {f"scores_{h}": out_heads[h] for h in preds} if multi_head else {"scores": scores_resident})
     print(json.dumps(line), flush=True)
 
 

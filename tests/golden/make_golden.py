@@ -3,11 +3,17 @@ contact-map half):   python tests/golden/make_golden.py
 
   cmap_golden.npz  - outputs of the UNMODIFIED reference (oracle/_ref: mDeepFRI/contact_map_utils.pyx
                      compiled by oracle/Makefile) + the NumPy glue of bio_utils.py:214-223.
+  cmap_random_golden.npz - pairwise_sqeuclidean (several threads) and align_contact_map on spec.cmap_random_cases():
+                     structures up to 300 residues, generated contacts 0-3, arbitrary sparse input.  Written from
+                     the reference like cmap_golden.npz; where the reference is not built,
+                     `python tests/golden/make_golden.py --cmap-random-from-port` writes this file alone from the C port
+                     (oracle/cmap_oracle.c).  Its `source` entry names which one wrote it.
   gcn_golden.npz   - outputs of oracle/gcn_oracle.py (fp32 NumPy ONNX interpreter) on seeded
                      random-init models.  PARITY UNPINNED: the reference has no golden vectors for
                      Predictor and onnxruntime is not available; these pin the CUDA path and the
                      oracle against regressions only.
 """
+import hashlib
 import os
 import sys
 import tempfile
@@ -48,7 +54,38 @@ def edge_cases():
     ]
 
 
+def digest(a):
+    return np.frombuffer(hashlib.blake2b(np.ascontiguousarray(a).tobytes(), digest_size=16).digest(), np.uint8)
+
+
+def write_cmap_random(pw, al, source):
+    """What `pw(coords)` and `al(gapped_q, gapped_t, sparse, gen)` return on spec.cmap_random_cases(): D as a digest of all
+    its bytes plus a seeded sample of 64 entries, the aligned maps bit-packed (np.packbits, row-major)."""
+    out = {"source": np.array(source)}
+    cases = spec.cmap_random_cases()
+    for k, (gq, gt, coords, thr, sp, gen) in enumerate(cases):
+        D = pw(coords)
+        if sp is None:
+            sp = np.argwhere(D < co.threshold_sq(thr)).astype(np.int32)          # bio_utils.py:220-223
+        aligned = al(gq, gt, sp, gen)
+        assert np.isin(aligned, (0, 1)).all()
+        idx = np.random.default_rng(k).integers(0, D.size, 64)
+        out[f"r{k}_coords"] = digest(coords)
+        out[f"r{k}_D"] = digest(D)
+        out[f"r{k}_D_idx"], out[f"r{k}_D_val"] = idx, D.ravel()[idx]
+        out[f"r{k}_Lq"] = np.array(aligned.shape[0])
+        out[f"r{k}_aligned"] = np.packbits(aligned.astype(bool))
+    out["n_cases"] = np.array(len(cases))
+    np.savez_compressed(os.path.join(HERE, "cmap_random_golden.npz"), **out)
+    print("cmap_random_golden.npz:", len(cases), "cases from", source)
+
+
 def main():
+    if "--cmap-random-from-port" in sys.argv[1:]:
+        write_cmap_random(lambda c: co.pairwise_sqeuclidean(c, threads=3),
+                          lambda q, t, sp, gen: co.align_contact_map(q, t, sp, gen, threads=2),
+                          "C port: oracle/cmap_oracle.c")
+        return
     ref = co.ref_module()
     if ref is None:
         raise SystemExit("oracle/_ref is not built (make -C oracle ref)")
@@ -80,6 +117,8 @@ def main():
     out["n_cases"] = np.array(k)
     np.savez_compressed(os.path.join(HERE, "cmap_golden.npz"), **out)
     print("cmap_golden.npz:", k, "cases")
+    write_cmap_random(lambda c: ref.pairwise_sqeuclidean(c, 2), lambda q, t, sp, gen: ref.align_contact_map(q, t, sp, gen, 2),
+                      "reference: mDeepFRI/contact_map_utils.pyx compiled unchanged (oracle/_ref)")
 
     # ---- GCN golden (oracle-generated)
     g = {}

@@ -16,6 +16,22 @@ def workload_seed(model_seed: int) -> int:
     return model_seed + 100
 
 
+def cmap_random_cases():
+    """Inputs of the random contact-map cases (cmap_random_golden.npz): 60 seeded structures of 1-300 residues, 6 / 10 A,
+    generated contacts 0-3.  -> [(gapped_q, gapped_t, coords, threshold, sparse, gen)]; sparse is None where the case uses
+    the structure's own map (np.argwhere), else arbitrary pairs: non-symmetric, out of range and negative."""
+    import numpy as np
+    from metagenomic_deepfri_b200 import synth
+    rng = np.random.default_rng(7)
+    wl = synth.make_workload(60, 1, 300, seed=9, threshold=6.0)
+    out = []
+    for i in range(len(wl)):
+        c = wl.coords[i]
+        sp = rng.integers(-3, len(c) + 5, size=(50, 2)).astype(np.int32) if i % 5 == 0 else None
+        out.append((wl.gapped_query[i], wl.gapped_target[i], c, (6.0, 10.0)[i % 2], sp, i % 4))
+    return out
+
+
 # ---- sequence-only DeepCNN cases: tag -> (CNNConfig kwargs, model seed, n sequences, Lmin, Lmax)
 CNN_CASES = {
     # odd / even widths, unequal filter counts, 1..300 residues (tiles of 128: one, two and three per protein)

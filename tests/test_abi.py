@@ -40,7 +40,20 @@ def test_version_and_row_words():
     assert [_lib.packed_row_words(L) for L in (0, 1, 128, 129, 300)] == [0, 4, 4, 8, 12]
 
 
-@pytest.mark.skipif(os.path.exists("/dev/nvidia0"), reason="GPU present")
+def cuda_device_count():
+    """Devices the CUDA driver reports (0 without a driver), as the library's context creation counts them: a GPU's device
+    node need not be /dev/nvidia0."""
+    try:
+        cu = ctypes.CDLL("libcuda.so.1")
+    except OSError:
+        return 0
+    n = ctypes.c_int(0)
+    if cu.cuInit(0) != 0 or cu.cuDeviceGetCount(ctypes.byref(n)) != 0:
+        return 0
+    return n.value
+
+
+@pytest.mark.skipif(cuda_device_count() > 0, reason="GPU present")
 def test_no_cpu_fallback_without_gpu(model_dir):
     from metagenomic_deepfri_b200 import contact_map_utils, predict
     with pytest.raises(RuntimeError, match="no CUDA device|CUDA"):

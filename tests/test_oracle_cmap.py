@@ -1,15 +1,17 @@
 """CPU tests: the contact-map oracle against the reference's own known-answer tests, the compiled
 reference (oracle/_ref, when built) and the committed golden vectors."""
+import os
+
 import numpy as np
 import pytest
 
 import cmap_oracle as co
 
 REF = co.ref_module()
-needs_ref = pytest.mark.skipif(REF is None, reason="oracle/_ref not built (needs /root/reference)")
 
 
 def impls():
+    """The port always; the reference's own compiled module only where it has been built into oracle/_ref."""
     out = [("port", co.pairwise_sqeuclidean, co.align_contact_map)]
     if REF is not None:
         out.append(("reference", REF.pairwise_sqeuclidean, REF.align_contact_map))
@@ -71,20 +73,34 @@ def test_port_matches_golden(cmap_golden):
         assert np.array_equal(co.pairwise_sqeuclidean_np(coords), g[f"c{k}_D"])
 
 
-@needs_ref
 def test_port_matches_reference_random():
-    from metagenomic_deepfri_b200 import synth
-    rng = np.random.default_rng(7)
-    wl = synth.make_workload(60, 1, 300, seed=9, threshold=6.0)
-    for i in range(len(wl)):
-        c = wl.coords[i]
-        assert np.array_equal(co.pairwise_sqeuclidean(c, threads=3), REF.pairwise_sqeuclidean(c, 2))
-        sp = co.calculate_contact_map(c, (6.0, 10.0)[i % 2], "sparse")
-        if i % 5 == 0:   # arbitrary (non-symmetric, out-of-range, negative) sparse input
-            sp = rng.integers(-3, len(c) + 5, size=(50, 2)).astype(np.int32)
-        gen = i % 4
-        assert np.array_equal(co.align_contact_map(wl.gapped_query[i], wl.gapped_target[i], sp, gen, threads=2),
-                              REF.align_contact_map(wl.gapped_query[i], wl.gapped_target[i], sp, gen, 2))
+    """The port on spec.cmap_random_cases() (up to 300 residues, generated contacts 0-3, arbitrary sparse input, several
+    threads) against the stored tests/golden/cmap_random_golden.npz, bit for bit; with the reference built, the
+    reference against the same file."""
+    import hashlib
+    import spec
+    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "cmap_random_golden.npz"))
+    digest = lambda a: np.frombuffer(hashlib.blake2b(np.ascontiguousarray(a).tobytes(), digest_size=16).digest(), np.uint8)
+    impls = [("port", lambda c: co.pairwise_sqeuclidean(c, threads=3),
+              lambda c, thr: co.calculate_contact_map(c, thr, "sparse"),
+              lambda q, t, sp, gen: co.align_contact_map(q, t, sp, gen, threads=2))]
+    if REF is not None:
+        impls.append(("reference", lambda c: REF.pairwise_sqeuclidean(c, 2),
+                      lambda c, thr: np.argwhere(REF.pairwise_sqeuclidean(c) < co.threshold_sq(thr)).astype(np.int32),
+                      lambda q, t, sp, gen: REF.align_contact_map(q, t, sp, gen, 2)))
+    cases = spec.cmap_random_cases()
+    assert len(cases) == int(g["n_cases"])
+    for k, (gq, gt, c, thr, sp_in, gen) in enumerate(cases):
+        assert np.array_equal(digest(c), g[f"r{k}_coords"]), f"case {k}: the generated inputs changed"
+        Lq = int(g[f"r{k}_Lq"])
+        want = np.unpackbits(g[f"r{k}_aligned"], count=Lq * Lq).reshape(Lq, Lq)
+        for name, pw, sparse, al in impls:
+            D = pw(c)
+            assert np.array_equal(D.ravel()[g[f"r{k}_D_idx"]], g[f"r{k}_D_val"]), f"{name}, case {k}: D differs"
+            assert np.array_equal(digest(D), g[f"r{k}_D"]), f"{name}, case {k}: D differs"
+            sp = sparse(c, thr) if sp_in is None else sp_in
+            got = al(gq, gt, sp, gen)
+            assert got.shape == (Lq, Lq) and np.array_equal(got, want), f"{name}, case {k}: aligned map differs"
 
 
 def test_insert_gaps_dialect():
