@@ -7,7 +7,7 @@
 //   X_l = act(d_i * sum_j A_hat[i,j] * d_j * (X_{l-1} W_l)[j] + b_l)      (l = 1..n_gc)
 //   pooled = sum_i concat_l X_l[i] ; fc = relu(pooled W + b) ; logits = fc W + b ;
 //   score[c] = softmax(logits[c, :])[0]
-// It is the on-device numerical reference for the tensor-core engine (gemm_tc.cu / lstm_tc.cu)
+// It is the on-device numerical reference for the tensor-core engine (gemm_tc.cu / lstm_fused.cu)
 // and shares every buffer layout with the C-ABI taps (mdf_batch_fetch).
 #include "gcn.cuh"
 

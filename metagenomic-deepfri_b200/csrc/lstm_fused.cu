@@ -33,7 +33,7 @@
 #include <vector>
 
 #include "gemm_tc.cuh"
-#include "lstm_tc.cuh"
+#include "lstm_fused.cuh"
 
 extern "C" char **environ;
 

@@ -16,14 +16,13 @@
 #include <stdlib.h>
 
 #include "gemm_tc.cuh"
-#include "lstm_tc.cuh"
+#include "lstm_fused.cuh"
 #include "tc_engine.cuh"
 
 namespace mdf {
 
 int head_forward(mdf_model *m, int n, const float *pooled, float *fc, float *logits, float *scores);
 int launch_softmax0(mdf_ctx *ctx, int64_t total, const float *logits, float *scores);
-int simt_lstm_stack(mdf_model *m, mdf_batch *b, float **Hl, float *pre, float *Cst, unsigned *barrier);
 
 using namespace tc;
 
@@ -45,22 +44,12 @@ struct TcModel {
     int adj_sparse = 1;                                    // adjacency GEMM skips all-zero 128 x 64 A tiles (MDF_ADJ_SPARSE=0: dense walk)
     int adj_expand = 1;                                    // adjacency GEMM expands its A tiles from the bit-packed map on the fly
     int gemm_pair = 1;                                     // CTA-pair (cta_group::2) kernels for the embedding and X.W GEMMs
-    __half *lstm_R[MDF_MAX_LSTM] = {nullptr};              // [H/16][2][64 x H] resident recurrent slices (hi, lo)
-    __half *lstm_Ralt[MDF_MAX_LSTM] = {nullptr};           // same, time-dithered pair (R_a, R_b = fp16(2R - R_a))
-    int lstm_alternate = 1;
-    __half *lstm_Rstream[MDF_MAX_LSTM][2] = {{nullptr}};   // streamed kernel: [4H rows (cta,gate,unit) x H], (R_a, R_b)
-    float *lstm_tab_full = nullptr;                        // [26][H][4] layer-1 table over all units
-    float *lstm_fused_tab = nullptr, *lstm_fused_b2 = nullptr;   // fused kernel: the same table / layer-2 bias with the i, o, f entries halved (see lstm_fused_W)
-    int lstm_stream_min = 2048;                            // proteins per batch from which the streamed kernel is used
+    float *lstm_fused_tab = nullptr, *lstm_fused_b2 = nullptr;   // fused kernel: layer-1 table / layer-2 bias with the i, o, f entries halved (see lstm_fused_W)
     __half *lstm_fused_W = nullptr;                        // fused kernel: [R1, W2, R2][phase][4H rows (slice, gate, unit) x H] images
     int lstm_phases = 5;                                   // time-dither period of the fused kernel's weights (sigma-delta rounding).  Measured:
                                                            // 8 phases (48 MB) do not stay in L2 between their uses - one 6 MB phase came from DRAM
                                                            // every tick (13.5 GB per launch, also with an evict_last hint); 5 phases (30 MB) do:
                                                            // 3.1 GB, kernel -3.7 %, score error unchanged (3.4e-4 -> 3.8e-4; 4 phases 5.2e-4)
-    int lstm_fused = 1;                                    // use the fused two-layer wavefront kernel when supported
-    float *lstm_tab = nullptr;                             // [H/16][26][16][4] layer-1 input table (bias folded)
-    __half *lstm_Win[MDF_MAX_LSTM][2] = {{nullptr}};       // layers >= 2: [4H rows in (unit,gate) order x H k]
-    float *lstm_bperm[MDF_MAX_LSTM] = {nullptr};           // layers >= 2: bias in (unit,gate) order
     bool ok = false;
 };
 
@@ -80,9 +69,9 @@ struct TcBatchMeta {
 
 // ------------------------------------------------------------------------------------------- weight images
 static void build_image_host(const float *src, int rows, int K, bool transposed_src, int ld,
-                             std::vector<__half> &hi, std::vector<__half> &lo, bool dither = false, float lo_scale = 1.0f)
+                             std::vector<__half> &hi, std::vector<__half> &lo, float lo_scale = 1.0f)
 {
-    // dither = false: (hi, lo) with hi + lo ~ v;  dither = true: (a, b) with a + b ~ 2v (time-dithered pair)
+    // (hi, lo) with hi + lo / lo_scale ~ v
     // element (r, k) = transposed_src ? src[k * ld + r] : src[r * ld + k]
     const int RT = cdiv(rows, TILE_ROWS), KB = cdiv(K, TILE_K);
     const size_t total = (size_t)RT * KB * (TILE_BYTES / 2);
@@ -92,7 +81,7 @@ static void build_image_host(const float *src, int rows, int K, bool transposed_
         for (int k = 0; k < K; ++k) {
             const float v = transposed_src ? src[(size_t)k * ld + r] : src[(size_t)r * ld + k];
             const __half h = __float2half_rn(v);
-            const __half l = dither ? __float2half_rn(2.0f * v - __half2float(h)) : __float2half_rn((v - __half2float(h)) * lo_scale);
+            const __half l = __float2half_rn((v - __half2float(h)) * lo_scale);
             const size_t off = image_offset_bytes(r, k, KB) / 2;
             hi[off] = h;
             lo[off] = l;
@@ -133,9 +122,6 @@ int tc_model_init(mdf_model *m, const mdf_model_desc *d)
 {
     TcModel *t = new TcModel();
     m->tc = t;
-    if (const char *e = getenv("MDF_LSTM_HILO")) t->lstm_alternate = atoi(e) ? 0 : 1;   // 1 = hi+lo on every step
-    if (const char *e = getenv("MDF_LSTM_STREAM_MIN")) t->lstm_stream_min = atoi(e);
-    if (const char *e = getenv("MDF_LSTM_FUSED")) t->lstm_fused = atoi(e);
     if (const char *e = getenv("MDF_LSTM_PHASES")) t->lstm_phases = std::min(64, std::max(1, atoi(e)));
     if (const char *e = getenv("MDF_GEMM_PAIR")) t->gemm_pair = atoi(e);
     if (const char *e = getenv("MDF_ADJ_EXPAND")) t->adj_expand = atoi(e);
@@ -147,8 +133,8 @@ int tc_model_init(mdf_model *m, const mdf_model_desc *d)
     if (const char *e = getenv("MDF_SINGLE_TERM")) t->single_term_mask = atoi(e);
     if (const char *e = getenv("MDF_HEAD_TC")) t->head_tc = atoi(e);
     if (const char *e = getenv("MDF_XW_MEAN")) t->xw_mean = atoi(e);
-    // shape constraints of the tile-image GEMMs
-    bool ok = m->H % 64 == 0 && m->E % 128 == 0;
+    // shape constraints of the tile-image GEMMs and of the fused LSTM kernel (two layers, H = 64 ... 512)
+    bool ok = m->H % 64 == 0 && m->E % 128 == 0 && lstm_fused_supported(m->H, m->n_lstm);
     for (int l = 0; l < m->n_gc; ++l) ok = ok && m->gc[l] % 128 == 0;
     if (!ok) return MDF_OK;           // engine stays unavailable; the SIMT engine serves this model
     std::vector<__half> hi, lo;
@@ -158,10 +144,10 @@ int tc_model_init(mdf_model *m, const mdf_model_desc *d)
     if (m->G % TILE_K == 0 && m->F % TILE_K == 0) {
         // head weights: hi and the residual scaled by 2^11 (HEAD_LO_SHIFT): unscaled, the residual of a 0.03-sized weight
         // is an fp16 denormal with ~8 significant bits, and after the sum-pool that is visible in the scores
-        build_image_host(d->fc_W, m->F, m->G, true, m->F, hi, lo, false, 2048.0f);            // rows = F, k = G : fc_W[k][f]
+        build_image_host(d->fc_W, m->F, m->G, true, m->F, hi, lo, 2048.0f);            // rows = F, k = G : fc_W[k][f]
         MDF_TRY(upload_half(m, &t->fc_W[0], hi));
         MDF_TRY(upload_half(m, &t->fc_W[1], lo));
-        build_image_host(d->out_W, 2 * m->C, m->F, true, 2 * m->C, hi, lo, false, 2048.0f);   // rows = 2C, k = F : out_W[k][c]
+        build_image_host(d->out_W, 2 * m->C, m->F, true, 2 * m->C, hi, lo, 2048.0f);   // rows = 2C, k = F : out_W[k][c]
         MDF_TRY(upload_half(m, &t->out_W[0], hi));
         MDF_TRY(upload_half(m, &t->out_W[1], lo));
         std::vector<float> bp((size_t)(2 * m->C + 3) / 4 * 4, 0.0f);
@@ -179,7 +165,7 @@ int tc_model_init(mdf_model *m, const mdf_model_desc *d)
             // rounding residual of the hi term, for the mean correction of the single-term X.W (tc_forward)
             std::vector<float> dw((size_t)prev * m->gc[l]);
             for (size_t i = 0; i < dw.size(); ++i) dw[i] = (d->gc_W[l][i] - __half2float(__float2half_rn(d->gc_W[l][i]))) * 2048.0f;
-            build_image_host(dw.data(), m->gc[l], prev, true, m->gc[l], hi, lo, false, 2048.0f);
+            build_image_host(dw.data(), m->gc[l], prev, true, m->gc[l], hi, lo, 2048.0f);
             MDF_TRY(upload_half(m, &t->gc_dW[l][0], hi));
             MDF_TRY(upload_half(m, &t->gc_dW[l][1], lo));
         }
@@ -197,82 +183,7 @@ int tc_model_init(mdf_model *m, const mdf_model_desc *d)
         }
         t->lm_hash = hsh ? hsh : 1;
     }
-    // ---- LSTM: resident recurrent slices, layer-1 table, input-GEMM weights of the upper layers
-    const int H = m->H, H4 = 4 * H, cpg = H / 16;
-    for (int l = 0; l < m->n_lstm; ++l) {
-        const float *R = d->lstm_R[l];                                  // ONNX [4H][H], gate order i,o,f,c
-        std::vector<__half> img((size_t)cpg * 2 * 64 * H, __float2half(0.0f)), alt((size_t)cpg * 2 * 64 * H, __float2half(0.0f));
-        for (int s = 0; s < cpg; ++s)
-            for (int r = 0; r < 64; ++r) {
-                const int gate = r >> 4, u = r & 15;
-                const float *src = R + (size_t)(gate * H + s * 16 + u) * H;
-                for (int k = 0; k < H; ++k) {
-                    const __half h = __float2half_rn(src[k]);
-                    const __half lo2 = __float2half_rn(src[k] - __half2float(h));
-                    const size_t off = (size_t)(((k >> 3) * 8 + (r >> 3)) * 128 + (r & 7) * 16 + (k & 7) * 2) / 2;
-                    img[((size_t)s * 2 + 0) * 64 * H + off] = h;
-                    img[((size_t)s * 2 + 1) * 64 * H + off] = lo2;
-                    alt[((size_t)s * 2 + 0) * 64 * H + off] = h;
-                    alt[((size_t)s * 2 + 1) * 64 * H + off] = __float2half_rn(2.0f * src[k] - __half2float(h));
-                }
-            }
-        MDF_TRY(upload_half(m, &t->lstm_R[l], img));
-        MDF_TRY(upload_half(m, &t->lstm_Ralt[l], alt));
-        if (lstm_stream_supported(H)) {
-            // streamed kernel: CTA s owns units [128s, 128s+128); its rows are ordered (gate, unit) so that the
-            // four gates of a unit share a TMEM lane: image row s*512 + gate*128 + u <- ONNX row gate*H + s*128 + u
-            std::vector<float> Rp((size_t)H4 * H);
-            for (int s = 0; s < H / 128; ++s)
-                for (int gate = 0; gate < 4; ++gate)
-                    for (int u = 0; u < 128; ++u)
-                        std::copy(R + (size_t)(gate * H + s * 128 + u) * H, R + (size_t)(gate * H + s * 128 + u + 1) * H,
-                                  Rp.begin() + (size_t)(s * 512 + gate * 128 + u) * H);
-            std::vector<__half> ra, rb;
-            build_image_host(Rp.data(), H4, H, false, H, ra, rb, true);
-            MDF_TRY(upload_half(m, &t->lstm_Rstream[l][0], ra));
-            MDF_TRY(upload_half(m, &t->lstm_Rstream[l][1], rb));
-        }
-        std::vector<float> bsum(H4, 0.0f);
-        if (d->lstm_B[l])
-            for (int r = 0; r < H4; ++r) bsum[r] = d->lstm_B[l][r] + d->lstm_B[l][H4 + r];
-        if (l == 0) {
-            std::vector<float> tab((size_t)cpg * 26 * 64);
-            for (int s = 0; s < cpg; ++s)
-                for (int aa = 0; aa < 26; ++aa)
-                    for (int u = 0; u < 16; ++u)
-                        for (int gate = 0; gate < 4; ++gate) {
-                            const int row = gate * H + s * 16 + u;
-                            tab[(((size_t)s * 26 + aa) * 16 + u) * 4 + gate] = d->lstm_W[0][(size_t)row * m->I + aa] + bsum[row];
-                        }
-            MDF_CUDA(cudaMalloc((void **)&t->lstm_tab, tab.size() * sizeof(float)));
-            m->owned.push_back(t->lstm_tab);
-            MDF_CUDA(cudaMemcpy(t->lstm_tab, tab.data(), tab.size() * sizeof(float), cudaMemcpyHostToDevice));
-            std::vector<float> full((size_t)26 * H * 4);                 // [aa][unit][gate]
-            for (int aa = 0; aa < 26; ++aa)
-                for (int unit = 0; unit < H; ++unit)
-                    for (int gate = 0; gate < 4; ++gate)
-                        full[((size_t)aa * H + unit) * 4 + gate] = d->lstm_W[0][(size_t)(gate * H + unit) * m->I + aa] + bsum[gate * H + unit];
-            MDF_CUDA(cudaMalloc((void **)&t->lstm_tab_full, full.size() * sizeof(float)));
-            m->owned.push_back(t->lstm_tab_full);
-            MDF_CUDA(cudaMemcpy(t->lstm_tab_full, full.data(), full.size() * sizeof(float), cudaMemcpyHostToDevice));
-        } else {
-            // B operand rows n' = unit*4 + gate  <-  ONNX row gate*H + unit ; k = input feature
-            std::vector<float> Wp((size_t)H4 * H), bp(H4);
-            for (int unit = 0; unit < H; ++unit)
-                for (int gate = 0; gate < 4; ++gate) {
-                    const int np = unit * 4 + gate, row = gate * H + unit;
-                    std::copy(d->lstm_W[l] + (size_t)row * H, d->lstm_W[l] + (size_t)(row + 1) * H, Wp.begin() + (size_t)np * H);
-                    bp[np] = bsum[row];
-                }
-            build_image_host(Wp.data(), H4, H, false, H, hi, lo);
-            MDF_TRY(upload_half(m, &t->lstm_Win[l][0], hi));
-            MDF_TRY(upload_half(m, &t->lstm_Win[l][1], lo));
-            MDF_CUDA(cudaMalloc((void **)&t->lstm_bperm[l], bp.size() * sizeof(float)));
-            m->owned.push_back(t->lstm_bperm[l]);
-            MDF_CUDA(cudaMemcpy(t->lstm_bperm[l], bp.data(), bp.size() * sizeof(float), cudaMemcpyHostToDevice));
-        }
-    }
-    if (lstm_fused_supported(H, m->n_lstm)) {
+    {
         // fused kernel: slice s owns units [64s, 64s+64) of both layers; rows ordered (slice, gate, unit) so that
         // TMEM column = gate*64 + unit: image row s*256 + gate*64 + u <- ONNX row gate*H + s*64 + u.
         // Per matrix, contiguous: P time-dither roundings, then the exact split (hi, lo) that long proteins use:
@@ -280,6 +191,7 @@ int tc_model_init(mdf_model *m, const mdf_model_desc *d)
         // The rows of the sigmoid gates (ONNX order i, o, f = gates 0..2) are stored HALVED, and so are their table / bias entries:
         // sigmoid(x) = 1/2 + 1/2 tanh(x/2), so the kernel's tanh-form cell receives x/2 straight from the accumulator (an exact
         // power-of-two scaling; three multiplies less per cell - at the power cap the cell update's instructions are paid in clock).
+        const int H = m->H, H4 = 4 * H;
         const float *src[3] = {d->lstm_R[0], d->lstm_W[1], d->lstm_R[1]};
         const int P = t->lstm_phases;
         const size_t img_elems = (size_t)H4 * H;
@@ -319,7 +231,6 @@ int tc_model_init(mdf_model *m, const mdf_model_desc *d)
         m->owned.push_back(t->lstm_fused_b2);
         MDF_CUDA(cudaMemcpy(t->lstm_fused_b2, fb2.data(), fb2.size() * sizeof(float), cudaMemcpyHostToDevice));
     }
-    if (lstm_tc_smem_bytes(H) > 227 * 1024) return MDF_OK;   // cannot keep the slices resident: engine unavailable
     t->ok = true;
     return MDF_OK;
 }
@@ -633,7 +544,7 @@ int tc_softmax0_strided(mdf_ctx *ctx, int n, int C, int ld, const float *logits,
 // host: W[k][row] (ONNX MatMul layout [K, rows]) -> hi image and residual image scaled by 2^11, rows x K
 void tc_build_split_weight_images(const float *src_kn, int rows, int K, std::vector<__half> &hi, std::vector<__half> &lo)
 {
-    build_image_host(src_kn, rows, K, true, rows, hi, lo, false, 2048.0f);
+    build_image_host(src_kn, rows, K, true, rows, hi, lo, 2048.0f);
 }
 
 // ------------------------------------------------------------------------------------------- batch metadata
@@ -737,13 +648,10 @@ size_t tc_workspace_bytes(const mdf_model *m, int n, const int64_t *seq_off)
     for (int l = 0; l < m->n_gc; ++l) gmax = std::max(gmax, m->gc[l]);
     size_t b = 0;
     auto add = [&](size_t x) { b += align_up(x, 256) + 256; };
-    const TcModel *tm = static_cast<const TcModel *>(m->tc);
-    const bool fused = tm && tm->lstm_fused && tm->lstm_fused_W;
     const bool taps = m->ctx->debug_taps;
     for (int l = 0; l < m->n_lstm; ++l)
-        if (!fused || l == m->n_lstm - 1 || taps) add((size_t)Tp * m->H * 2);   // H_l images
-    if (!fused) add((size_t)Tp * 4 * m->H * 4);       // input pre-activations of the upper LSTM layers
-    add(std::max({lstm_tc_scratch_bytes(m->ctx, m->H), lstm_stream_scratch_bytes(m->ctx, m->H), lstm_fused_scratch_bytes(m->ctx, m->H)}));
+        if (l == m->n_lstm - 1 || taps) add((size_t)Tp * m->H * 2);   // H_l images
+    add(lstm_fused_scratch_bytes(m->ctx, m->H));
     if (taps) for (int l = 0; l < m->n_lstm; ++l) add((size_t)T * m->H * 4);    // optional fp32 taps
     add((size_t)Tp * 4 + (size_t)Tp / 128 * 32 + (size_t)(tiles + 1) * 16 + (size_t)(n + 1) * 8 + 2048);   // metadata
     add((size_t)Tp * 4); add((size_t)Tp);             // deg_pad, idx_pad
@@ -796,17 +704,12 @@ int tc_forward(mdf_model *m, mdf_batch *b, int upto, const std::function<int()> 
 
     float *deg_pad; uint8_t *idx_pad; __half *X0img, *Yt, *Xa, *Xb, *Aimg;
     __half *Hlimg[MDF_MAX_LSTM] = {nullptr};
-    float *pre = nullptr;
     void *scratch = nullptr;
     MDF_TRY(ctx->alloc_n(&deg_pad, (size_t)Tp));
     MDF_TRY(ctx->alloc_n(&idx_pad, (size_t)Tp));
-    const bool fused_lstm = tm->lstm_fused && tm->lstm_fused_W != nullptr;
     for (int l = 0; l < m->n_lstm; ++l)      // the fused LSTM keeps layer 1 on chip: its image only exists for the debug taps
-        if (!fused_lstm || l == m->n_lstm - 1 || ctx->debug_taps) MDF_TRY(ctx->alloc_n(&Hlimg[l], (size_t)Tp * m->H));
-    if (m->n_lstm > 1 && !(tm->lstm_fused && tm->lstm_fused_W)) MDF_TRY(ctx->alloc_n(&pre, (size_t)Tp * 4 * m->H));
-    const bool fused = tm->lstm_fused && tm->lstm_fused_W != nullptr;
-    MDF_TRY(ctx->alloc(&scratch, std::max({lstm_tc_scratch_bytes(ctx, m->H), lstm_stream_scratch_bytes(ctx, m->H),
-                                           lstm_fused_scratch_bytes(ctx, m->H)})));
+        if (l == m->n_lstm - 1 || ctx->debug_taps) MDF_TRY(ctx->alloc_n(&Hlimg[l], (size_t)Tp * m->H));
+    MDF_TRY(ctx->alloc(&scratch, lstm_fused_scratch_bytes(ctx, m->H)));
     MDF_TRY(ctx->alloc_n(&X0img, (size_t)Tp * m->E));
     MDF_TRY(ctx->alloc_n(&Yt, (size_t)Tp * gmax));
     MDF_TRY(ctx->alloc_n(&Xa, (size_t)Tp * gmax));
@@ -831,40 +734,13 @@ int tc_forward(mdf_model *m, mdf_batch *b, int upto, const std::function<int()> 
         }
         Hlimg[m->n_lstm - 1] = static_cast<__half *>(b->lm_cache);
     }
-    if (lm_cached) {
-        b->tap_h[0] = b->tap_h[1] = nullptr;
-    } else if (fused) {
+    b->tap_h[0] = b->tap_h[1] = nullptr;
+    if (!lm_cached) {
         // both layers + the layer-2 input projection in one persistent wavefront kernel (lstm_fused.cu)
         ProfScope ps(ctx, "lstm_fused", 3.0 * 2.0 * T * 4 * m->H * m->H);
         MDF_TRY(launch_lstm_fused(ctx, m->H, n, tm->lstm_fused_W, tm->lstm_phases, tm->lstm_fused_tab, tm->lstm_fused_b2, idx_pad, b->d_order,
                                   b->d_seq_off, row_off, ctx->debug_taps ? Hlimg[0] : nullptr, Hlimg[1], scratch, b->h_order.data(),
                                   b->h_seq_off.data()));
-        b->tap_h[0] = b->tap_h[1] = nullptr;
-    }
-    // fallback: persistent tcgen05 recurrence per layer, input GEMM between layers
-    for (int l = 0; l < ((fused || lm_cached) ? 0 : m->n_lstm); ++l) {
-        if (l > 0) {
-            ProfScope ps(ctx, "lstm_input_gemm", 2.0 * T * 4 * m->H * m->H);
-            GemmArgs g;                                   // pre[Tp x 4H] = H_{l-1} . W_in^T + b   ([unit][gate] columns)
-            g.A[0] = Hlimg[l - 1]; g.KB_A = m->H / TILE_K;
-            g.B[0] = tm->lstm_Win[l][0]; g.B[1] = tm->lstm_Win[l][1]; g.KB_B = m->H / TILE_K;
-            g.m_tiles = meta->m_tiles; g.n_tiles = 4 * m->H / 128; g.nkb = m->H / TILE_K;
-            g.out_f32 = pre; g.ldc = 4 * m->H; g.bias = tm->lstm_bperm[l];
-            g.m_valid = (int)Tp; g.n_valid = 4 * m->H;
-            MDF_TRY(launch_gemm_tc(ctx, EPI_F32_BIAS, 128, 1, 2, g));
-        }
-        {
-            ProfScope ps(ctx, "lstm_recurrent", 2.0 * T * 4 * m->H * m->H);
-            if (tm->lstm_Rstream[l][0] && n >= tm->lstm_stream_min)      // large batch: streamed weights, N = 128
-                MDF_TRY(launch_lstm_stream(ctx, m->H, n, tm->lstm_Rstream[l][0], tm->lstm_Rstream[l][1],
-                                           l == 0 ? tm->lstm_tab_full : nullptr, l > 0 ? pre : nullptr, idx_pad, b->d_order,
-                                           b->d_seq_off, row_off, Hlimg[l], scratch));
-            else                                                         // small batch: weights resident in smem, N = 32
-                MDF_TRY(launch_lstm_tc(ctx, m->H, n, tm->lstm_alternate ? tm->lstm_Ralt[l] : tm->lstm_R[l],
-                                       l == 0 ? tm->lstm_tab : nullptr, l > 0 ? pre : nullptr, idx_pad, b->d_order,
-                                       b->d_seq_off, row_off, Hlimg[l], scratch, tm->lstm_alternate));
-        }
-        b->tap_h[l] = nullptr;
     }
     if (b->owns_memory && b->reuse && !ctx->debug_taps) b->lm_hash = tm->lm_hash;
     if (ctx->debug_taps) {                                // fp32 copies of the LSTM outputs over packed residues

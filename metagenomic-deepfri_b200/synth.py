@@ -26,7 +26,8 @@ HEAD_SIZES = {"mf": 489, "bp": 1943, "cc": 320, "ec": 538}
 @dataclass
 class GCNConfig:
     n_channels: int = 26
-    lstm_hidden: int = 512          # LSTM-LM hidden size H (both layers)
+    lstm_hidden: int = 512          # LSTM-LM hidden size H (every layer)
+    lstm_layers: int = 2            # LSTM-LM depth (upstream DeepFRI: 2)
     lm_dim: int = 1024              # embedding width E
     gc_dims: Tuple[int, ...] = (512, 512, 512)
     fc_dim: int = 1024
@@ -53,7 +54,8 @@ def make_weights(cfg: GCNConfig, seed: int = 1234, lm_seed: int = 99) -> Dict[st
     rng = np.random.default_rng(seed)
     w: Dict[str, np.ndarray] = {}
     rec = np.sqrt(3.0 / H) * 1.5
-    for l, inp in ((1, I), (2, H)):
+    for l in range(1, cfg.lstm_layers + 1):
+        inp = I if l == 1 else H
         # ONNX LSTM layout: W[1,4H,in], R[1,4H,H], B[1,8H]; gate order i,o,f,c
         w[f"lstm{l}_W"] = _uniform(lm, 1.5 if l == 1 else rec * 2.0, (1, 4 * H, inp))
         w[f"lstm{l}_R"] = _uniform(lm, rec, (1, 4 * H, H))
@@ -116,7 +118,7 @@ def build_gcn_model(cfg: GCNConfig, weights: Optional[Dict[str, np.ndarray]] = N
     x = add("Transpose", ["seq"], ["lm/seq_tm"], perm=[1, 0, 2])
     if style == "tf2onnx":
         init["lm/zero_state"] = np.zeros((1, 1, H), np.float32)
-    for l in (1, 2):
+    for l in range(1, cfg.lstm_layers + 1):
         if style == "tf2onnx":
             y = add("LSTM", [x, f"lstm{l}_W", f"lstm{l}_R", f"lstm{l}_B", "", "lm/zero_state", "lm/zero_state"],
                     [f"lm/LSTM{l}_Y", f"lm/LSTM{l}_Yh", f"lm/LSTM{l}_Yc"], hidden_size=H, direction="forward")
@@ -124,7 +126,7 @@ def build_gcn_model(cfg: GCNConfig, weights: Optional[Dict[str, np.ndarray]] = N
             y = add("LSTM", [x, f"lstm{l}_W", f"lstm{l}_R", f"lstm{l}_B"],
                     [f"lm/LSTM{l}_Y"], hidden_size=H, direction="forward")
         x = add("Squeeze", [y, "const_axes_1"], [f"lm/LSTM{l}_out"])
-    lm_out = add("Transpose", [x], ["lm/LSTM2_bm"], perm=[1, 0, 2])
+    lm_out = add("Transpose", [x], [f"lm/LSTM{cfg.lstm_layers}_bm"], perm=[1, 0, 2])
     x_lm = add("MatMul", [lm_out, "LM_embedding_W"], ["LM_embedding/MatMul"])
     x_lm = add("Add", [x_lm, "LM_embedding_b"], ["LM_embedding/BiasAdd"])
     x_aa = add("MatMul", ["seq", "AA_embedding_W"], ["AA_embedding/MatMul"])

@@ -99,6 +99,28 @@ def test_path_against_oracle_config0_sample(engine, engines, model_dir):
     b.close()
 
 
+@pytest.mark.parametrize("layers", [1, 3])
+def test_lstm_depth_other_than_two_runs_on_simt(layers, tmp_path):
+    """The tensor-core engine computes the two-layer LSTM-LM that DeepFRI ships.  A model of another depth gets the exact-fp32
+    engine, which runs any depth, and cannot be switched to the tensor-core one."""
+    kw, seed, n, lo, hi = spec.GCN_CASES["tc_small"]
+    path = str(tmp_path / f"lstm{layers}.onnx")
+    synth.write_gcn_model(path, synth.GCNConfig(lstm_layers=layers, **kw), seed=seed)
+    pred = predict.Predictor(path)
+    try:
+        assert pred.engine == "simt"
+        with pytest.raises(ValueError, match="unavailable"):
+            pred.set_engine("tc")
+        wl = golden_workload("tc_small")
+        oracle = go.Predictor(path)
+        want = np.stack([oracle.forward_pass(s, c) for s, c in zip(wl.query_seqs, oracle_maps(wl))])
+        got = pred.forward_structures(wl.query_seqs, wl.gapped_query, wl.gapped_target, wl.coords, wl.threshold,
+                                      wl.generated_contacts)
+        assert_scores(got, want, TOL_SIMT)
+    finally:
+        pred.close()
+
+
 def test_batch_invariance_and_order(engines):
     """Scores of a protein do not depend on what else is in the batch or on its position."""
     pred = engines["small"]

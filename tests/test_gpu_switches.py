@@ -1,6 +1,6 @@
-"""The environment switches that remain in the library select code paths the default run never takes (the layer-by-layer LSTM
-kernels behind MDF_LSTM_FUSED=0, the padded residue axis, the dense adjacency walk, the separate pooling kernel, the
-full-square contact-map kernel ...).  Each one is exercised here against the exact-fp32 engine / the oracle so that it cannot
+"""The environment switches that remain in the library select code paths the default run never takes (the padded residue
+axis, the dense adjacency walk, the separate pooling kernel, the full-square contact-map kernel, the fused LSTM kernel without
+CTA pairs ...).  Each one is exercised here against the exact-fp32 engine / the oracle so that it cannot
 rot; the measured-and-rejected experiments of round 1 (CTA-pair adjacency kernel, N = 256 adjacency MMA, tile-dithered weights,
 CNN weight multicast) were deleted instead."""
 import os
@@ -12,8 +12,7 @@ import pytest
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
-SWITCHES = [{}, {"MDF_LSTM_FUSED": "0"}, {"MDF_LSTM_FUSED": "0", "MDF_LSTM_STREAM_MIN": "1"}, {"MDF_LSTM_FUSED": "0", "MDF_LSTM_HILO": "1"},
-            {"MDF_COMPACT": "0"}, {"MDF_ADJ_SPARSE": "0"}, {"MDF_POOL_FUSED": "0"}, {"MDF_ADJ_LEAN": "0"}, {"MDF_ADJ_EXPAND": "0"},
+SWITCHES = [{}, {"MDF_COMPACT": "0"}, {"MDF_ADJ_SPARSE": "0"}, {"MDF_POOL_FUSED": "0"}, {"MDF_ADJ_LEAN": "0"}, {"MDF_ADJ_EXPAND": "0"},
             {"MDF_GEMM_PAIR": "0"}, {"MDF_EMBED_STAGED": "0"}, {"MDF_HEAD_TC": "0"}, {"MDF_CMAP_SYM": "0"}, {"MDF_XW_MEAN": "0"}, {"MDF_LSTM_COOP": "0"},
             {"MDF_LSTM_PAIR": "0"}, {"MDF_LSTM_CELL": "0"}, {"MDF_LSTM_ABLATE": "64"}, {"MDF_LSTM_ABLATE": "384"}, {"MDF_LSTM_CLUSTER": "8"}, {"MDF_LSTM_PRECISE_LEN": "100"}, {"MDF_HOST_THREADS": "1"}]
 
