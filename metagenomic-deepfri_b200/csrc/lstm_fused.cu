@@ -62,6 +62,8 @@ constexpr int LF_MAX_KB = 8;
 #define LF_EPI_SLEEP_NS 200
 #endif
 constexpr size_t LF_SCRATCH_HEAD = 1 << 20;   // flags (8 KiB) + schedule, ahead of the exchange buffers
+constexpr size_t LF_FLAG_BYTES = 8192;         // release counters: [n_groups][halves][2 layers][LF_MAX_KB]
+constexpr int LF_MAX_GROUPS = (int)(LF_FLAG_BYTES / (2 * 2 * LF_MAX_KB * sizeof(unsigned)));   // groups the flag area holds (64)
 
 struct LstmFusedArgs {
     int H, n, n_groups, cpg, n_sub;
@@ -761,7 +763,9 @@ int launch_lstm_fused(mdf_ctx *ctx, int H, int n, const __half *W, int phases, c
     // cluster of 8 (h operand multicast to 4 slices) measured: same tick, but only 8 groups fit (GPC granularity) -> 2 is the default
     static const int cluster_env = getenv("MDF_LSTM_CLUSTER") ? atoi(getenv("MDF_LSTM_CLUSTER")) : 2;
     a.spc = (pair && cluster_env >= 8 && a.cpg % 4 == 0) ? 4 : 1;
-    int max_groups = std::max(1, ctx->sm_count / (a.cpg * (pair ? 2 : 1)));
+    // one group per cpg slices (CTA pairs in pair mode), at most what the flag area holds: at small H a full GPU has room for more
+    // groups (148 SMs, H = 64 in pairs: 74); the sub-batches beyond the groups are scheduled onto them below
+    int max_groups = std::max(1, std::min(LF_MAX_GROUPS, ctx->sm_count / (a.cpg * (pair ? 2 : 1))));
     if (pair && a.spc > 1) {
         // clusters of 2*spc CTAs must fit inside a GPC: ask the driver how many can be co-resident
         static int max_clusters = -1;
@@ -787,10 +791,10 @@ int launch_lstm_fused(mdf_ctx *ctx, int H, int n, const __half *W, int phases, c
     a.precise_len = precise_env;
     a.tab = tab; a.b2 = b2; a.idx_pad = idx_pad; a.order = order;
     a.seq_off = seq_off; a.seg_off = seg_off; a.H1img = H1img; a.H2img = H2img;
-    if ((size_t)a.n_groups * 2 * 2 * LF_MAX_KB * sizeof(unsigned) > 8192) { set_error("lstm_fused: too many groups"); return MDF_EUNSUPPORTED; }
+    if (a.n_groups > LF_MAX_GROUPS) { set_error("lstm_fused: internal error: %d groups, the flag area holds %d", a.n_groups, LF_MAX_GROUPS); return MDF_EUNSUPPORTED; }
     a.flags = reinterpret_cast<unsigned *>(scratch);
     a.hbuf = reinterpret_cast<__half *>(reinterpret_cast<uint8_t *>(scratch) + LF_SCRATCH_HEAD);
-    MDF_CUDA(cudaMemsetAsync(scratch, 0, 8192, ctx->stream));
+    MDF_CUDA(cudaMemsetAsync(scratch, 0, LF_FLAG_BYTES, ctx->stream));
     {
         // Schedule: sub-batch j = proteins order[j*sub_n ..] (length-descending) costs Lmax_j + 1 ticks whatever its other
         // members' lengths; longest-processing-time-first over the groups keeps them within one sub-batch of each other

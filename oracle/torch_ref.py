@@ -9,7 +9,7 @@ published ONNX operator semantics (opset 15), decoded by `oracle/onnx_pb.py` (Go
 `tests/test_oracle_torch.py` requires the NumPy oracle and this executor to agree to <= 1e-5 on every
 golden case, so a shared misreading of the LSTM weight layout, the gate order, the bias split, the
 Conv padding or the [C, 2] reshape would have to be made three times (here, in the NumPy oracle and in the
-float64 layer-equation restatement of `tests/test_onnx.py`) to go unnoticed.
+float64 layer-equation restatement of `oracle/gcn_f64.py`) to go unnoticed.
 """
 from __future__ import annotations
 

@@ -1,11 +1,12 @@
 """CPU tests: ONNX wire format, graph recognition by the library's own loader (`csrc/onnx_load.cu` through
 `mdf_onnx_inspect` / `mdf_onnx_tensor`: host-only entry points, no GPU needed), and the GCN oracle against an independent
-NumPy restatement of upstream DeepFRI's layer equations (SURVEY.md §3.3)."""
+NumPy restatement of upstream DeepFRI's layer equations (SURVEY.md §3.3, `oracle/gcn_f64.py`)."""
 import numpy as np
 import pytest
 
 import cmap_oracle as co
 import gcn_oracle as go
+from gcn_f64 import deepfri_numpy
 from conftest import golden_workload, recognise
 from metagenomic_deepfri_b200 import onnx_lite as ox
 from metagenomic_deepfri_b200 import synth
@@ -172,43 +173,6 @@ def test_heads_share_language_model():
     c = dict(a)
     c["lstm2_R"] = a["lstm2_R"] + np.float32(1e-3)
     assert recognise(synth.build_gcn_model(synth.GCNConfig(n_terms=489), c)).lm_fingerprint != pa.lm_fingerprint
-
-
-def deepfri_numpy(w, cfg, seq, cmap):
-    """Independent float64 restatement of upstream DeepFRI's equations (not the ONNX interpreter)."""
-    S = co.seq2onehot(seq).astype(np.float64)
-    H = cfg.lstm_hidden
-    sig = lambda x: 1 / (1 + np.exp(-x))
-
-    def lstm(X, W, R, B):
-        W, R = W[0].astype(np.float64), R[0].astype(np.float64)
-        b = (B[0, :4 * H] + B[0, 4 * H:]).astype(np.float64)
-        h = np.zeros(H); c = np.zeros(H); out = []
-        for x in X:
-            z = W @ x + R @ h + b
-            i, o, f, g = sig(z[:H]), sig(z[H:2 * H]), sig(z[2 * H:3 * H]), np.tanh(z[3 * H:])
-            c = f * c + i * g
-            h = o * np.tanh(c)
-            out.append(h)
-        return np.array(out)
-    h = lstm(lstm(S, w["lstm1_W"], w["lstm1_R"], w["lstm1_B"]), w["lstm2_W"], w["lstm2_R"], w["lstm2_B"])
-    x = np.maximum(h @ w["LM_embedding_W"] + w["LM_embedding_b"] + S @ w["AA_embedding_W"], 0)
-    A = cmap.astype(np.float64)
-    A = A - np.diag(np.diag(A)) + np.eye(len(A))
-    d = 1.0 / (cfg.eps + np.sqrt(A.sum(1)))
-    An = d[:, None] * A * d[None, :]
-    outs = []
-    for l in range(1, len(cfg.gc_dims) + 1):
-        z = (An @ x) @ w[f"GraphConv_{l}_W"]
-        if cfg.gc_bias:
-            z = z + w[f"GraphConv_{l}_b"]
-        x = np.where(z > 0, z, np.exp(np.minimum(z, 0)) - 1) if cfg.gc_activation == "Elu" else np.maximum(z, 0)
-        outs.append(x)
-    p = np.concatenate(outs, 1).sum(0)
-    f = np.maximum(p @ w["dense_W"] + w["dense_b"], 0)
-    o = (f @ w["labels_W"] + w["labels_b"]).reshape(-1, 2)
-    e = np.exp(o - o.max(1, keepdims=True))
-    return (e / e.sum(1, keepdims=True))[:, 0]
 
 
 @pytest.mark.parametrize("tag", ["small", "small_relu_bias"])
