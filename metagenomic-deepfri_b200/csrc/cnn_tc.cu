@@ -375,7 +375,8 @@ extern "C" int mdf_cnn_model_create(mdf_ctx *ctx, const mdf_cnn_desc *d, mdf_cnn
 {
     MDF_REQUIRE(ctx && d && out, "mdf_cnn_model_create: bad arguments");
     MDF_REQUIRE(d->n_channels == 26, "cnn model: expected 26 input channels, got %d", d->n_channels);
-    MDF_REQUIRE(d->n_conv >= 1 && d->n_conv <= MDF_MAX_CONV, "cnn model: %d conv layers unsupported", d->n_conv);
+    MDF_REQUIRE(d->n_conv >= 1 && d->n_conv <= MDF_MAX_CONV, "cnn model: %d Conv layers unsupported: the kernel takes 1 to at most %d",
+                d->n_conv, MDF_MAX_CONV);
     MDF_REQUIRE(d->scale && d->shift && d->out_W && d->n_terms > 0, "cnn model: missing weights");
     MDF_CUDA(cudaSetDevice(ctx->device));
     mdf_cnn_model *m = new mdf_cnn_model();
@@ -387,7 +388,8 @@ extern "C" int mdf_cnn_model_create(mdf_ctx *ctx, const mdf_cnn_desc *d, mdf_cnn
     for (int c = 0; c < d->n_conv; ++c) {
         const int w = d->conv_width[c], F = d->conv_filters[c], pl = d->conv_pad_left[c];
         if (w < 1 || w > 128 || F < 128 || F % 128 != 0 || pl < 0 || pl >= w || !d->conv_W[c]) {
-            set_error("cnn model: conv layer %d (width %d, %d filters, pad %d) unsupported: width <= 128, filters a multiple of 128", c, w, F, pl);
+            set_error("cnn model: conv layer %d (width %d, %d filters, left pad %d) unsupported: the kernel takes widths 1..128, filters "
+                      "a multiple of 128 and 0 <= pad < width", c, w, F, pl);
             return fail(MDF_EUNSUPPORTED);
         }
         const int steps = w + (w + 1) / 2 + ((w + 3) / 4 + 1) / 2;      // K = 16 steps (see the header): 13 per 8 positions
@@ -399,8 +401,13 @@ extern "C" int mdf_cnn_model_create(mdf_ctx *ctx, const mdf_cnn_desc *d, mdf_cnn
         m->macs_per_residue += 26.0 * w * F;
         m->issued_macs_per_row += 16.0 * 4 * m->kb[c] * F;
     }
-    if (m->n_items > CNN_MAX_ITEMS || 128 + m->pl_max + pr_max + 1 > CNN_WIN) {      // + 1: the partner row of a zero column
-        set_error("cnn model: %d filter blocks / window of %d residues exceed the kernel's limits", m->n_items, 128 + m->pl_max + pr_max);
+    if (m->n_items > CNN_MAX_ITEMS) {
+        set_error("cnn model: %d filter blocks of 128 filters unsupported: the kernel takes at most %d", m->n_items, CNN_MAX_ITEMS);
+        return fail(MDF_EUNSUPPORTED);
+    }
+    if (128 + m->pl_max + pr_max + 1 > CNN_WIN) {                                       // + 1: the partner row of a zero column
+        set_error("cnn model: one-hot window of %d residues (128 + left reach %d + right reach %d + 1) unsupported: the kernel's image "
+                  "holds at most %d", 128 + m->pl_max + pr_max + 1, m->pl_max, pr_max, CNN_WIN);
         return fail(MDF_EUNSUPPORTED);
     }
     int r;

@@ -1239,7 +1239,10 @@ extern "C" int mdf_cnn_model_load(mdf_ctx *ctx, const char *onnx_path, mdf_cnn_m
     Plan p;
     MDF_TRY(load_plan(onnx_path, p));
     if (!p.is_cnn) { set_error("%s: two-input model: this is a GCN head, use mdf_model_load", onnx_path); return MDF_EUNSUPPORTED; }
-    if (p.conv_W.size() > MDF_MAX_CONV) { set_error("%s: DeepCNN model has more parallel Conv layers than the kernel supports", onnx_path); return MDF_EUNSUPPORTED; }
+    if (p.conv_W.size() > MDF_MAX_CONV) {
+        set_error("%s: DeepCNN model has %zu parallel Conv layers: the kernel takes at most %d", onnx_path, p.conv_W.size(), MDF_MAX_CONV);
+        return MDF_EUNSUPPORTED;
+    }
     mdf_cnn_desc d;
     memset(&d, 0, sizeof d);
     d.n_channels = 26; d.n_conv = (int)p.conv_W.size();

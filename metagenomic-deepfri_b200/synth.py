@@ -199,6 +199,7 @@ class CNNConfig:
     n_terms: int = 489
     bn_epsilon: float = 1e-3          # Keras BatchNormalization default
     logit_scale: float = 0.15
+    pad_left: Optional[Tuple[int, ...]] = None   # zeros before position 0 per conv; None: Keras 'same', (k - 1) // 2
 
 
 def make_cnn_weights(cfg: CNNConfig, seed: int = 4321) -> Dict[str, np.ndarray]:
@@ -221,7 +222,8 @@ def make_cnn_weights(cfg: CNNConfig, seed: int = 4321) -> Dict[str, np.ndarray]:
 
 def build_cnn_model(cfg: CNNConfig, weights: Optional[Dict[str, np.ndarray]] = None, seed: int = 4321) -> ox.Model:
     """DeepCNN head as an ONNX graph in tf2onnx style: one input `seq` [b, L, 26] (the reference feeds it alone,
-    `predict.pyx:91-95`), channels-first Conv nodes with explicit TF 'same' pads ((k-1)//2 before, the rest after),
+    `predict.pyx:91-95`), channels-first Conv nodes with explicit pads (cfg.pad_left before, default TF 'same' (k-1)//2,
+    and the rest of k - 1 after),
     Concat, BatchNormalization, Relu, ReduceMax over residues, MatMul/Add, Reshape, Softmax -> [1, C, 2]."""
     w = dict(weights) if weights is not None else make_cnn_weights(cfg, seed)
     g = ox.Graph(name="DeepCNN")
@@ -241,7 +243,7 @@ def build_cnn_model(cfg: CNNConfig, weights: Optional[Dict[str, np.ndarray]] = N
     x = add("Unsqueeze", [x, "const_axes_2"], ["seq_cf4"])                    # [b, 26, 1, L]
     outs = []
     for l, k in enumerate(cfg.filter_lens, 1):
-        pl = (k - 1) // 2
+        pl = cfg.pad_left[l - 1] if cfg.pad_left is not None else (k - 1) // 2
         y = add("Conv", [x, f"conv1d_{l}_W", f"conv1d_{l}_b"], [f"conv1d_{l}/Conv2D"], kernel_shape=[1, k], strides=[1, 1],
                 dilations=[1, 1], group=1, pads=[0, pl, 0, k - 1 - pl])
         outs.append(add("Squeeze", [y, "const_axes_2"], [f"conv1d_{l}/Squeeze"]))   # [b, F, L]

@@ -111,3 +111,170 @@ def tc_shape_lengths(seed, long=False):
     lengths = list(TC_EXACT_LENGTHS) + [int(L) for L in rng.integers(1, 401, 15)] + ([TC_LONG[0]] if long else [])
     rng.shuffle(lengths)
     return lengths
+
+
+# ---- shape matrix of the DeepCNN tensor-core kernel (tests/test_gpu_cnn_shapes.py; the float64 reference oracle/cnn_f64.py is
+# pinned and the matrix's reach is restated on the CPU by tests/test_cnn_f64_reference.py).
+# tag -> (CNNConfig kwargs, model seed, graph edits (cnn_case), the branch the shape reaches).  w = width, F = filters, KB =
+# 64-wide k-blocks of a conv, window = 128 + pl_max + pr_max + 1 residues of the shared-memory one-hot image (at most 256).
+# logit_scale puts at least half of the float64 reference scores of the case's batch in [0.05, 0.95] (asserted).
+def _cycle_pads(widths):
+    """Keras, SAME_LOWER, 0, w - 1 in turn."""
+    return tuple((w - 1) // 2 if i % 4 == 0 else w // 2 if i % 4 == 1 else 0 if i % 4 == 2 else w - 1 for i, w in enumerate(widths))
+
+
+CNN_SHAPES = {
+    "w1": (dict(filter_lens=(1,), num_filters=(128,), pad_left=(0,), n_terms=1, logit_scale=0.5), 61, (),
+           "KB = 1 with an all-zero K step; plane-2 and plane-3 zero partners; 2C = 2 in one head tile"),
+    "narrow": (dict(filter_lens=(2, 3, 4, 5, 7, 8, 9), num_filters=(128,) * 7, n_terms=3, logit_scale=0.4), 62, (),
+               "KB 1 ... 4; exact fit (w = 2, 9) and padded k-blocks; 2C = 6 -> ld 8"),
+    "lower": (dict(filter_lens=(2, 4, 6, 16, 64, 128), num_filters=(128, 256, 128, 256, 128, 256), pad_left=(1, 2, 3, 8, 32, 64),
+                   n_terms=24, logit_scale=0.5), 63, ("same_lower",),
+              "auto_pad SAME_LOWER (pl = w / 2); window exactly 256 (128 + 64 + 63 + 1)"),
+    "skew": (dict(filter_lens=(64, 64, 1), num_filters=(128, 128, 128), pad_left=(63, 0, 0), n_terms=24, logit_scale=0.5), 64, (),
+             "explicit asymmetric pads; pl_max and pr_max from different convs, window 255"),
+    "edge_right": (dict(filter_lens=(128, 125), num_filters=(128, 128), pad_left=(0, 0), n_terms=24, logit_scale=0.5), 65, (),
+                   "window 256 from the right; plane-3 columns reach past the kernel (w = 125)"),
+    "edge_left": (dict(filter_lens=(128, 4), num_filters=(128, 128), pad_left=(127, 3), n_terms=24, logit_scale=0.5), 66, (),
+                  "window 256 from the left"),
+    "conv32": (dict(filter_lens=tuple(range(1, 33)), num_filters=(128,) * 32, pad_left=_cycle_pads(range(1, 33)), n_terms=40,
+                    logit_scale=0.3), 67, (),
+               "MDF_MAX_CONV = 32 convs: 32 K-step table offsets and channel offsets"),
+    "items256": (dict(filter_lens=(3,), num_filters=(32768,), pad_left=(1,), n_terms=24, logit_scale=0.3), 68, (),
+                 "256 filter blocks, item_fb up to 255 (unsigned char); head K = 32768"),
+    "mf_negbn": (dict(n_terms=1943, logit_scale=0.3), 69, ("neg_gamma",),
+                 "BN gamma < 0 on a quarter of the channels: negative scale in the epilogue FMA; the widest head (2C = 3886)"),
+    "lowering": (dict(filter_lens=(5, 8, 16), num_filters=(128, 256, 128), n_terms=24, logit_scale=0.5), 70,
+                 ("permute_concat", "no_bn", "no_conv_bias", "gemm_transB"),
+                 "loader: Concat inputs out of node order, no BatchNormalization, Conv without bias, Gemm(transB = 1) head "
+                 "without bias"),
+}
+# shapes whose load must raise NotImplementedError naming the limit: tag -> (CNNConfig kwargs, seed, message pattern)
+CNN_REFUSED = {
+    "w129": (dict(filter_lens=(129,), num_filters=(128,), n_terms=5), 71, r"widths 1\.\.128"),
+    "f192": (dict(filter_lens=(8,), num_filters=(192,), n_terms=5), 72, r"multiple of 128"),
+    "window257": (dict(filter_lens=(128, 2), num_filters=(128, 128), pad_left=(0, 1), n_terms=5), 73, r"window of 257 residues .* at most 256"),
+    "blocks257": (dict(filter_lens=(1, 1), num_filters=(32768, 128), n_terms=5), 74, r"257 filter blocks .* at most 256"),
+    "conv33": (dict(filter_lens=tuple(range(1, 34)), num_filters=(128,) * 33, n_terms=5), 75, r"33 parallel Conv layers: .* at most 32"),
+    "pad_neg": (dict(filter_lens=(8,), num_filters=(128,), pad_left=(-1,), n_terms=5), 76, r"0 <= pad < width"),
+    "pad_w": (dict(filter_lens=(8,), num_filters=(128,), pad_left=(8,), n_terms=5), 77, r"0 <= pad < width"),
+}
+# oracle/cnn_f64.MUTANTS -> the shapes whose batch must show it: the shape that claims the branch, and `lowering` where the
+# defect can show there (it has no BatchNormalization and no conv bias: every scale is 1 and every shift 0, so the epilogue
+# mutants take conv32; abs_scale changes nothing where every scale is positive: only mf_negbn has negative ones)
+CNN_MUTANT_SHAPES = {
+    "pad_shift": ("skew", "lowering"),
+    "drop_last_position": ("narrow", "lowering"),
+    "swap_24_25": ("w1", "lowering"),
+    "plane3_next_residue": ("edge_right", "lowering"),
+    "pad_rows": ("w1", "lowering"),
+    "first_512": ("conv32", "lowering"),
+    "neighbour_block_bn": ("items256", "conv32"),
+    "abs_scale": ("mf_negbn",),
+}
+# shapes whose reference is costly (wide convs or heads): a shorter batch (cnn_shape_sequences)
+CNN_WIDE = ("items256", "mf_negbn")
+CNN_EXACT_LENGTHS = (1, 2, 3, 127, 128, 129, 255, 256, 257, 511, 512, 513, 640, 1000)
+CNN_PROBE_POS = (0, 1, 2, 3, 126, 127, 128, 129)      # and L - 1: a single R / M on a poly-A background
+
+# Bounds of the GPU shape matrix, shared with the CPU sensitivity test (every mutant of oracle/cnn_f64.MUTANTS must exceed
+# 10 x CNN_BOUNDS["pooled_r16"]).  The bounds are to be set to twice the worst value over the matrix and the batch-structure
+# cases measured on an NVIDIA B200 (the test prints the worst per metric with its shape and protein length); until then they
+# are the expected orders below, NOT MEASURED on the GPU:
+#   pooled_r16: max |G - R16| over a batch's pooled features / RMS of R16's pooled features
+#   pooled_r64: the same against R64 (includes the fp16 rounding of the conv weights)
+#   head:       max |scores - float64 dense + softmax of the kernel's own pooled vector|
+#   scores:     max |scores - R64 scores| (with the +-1e-3 guard band around the 0.1 call)
+CNN_BOUNDS = {
+    "pooled_r16": 2e-5,    # fp32 accumulation of at most 128 exact fp16 x 1.0 products per output: ~1e-6 expected
+    "pooled_r64": 2e-3,    # R64 - R16 alone (the fp16 rounding of the conv weights) is up to 8.2e-4 over the matrix (lower)
+    "head": 1e-4,          # the exact hi + lo split of the dense weights: fp32-level error expected
+    "scores": 1e-3,        # the north-star tolerance of every score test
+}
+
+
+def cnn_case(kw, seed, edits=()):
+    """A DeepCNN case -> (cfg, w, model): the ONNX model with `edits` applied, and the config and weight dict the float64
+    reference reads for the same function (conv order = Concat order; weights the graph does not have are left out).
+      same_lower:     auto_pad SAME_LOWER instead of explicit pads (cfg.pad_left must be the SAME_LOWER pads);
+      neg_gamma:      BN gamma negated on every fourth channel (1, 5, 9, ...);
+      permute_concat: Concat inputs in reverse node order;
+      no_bn:          no BatchNormalization node;  no_conv_bias: Convs without bias;
+      gemm_transB:    Gemm(transB = 1) with the transposed weight and no bias in place of MatMul + Add."""
+    import dataclasses
+    import numpy as np
+    from metagenomic_deepfri_b200 import synth
+    cfg = synth.CNNConfig(**kw)
+    w = synth.make_cnn_weights(cfg, seed)
+    if "neg_gamma" in edits:
+        g = w["bn_gamma"].copy()
+        g[1::4] *= -1
+        w["bn_gamma"] = g
+    m = synth.build_cnn_model(cfg, w)
+    g = m.graph
+    convs = [n for n in g.nodes if n.op_type == "Conv"]
+    if "same_lower" in edits:
+        if cfg.pad_left != tuple(k - 1 - (k - 1) // 2 for k in cfg.filter_lens):
+            raise ValueError("same_lower: cfg.pad_left is not SAME_LOWER's")
+        for n in convs:
+            n.attrs.pop("pads")
+            n.attrs["auto_pad"] = "SAME_LOWER"
+    if "no_conv_bias" in edits:
+        for l, n in enumerate(convs, 1):
+            del n.inputs[2:]
+            del g.initializers[f"conv1d_{l}_b"]
+            del w[f"conv1d_{l}_b"]
+    if "no_bn" in edits:
+        bn = next(n for n in g.nodes if n.op_type == "BatchNormalization")
+        relu = next(n for n in g.nodes if n.op_type == "Relu")
+        relu.inputs[0] = bn.inputs[0]
+        g.nodes.remove(bn)
+        for k in ("bn_gamma", "bn_beta", "bn_mean", "bn_var"):
+            del g.initializers[k]
+            del w[k]
+    if "gemm_transB" in edits:
+        mm = next(n for n in g.nodes if n.op_type == "MatMul")
+        add = next(n for n in g.nodes if n.op_type == "Add" and mm.outputs[0] in n.inputs)
+        g.initializers["labels_W_T"] = np.ascontiguousarray(w["labels_W"].T)
+        g.nodes[g.nodes.index(mm)] = type(mm)("Gemm", [mm.inputs[0], "labels_W_T"], [add.outputs[0]], name="Gemm__head",
+                                              attrs={"transB": 1})
+        g.nodes.remove(add)
+        del g.initializers["labels_W"], g.initializers["labels_b"]
+        del w["labels_b"]
+    if "permute_concat" in edits:
+        cat = next(n for n in g.nodes if n.op_type == "Concat")
+        cat.inputs.reverse()
+        nc = len(convs)
+        wr = {k: v for k, v in w.items() if not k.startswith("conv1d_")}
+        for l in range(1, nc + 1):
+            for s in ("W", "b"):
+                if f"conv1d_{nc + 1 - l}_{s}" in w:
+                    wr[f"conv1d_{l}_{s}"] = w[f"conv1d_{nc + 1 - l}_{s}"]
+        pads = cfg.pad_left if cfg.pad_left is not None else tuple((k - 1) // 2 for k in cfg.filter_lens)
+        cfg = dataclasses.replace(cfg, filter_lens=cfg.filter_lens[::-1], num_filters=cfg.num_filters[::-1], pad_left=pads[::-1])
+        w = wr
+    return cfg, w, m
+
+
+def cnn_shape_sequences(tag):
+    """The batch of a CNN_SHAPES case over the full 26-letter alphabet, in shuffled order: the tile and group edges of
+    CNN_EXACT_LENGTHS, random lengths in 1-400, R / M / '-' homopolymers, a single R or M on a poly-A background at
+    CNN_PROBE_POS and at L - 1, and one protein of about 2,000 residues.  The wide shapes (CNN_WIDE) get fewer and shorter
+    ones, to keep their float64 reference to a few thousand residues."""
+    import numpy as np
+    seed = CNN_SHAPES[tag][1]
+    rng = np.random.default_rng(seed + 100)
+    letters = np.array(list(CNN_ALPHABET))
+    wide = tag in CNN_WIDE
+    lengths = [L for L in CNN_EXACT_LENGTHS if not wide or L <= 513] + [int(L) for L in rng.integers(1, 401, 5 if wide else 15)]
+    if not wide:
+        lengths.append(int(rng.integers(1950, 2051)))
+    seqs = ["".join(rng.choice(letters, L)) for L in lengths]
+    hl = 40 if wide else 150
+    seqs += ["R" * hl, "M" * hl, "-" * hl]
+    pl = 131
+    for ch in ("RM"[:1] if wide else "RM"):
+        for p in CNN_PROBE_POS + (pl - 1,):
+            seqs.append("A" * p + ch + "A" * (pl - 1 - p))
+    order = rng.permutation(len(seqs))
+    return [seqs[i] for i in order]

@@ -7,6 +7,7 @@ import numpy as np
 import pytest
 
 import gcn_oracle as go
+from cnn_f64 import deepcnn_f64
 from metagenomic_deepfri_b200 import onnx_lite as ox
 from metagenomic_deepfri_b200 import synth
 from metagenomic_deepfri_b200._lib import UnsupportedModelError
@@ -14,31 +15,6 @@ from conftest import recognise
 import spec
 
 ALPHABET = "-DGULNTKHYWCPVSOIEFXQABZRM"
-
-
-def deepcnn_f64(w, cfg, seq):
-    """Keras semantics, loop form: Conv1D(padding='same') pads (k-1)//2 zeros before and the rest after; BatchNormalization
-    (inference) ; ReLU ; GlobalMaxPooling1D ; dense ; softmax over (C, 2) pairs."""
-    L = len(seq)
-    idx = [ALPHABET.index(ch) for ch in seq]
-    feats = []
-    for l, k in enumerate(cfg.filter_lens, 1):
-        W = w[f"conv1d_{l}_W"][:, :, 0, :].astype(np.float64)       # [F, 26, k]
-        b = w[f"conv1d_{l}_b"].astype(np.float64)
-        pl = (k - 1) // 2
-        y = np.tile(b, (L, 1))
-        for t in range(L):
-            for j in range(k):
-                r = t + j - pl
-                if 0 <= r < L:
-                    y[t] += W[:, idx[r], j]
-        feats.append(y)
-    x = np.concatenate(feats, axis=1)
-    x = (x - w["bn_mean"]) / np.sqrt(w["bn_var"].astype(np.float64) + cfg.bn_epsilon) * w["bn_gamma"] + w["bn_beta"]
-    p = np.maximum(x, 0).max(axis=0)
-    z = (p @ w["labels_W"].astype(np.float64) + w["labels_b"]).reshape(cfg.n_terms, 2)
-    e = np.exp(z - z.max(axis=1, keepdims=True))
-    return (e / e.sum(axis=1, keepdims=True))[:, 0]
 
 
 @pytest.mark.parametrize("tag", ["cnn_small"])
