@@ -1121,11 +1121,14 @@ extern "C" int mdf_model_create(mdf_ctx *ctx, const mdf_model_desc *d, mdf_model
 {
     MDF_REQUIRE(ctx && d && out, "mdf_model_create: bad arguments");
     MDF_REQUIRE(d->n_channels == 26, "model: expected 26 input channels, got %d", d->n_channels);
-    MDF_REQUIRE(d->n_lstm >= 1 && d->n_lstm <= MDF_MAX_LSTM, "model: unsupported LSTM depth %d", d->n_lstm);
+    MDF_REQUIRE(d->n_lstm >= 1 && d->n_lstm <= MDF_MAX_LSTM, "model: %d LSTM layers: the engines take at least 1 and at most %d",
+                d->n_lstm, MDF_MAX_LSTM);
     MDF_REQUIRE(d->lstm_hidden >= 16 && d->lstm_hidden % 16 == 0 && d->lstm_hidden <= 512,
-                "model: LSTM hidden size %d unsupported (multiple of 16, <= 512)", d->lstm_hidden);
-    MDF_REQUIRE(d->n_gc >= 1 && d->n_gc <= MDF_MAX_GC, "model: unsupported GraphConv depth %d", d->n_gc);
-    MDF_REQUIRE(d->lm_dim > 0 && d->lm_dim % 4 == 0 && d->fc_dim > 0 && d->n_terms > 0, "model: bad dense dimensions");
+                "model: LSTM hidden size %d unsupported: the LSTM kernel takes a multiple of 16 from 16 to 512", d->lstm_hidden);
+    MDF_REQUIRE(d->n_gc >= 1 && d->n_gc <= MDF_MAX_GC, "model: %d GraphConv layers: the engines take at least 1 and at most %d",
+                d->n_gc, MDF_MAX_GC);
+    MDF_REQUIRE(d->lm_dim > 0 && d->lm_dim % 4 == 0, "model: embedding width %d: the engines take a positive multiple of 4", d->lm_dim);
+    MDF_REQUIRE(d->fc_dim > 0 && d->n_terms > 0, "model: dense width %d and %d GO terms: both must be positive", d->fc_dim, d->n_terms);
     MDF_REQUIRE(d->aa_W && d->lm_W && d->fc_W && d->out_W, "model: missing dense weights");
     MDF_REQUIRE(d->gc_activation >= 0 && d->gc_activation <= 2, "model: unknown GraphConv activation %d", d->gc_activation);
     MDF_CUDA(cudaSetDevice(ctx->device));
@@ -1169,7 +1172,11 @@ extern "C" int mdf_model_create(mdf_ctx *ctx, const mdf_model_desc *d, mdf_model
     m->G = 0;
     for (int l = 0; l < m->n_gc; ++l) {
         m->gc[l] = d->gc_dims[l];
-        if (m->gc[l] <= 0 || m->gc[l] % 4 != 0 || !d->gc_W[l]) { set_error("model: GraphConv layer %d invalid", l); return fail(MDF_EINVAL); }
+        if (m->gc[l] <= 0 || m->gc[l] % 4 != 0) {
+            set_error("model: GraphConv layer %d has width %d: the engines take a positive multiple of 4", l + 1, m->gc[l]);
+            return fail(MDF_EINVAL);
+        }
+        if (!d->gc_W[l]) { set_error("model: GraphConv layer %d weights missing", l + 1); return fail(MDF_EINVAL); }
         if ((r = upload_or_zero(m, &m->gc_W[l], d->gc_W[l], (size_t)prev * m->gc[l])) != MDF_OK) return fail(r);
         if (d->gc_b[l]) {
             if ((r = upload_or_zero(m, &m->gc_b[l], d->gc_b[l], (size_t)m->gc[l])) != MDF_OK) return fail(r);

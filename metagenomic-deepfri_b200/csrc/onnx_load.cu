@@ -1219,7 +1219,14 @@ extern "C" int mdf_model_load(mdf_ctx *ctx, const char *onnx_path, mdf_model **o
     Plan p;
     MDF_TRY(load_plan(onnx_path, p));
     if (p.is_cnn) { set_error("%s: single-input model: this is a sequence-only DeepCNN head, use mdf_cnn_model_load", onnx_path); return MDF_EUNSUPPORTED; }
-    if (p.lstm_W.size() > MDF_MAX_LSTM || p.gc_W.size() > MDF_MAX_GC) { set_error("%s: model deeper than the fused pipeline supports", onnx_path); return MDF_EUNSUPPORTED; }
+    if (p.lstm_W.size() > MDF_MAX_LSTM) {
+        set_error("%s: %zu LSTM layers: the engines take at most %d", onnx_path, p.lstm_W.size(), MDF_MAX_LSTM);
+        return MDF_EUNSUPPORTED;
+    }
+    if (p.gc_W.size() > MDF_MAX_GC) {
+        set_error("%s: %zu GraphConv layers: the engines take at most %d", onnx_path, p.gc_W.size(), MDF_MAX_GC);
+        return MDF_EUNSUPPORTED;
+    }
     mdf_model_desc d;
     memset(&d, 0, sizeof d);
     d.n_channels = 26; d.lstm_hidden = p.H; d.n_lstm = (int)p.lstm_W.size();

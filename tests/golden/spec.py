@@ -89,9 +89,10 @@ TC_EXACT_LENGTHS = (1, 2, 3, 63, 64, 65, 127, 128, 129, 255, 256, 257, 511, 512,
 TC_LONG = (901, 1103)     # the second crosses MDF_LSTM_PRECISE_LEN (1000): the LSTM's exact weight split
 
 
-def structure_batch(lengths, seed):
+def structure_batch(lengths, seed, maps_for=None):
     """Seeded proteins of exactly these lengths with their own structures (ungapped self-alignments, 10 A, 2 generated
-    contacts) -> (Workload, dense contact maps of the oracle)."""
+    contacts) -> (Workload, dense contact maps of the oracle).  `maps_for`: the proteins whose maps to build (default all;
+    the others get None), for batches too large to hold every dense map."""
     import numpy as np
     import cmap_oracle as co
     from metagenomic_deepfri_b200 import synth
@@ -100,7 +101,9 @@ def structure_batch(lengths, seed):
     seqs = synth.random_sequences(rng, lengths)
     coords = synth.random_walk_coords(rng, lengths)
     wl = synth.Workload(seqs, list(seqs), list(seqs), coords, THRESHOLD, GEN, f"exact_lengths_seed{seed}")
-    return wl, [co.build_align_contact_map(s, s, c, THRESHOLD, GEN) for s, c in zip(seqs, coords)]
+    want = range(len(seqs)) if maps_for is None else set(int(i) for i in maps_for)
+    return wl, [co.build_align_contact_map(s, s, c, THRESHOLD, GEN) if i in want else None
+                for i, (s, c) in enumerate(zip(seqs, coords))]
 
 
 def tc_shape_lengths(seed, long=False):
@@ -278,3 +281,113 @@ def cnn_shape_sequences(tag):
             seqs.append("A" * p + ch + "A" * (pl - 1 - p))
     order = rng.permutation(len(seqs))
     return [seqs[i] for i in order]
+
+
+# ---- shape matrix of the exact-fp32 engine (tests/test_gpu_simt_shapes.py; the float64 reference's mutants and the matrix's
+# reach are restated on the CPU by tests/test_gcn_f64_simt_reference.py).  Every shape is one the tensor-core engine refuses
+# and the exact-fp32 engine serves (mdf_model_create: 1-4 LSTM layers, H = 16 ... 512 in steps of 16, 1-8 GraphConv layers,
+# E and every width a multiple of 4, any F and C).  tag -> (GCNConfig kwargs, model seed, the branch the shape reaches).
+# cpg = H / 16 CTAs per LSTM group, 148 / cpg groups on a B200; GEMM tiles are 64 x 64 x 16 (BK = 16), the aggregate takes
+# 512 columns per pass.  logit_scale puts at least half of the float64 reference scores of the case's batch in [0.05, 0.95].
+SIMT_SHAPES = {
+    "h16_min": (dict(lstm_hidden=16, lstm_layers=1, lm_dim=4, gc_dims=(4,), fc_dim=1, n_terms=1, logit_scale=0.03), 91,
+                "cpg = 1 (148 groups of one CTA); K = 4 (X.W, dense) and 1 (labels) < BK; 127 of 128 aggregate threads idle"),
+    "h32_d4": (dict(lstm_hidden=32, lstm_layers=4, lm_dim=20, gc_dims=(12, 36), fc_dim=10, n_terms=3, logit_scale=0.01), 92,
+               "MDF_MAX_LSTM = 4: three input GEMMs through the shared pre buffer; K tails of 20 and 12; cpg = 2"),
+    "h48_gc8": (dict(lstm_hidden=48, lstm_layers=3, lm_dim=52, gc_dims=(8,) * 8, fc_dim=24, n_terms=7, gc_activation="Relu",
+                     gc_bias=True, logit_scale=0.005), 93,
+                "MDF_MAX_GC = 8: eight pooled slices at offsets 0, 8 ... 56; Relu + bias; cpg = 3; 3 LSTM layers"),
+    "h80_cols": (dict(lstm_hidden=80, lm_dim=100, gc_dims=(516, 4), fc_dim=40, n_terms=5, logit_scale=0.03), 94,
+                 "cpg = 5; a second column pass with a 4-column remainder; K = 516 into the next layer"),
+    "h144_wide": (dict(lstm_hidden=144, lm_dim=64, gc_dims=(60, 1028), fc_dim=72, n_terms=24, logit_scale=0.02), 95,
+                  "cpg = 9; three column passes (1028 = 2 x 512 + 4)"),
+    "h496": (dict(lstm_hidden=496, lm_dim=36, gc_dims=(100, 200, 300), fc_dim=1000, n_terms=1943, logit_scale=0.03), 96,
+             "cpg = 31, 4 groups, 186 KiB of shared memory; the widest head (2C = 3886)"),
+    "h512_d1": (dict(lstm_hidden=512, lstm_layers=1, lm_dim=512, gc_dims=(256,), fc_dim=128, n_terms=64, logit_scale=0.03), 97,
+                "192 KiB of shared memory, the largest H; the embedding reads layer 1 directly"),
+    "h512_d4": (dict(lstm_hidden=512, lstm_layers=4, n_terms=489, logit_scale=0.02), 98,
+                "the deepest stack at the largest H, MF widths (E 1024, gc 512 x 3, F 1024)"),
+    "e_wide": (dict(lstm_hidden=64, lm_dim=2052, gc_dims=(2048,), fc_dim=64, n_terms=24, logit_scale=0.01), 99,
+               "a long-K X.W (K = 2052 = 128 x 16 + 4) with a K tail; E not a multiple of 128"),
+}
+# oracle/gcn_f64.MUTANTS -> the shapes whose batch must show it (tests/test_gcn_f64_simt_reference.py); "chunks" is the
+# batch-structure case of SIMT_CHUNKS
+SIMT_MUTANT_SHAPES = {
+    "slice_edge": ("h32_d4", "h80_cols", "h496"),
+    "gate_order": ("h16_min", "h512_d1"),
+    "one_bias": ("h16_min", "h48_gc8"),
+    "k_tail": ("h16_min", "h32_d4", "h80_cols", "e_wide"),
+    "col_tail": ("h80_cols", "h144_wide"),
+    "row31": ("h16_min", "h48_gc8"),
+    "pool_offset": ("h48_gc8", "h496"),
+    "depth_input": ("h32_d4", "h48_gc8", "h512_d4"),
+    "second_chunk_stale_h": ("chunks",),
+}
+SIMT_EXACT_LENGTHS = (1, 2, 31, 32, 33, 63, 64, 65, 127, 128, 129, 255, 256, 257, 511, 512, 513)
+SIMT_LONG = (1090, 1110)       # one protein of about 1,100 residues per shape
+# batch-structure case "chunks": H 512 (4 groups of 32 CTAs on 148 SMs), 300 proteins of lengths 1 ... 300: 75 per group,
+# 3 chunks of 32 proteins per time step, and the number of running proteins crosses the chunk boundaries as they end
+SIMT_CHUNKS = ("h512_d1", tuple(range(1, 301)))
+
+
+def simt_chunk_lengths():
+    """The chunks case's lengths in seeded shuffled order."""
+    import numpy as np
+    lengths = list(SIMT_CHUNKS[1])
+    np.random.default_rng(SIMT_SHAPES[SIMT_CHUNKS[0]][1]).shuffle(lengths)
+    return lengths
+# a batch of more than 65535 x 64 rows: the SGEMMs split it into launches of at most that many rows
+SIMT_MAX_ROWS = 65535 * 64
+
+# shapes mdf_model_create (or the loader, for the depths) must refuse: tag -> (GCNConfig kwargs, seed, message pattern)
+_R = dict(lm_dim=8, gc_dims=(8,), fc_dim=4, n_terms=2)
+SIMT_REFUSED = {
+    "h8": (dict(lstm_hidden=8, **_R), 101, r"LSTM hidden size 8 .*multiple of 16 from 16 to 512"),
+    "h24": (dict(lstm_hidden=24, **_R), 102, r"LSTM hidden size 24 .*multiple of 16 from 16 to 512"),
+    "h528": (dict(lstm_hidden=528, **_R), 103, r"LSTM hidden size 528 .*multiple of 16 from 16 to 512"),
+    "lstm5": (dict(lstm_hidden=16, lstm_layers=5, **_R), 104, r"5 LSTM layers: .*at most 4"),
+    "gc9": (dict(lstm_hidden=16, lm_dim=8, gc_dims=(4,) * 9, fc_dim=4, n_terms=2), 105, r"9 GraphConv layers: .*at most 8"),
+    "gc_w6": (dict(lstm_hidden=16, lm_dim=8, gc_dims=(8, 6), fc_dim=4, n_terms=2), 106,
+              r"GraphConv layer 2 has width 6: .*multiple of 4"),
+    "e6": (dict(lstm_hidden=16, lm_dim=6, gc_dims=(8,), fc_dim=4, n_terms=2), 107, r"embedding width 6: .*multiple of 4"),
+}
+
+# Bounds of the exact-fp32 engine, one per (stage, metric), shared with the CPU sensitivity test (every mutant of
+# oracle/gcn_f64.MUTANTS must exceed 10 x the bound of some stage on the shape that claims it).  "max" and "coh" are
+# tests/test_gpu_tc_shapes.py's definitions (normalised by the RMS of the stage's reference over the batch); ("pool", "coh")
+# applies to every GraphConv layer's pooled slice; scores are absolute.  The stage bounds are twice the worst value over
+# SIMT_SHAPES and the batch-structure cases of tests/test_gpu_simt_shapes.py, measured on an NVIDIA B200 (1000 W power
+# limit), rounded up; the scores keep the project's exact-fp32 tolerances.
+SIMT_BOUNDS = {                      # measured worst: value (case, protein length)
+    ("lstm1", "max"): 8.3e-6,        # 4.10e-6 (chunks, L 207)
+    ("lstm1", "coh"): 1.2e-6,        # 5.96e-7 (h512_d1, L 2)
+    ("lstm2", "max"): 1.2e-4,        # 5.80e-5 (h512_d4, L 161): the fourth H = 512 layer
+    ("lstm2", "coh"): 8.6e-6,        # 4.27e-6 (h512_d4, L 54)
+    ("x0", "max"): 3.3e-5,           # 1.61e-5 (h512_d4, L 161)
+    ("x0", "coh"): 4.7e-6,           # 2.33e-6 (h512_d4, L 65)
+    ("gc_last", "max"): 1.6e-5,      # 7.99e-6 (h512_d4, L 65)
+    ("gc_last", "coh"): 8.7e-6,      # 4.32e-6 (e_wide, L 1)
+    ("pool", "coh"): 8.7e-6,         # 4.32e-6 (e_wide, L 1)
+    ("scores", "abs"): 2e-5,         # L <= 513; 5.60e-6 (h512_d4, L 513)
+    ("scores_long", "abs"): 5e-5,    # L ~ 1100; 8.94e-6 (h512_d4, L 1090)
+}
+SIMT_LONG_MIN = 1000                 # proteins of at least this length are held to ("scores_long", "abs")
+
+
+def simt_bound(stage, metric, L=0):
+    """SIMT_BOUNDS entry of a stage_errors key (pool<l> -> pool; scores of a long protein -> scores_long)."""
+    if stage.startswith("pool"):
+        stage = "pool"
+    if stage == "scores" and L >= SIMT_LONG_MIN:
+        stage = "scores_long"
+    return SIMT_BOUNDS.get((stage, metric))
+
+
+def simt_shape_lengths(seed):
+    """The lengths of a SIMT_SHAPES case's batch: the 32-row block edges of SIMT_EXACT_LENGTHS, 15 random lengths in 1-400
+    and one of SIMT_LONG, in shuffled order."""
+    import numpy as np
+    rng = np.random.default_rng(seed)
+    lengths = list(SIMT_EXACT_LENGTHS) + [int(L) for L in rng.integers(1, 401, 15)] + [int(rng.integers(SIMT_LONG[0], SIMT_LONG[1] + 1))]
+    rng.shuffle(lengths)
+    return lengths
