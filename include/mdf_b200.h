@@ -194,6 +194,23 @@ int mdf_path_submit_ragged(mdf_model *model, int n,
                            const char *const *q_aln, const char *const *t_aln, const int *aln_len,
                            float thr2, int generated_contacts, float *scores, mdf_job **job);
 int mdf_path_wait(mdf_job *job);
+/* Alignment and prediction in one job: pair p is (query[p], target[p], coords[p]) - the GCN's query sequence (q_len[p] residues),
+ * its best-hit target sequence (t_len[p]) and the target's C-alpha coordinates (float32 [coord_rows[p], 3]).  The pairs are
+ * aligned on the device (global Needleman-Wunsch with affine gaps, exactly as mdf_nw_align: same matrix / alphabet / A <= 32 /
+ * gap rules, same scores and alignment strings) and the traceback writes the query-frame coordinate table of the contact-map
+ * stage directly - the result equals mdf_path_submit_ragged over the gapped strings insert_gaps (alignment.py:38-62) makes from
+ * that alignment.  Per pair the job also returns the NW score, the alignment length and the number of M columns (identity =
+ * n_match / aln_len); with `ops`, the alignment string of pair p at byte ops_off[p] (room for q_len[p] + t_len[p] columns),
+ * ops_len[p] columns.  A residue outside the matrix alphabet fails here, naming the pair; a query residue outside the GCN
+ * alphabet is reported by mdf_path_wait.  Job slots, asynchrony and mdf_path_wait as mdf_path_submit_ragged; the per-pair
+ * outputs are complete when mdf_path_wait returns. */
+int mdf_path_submit_pairs(mdf_model *model, int n,
+                          const char *const *query, const int *q_len, const char *const *target, const int *t_len,
+                          const float *const *coords, const int *coord_rows,
+                          const int8_t *matrix, const char *alphabet, int A, int gap_open, int gap_extend,
+                          float thr2, int generated_contacts, float *scores,
+                          int32_t *nw_score, int32_t *aln_len, int32_t *n_match,
+                          char *ops, const int64_t *ops_off, int *ops_len, mdf_job **job);
 
 /* Same path split into upload / run / fetch so that the compute can be timed with inputs
  * already resident in HBM (bench.py `value`). */
@@ -202,6 +219,18 @@ int mdf_batch_upload(mdf_ctx *ctx, int n,
                      const float *coords, const int64_t *coord_off,
                      const char *q_aln, const char *t_aln, const int64_t *aln_off,
                      mdf_batch **out);
+/* Resident form of mdf_path_submit_pairs: query p = seq[seq_off[p] .. seq_off[p+1]), target p = target[target_off[p] ..
+ * target_off[p+1]), coordinates p = rows coord_off[p] .. coord_off[p+1] of coords (float32 [*, 3]).  The pairs are aligned once,
+ * here; mdf_path_run / mdf_path_run_shared / mdf_batch_fetch / mdf_batch_unpack_dense then work on the batch as on any other.
+ * mdf_batch_fetch_alignment returns the per-pair outputs of the alignment (as mdf_path_submit_pairs; ops == NULL: none). */
+int mdf_batch_upload_pairs(mdf_ctx *ctx, int n,
+                           const char *seq, const int64_t *seq_off,
+                           const char *target, const int64_t *target_off,
+                           const float *coords, const int64_t *coord_off,
+                           const int8_t *matrix, const char *alphabet, int A, int gap_open, int gap_extend,
+                           mdf_batch **out);
+int mdf_batch_fetch_alignment(mdf_batch *batch, int32_t *nw_score, int32_t *aln_len, int32_t *n_match,
+                              char *ops, const int64_t *ops_off, int *ops_len);
 int mdf_batch_destroy(mdf_batch *batch);
 int mdf_path_run(mdf_model *model, mdf_batch *batch, float thr2, int generated_contacts);
 /* mdf_path_run that keeps what an earlier run on this batch computed and this head shares: the contact maps and degrees

@@ -105,10 +105,17 @@ def lib() -> C.CDLL:
                                        C.c_float, C.c_int, vp]
         L.mdf_path_submit.argtypes = [vp, C.c_int, vp, c_i64p, vp, c_i64p, vp, vp, c_i64p, C.c_float, C.c_int, vp, C.POINTER(vp)]
         L.mdf_path_submit_ragged.argtypes = [vp, C.c_int, vp, vp, vp, vp, vp, vp, vp, C.c_float, C.c_int, vp, C.POINTER(vp)]
+        L.mdf_path_submit_pairs.argtypes = [vp, C.c_int, vp, vp, vp, vp, vp, vp, vp, C.c_char_p, C.c_int, C.c_int, C.c_int,
+                                            C.c_float, C.c_int, vp, vp, vp, vp, vp, vp, vp, C.POINTER(vp)]
         L.mdf_path_wait.argtypes = [vp]
-        for name in ("mdf_path_submit", "mdf_path_submit_ragged", "mdf_path_wait"):
+        for name in ("mdf_path_submit", "mdf_path_submit_ragged", "mdf_path_submit_pairs", "mdf_path_wait"):
             getattr(L, name).restype = C.c_int
         L.mdf_batch_upload.argtypes = [vp, C.c_int, vp, c_i64p, vp, c_i64p, vp, vp, c_i64p, C.POINTER(vp)]
+        L.mdf_batch_upload_pairs.argtypes = [vp, C.c_int, vp, c_i64p, vp, c_i64p, vp, c_i64p, vp, C.c_char_p, C.c_int, C.c_int, C.c_int,
+                                             C.POINTER(vp)]
+        L.mdf_batch_fetch_alignment.argtypes = [vp, vp, vp, vp, vp, vp, vp]
+        for name in ("mdf_batch_upload_pairs", "mdf_batch_fetch_alignment"):
+            getattr(L, name).restype = C.c_int
         L.mdf_batch_destroy.argtypes = [vp]
         L.mdf_path_run.argtypes = [vp, vp, C.c_float, C.c_int]
         L.mdf_path_run_stages.argtypes = [vp, vp, C.c_float, C.c_int, C.c_int]
@@ -165,7 +172,8 @@ EXPORTED_SYMBOLS = [
     "mdf_batch_upload", "mdf_batch_destroy", "mdf_path_run", "mdf_path_run_stages", "mdf_path_run_shared",
     "mdf_batch_fetch_scores", "mdf_batch_fetch", "mdf_batch_scores_device", "mdf_batch_unpack_dense", "mdf_batch_invalidate",
     "mdf_cnn_model_create", "mdf_cnn_model_destroy", "mdf_cnn_forward", "mdf_cnn_upload", "mdf_cnn_run", "mdf_cnn_fetch",
-    "mdf_path_submit", "mdf_path_submit_ragged", "mdf_path_wait", "mdf_cmap_build_transfer_ragged",
+    "mdf_path_submit", "mdf_path_submit_ragged", "mdf_path_submit_pairs", "mdf_path_wait", "mdf_cmap_build_transfer_ragged",
+    "mdf_batch_upload_pairs", "mdf_batch_fetch_alignment",
     "mdf_pdb_calpha", "mdf_pdb_calpha_batch", "mdf_coords_cache_create", "mdf_coords_cache_open", "mdf_coords_cache_close",
     "mdf_coords_cache_size", "mdf_coords_cache_lookup", "mdf_coords_cache_entry",
     "mdf_nw_align",

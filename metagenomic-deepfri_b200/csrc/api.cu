@@ -8,6 +8,7 @@
 
 #include "cmap_kernels.cuh"
 #include "gcn.cuh"
+#include "nw_align.cuh"
 #include "tc_engine.cuh"
 
 namespace mdf {
@@ -348,8 +349,18 @@ struct Carver {   // sub-allocates one block; first pass (base == nullptr) only 
     }
 };
 
+// residue codes and alignment table of a pairs batch, in host memory its copies may read (pinned for jobs)
+struct PairInputs {
+    const NwPlan *plan;
+    const uint8_t *codes;       // plan->off[n] bytes
+    const NwPair *table;        // plan->pairs
+    const int8_t *matrix32;     // [32][32]
+    int A, open, ext;
+    bool ops;                   // also write the alignment strings
+};
+
 static void carve_batch(mdf_batch *b, Carver &c, size_t seq_bytes, size_t ncoord_rows, size_t aln_bytes,
-                        size_t packed_words, int G, int C)
+                        size_t packed_words, int G, int C, const PairInputs *pin)
 {
     const size_t n = b->n, T = (size_t)b->T;
     b->d_seq = c.take<char>(seq_bytes + 16);
@@ -372,6 +383,14 @@ static void carve_batch(mdf_batch *b, Carver &c, size_t seq_bytes, size_t ncoord
         b->d_scores = c.take<float>(n * (size_t)C + 1);
         b->out_G = G; b->out_C = C;
     }
+    if (pin) {
+        const size_t codes = (size_t)pin->plan->off[n];
+        b->d_nw_codes = c.take<uint8_t>(codes + 16);
+        b->d_nw_pairs = c.take<NwPair>(n + 1);
+        b->d_nw_matrix = c.take<int8_t>(1024);
+        b->d_nw_stats = c.take<int32_t>(3 * n + 1);
+        b->d_ops = pin->ops ? c.take<char>(codes + 16) : nullptr;
+    }
 }
 
 // Builds host metadata, allocates (cudaMalloc when `persistent`, arena otherwise) and uploads.
@@ -385,7 +404,8 @@ __global__ void fill_res_prot_kernel(int n, const int64_t *__restrict__ seq_off,
 
 static int batch_build(mdf_ctx *ctx, mdf_batch *b, bool persistent, int n, const char *seq, const int64_t *seq_off,
                        const float *coords, const int64_t *coord_off, const char *q_aln, const char *t_aln,
-                       const int64_t *aln_off, const uint32_t *packed_host, int G, int C, size_t extra_reserve, mdf_job *slot = nullptr)
+                       const int64_t *aln_off, const uint32_t *packed_host, int G, int C, size_t extra_reserve, mdf_job *slot = nullptr,
+                       const PairInputs *pin = nullptr)
 {
     MDF_REQUIRE(n >= 0 && seq_off && (n == 0 || seq), "batch: sequences missing");
     b->ctx = ctx;
@@ -413,17 +433,17 @@ static int batch_build(mdf_ctx *ctx, mdf_batch *b, bool persistent, int n, const
     b->has_structure = coords != nullptr;
     size_t ncoord = 0, alnb = 0;
     b->n_coord_rows = coords ? coord_off[n] : 0;
-    b->n_aln_cols = coords ? aln_off[n] : 0;
+    b->n_aln_cols = coords && !pin ? aln_off[n] : 0;
     if (b->has_structure) {
-        MDF_REQUIRE(coord_off && q_aln && t_aln && aln_off, "batch: structure inputs incomplete");
-        MDF_REQUIRE(coord_off[0] == 0 && aln_off[0] == 0, "batch: offsets must start at 0");
+        MDF_REQUIRE(coord_off && (pin || (q_aln && t_aln && aln_off)), "batch: structure inputs incomplete");
+        MDF_REQUIRE(coord_off[0] == 0 && (pin || aln_off[0] == 0), "batch: offsets must start at 0");
         ncoord = (size_t)coord_off[n];
-        alnb = (size_t)aln_off[n];
+        alnb = pin ? 0 : (size_t)aln_off[n];
         for (int p = 0; p < n; ++p)
-            MDF_REQUIRE(coord_off[p + 1] >= coord_off[p] && aln_off[p + 1] >= aln_off[p], "batch: offsets not monotone");
+            MDF_REQUIRE(coord_off[p + 1] >= coord_off[p] && (pin || aln_off[p + 1] >= aln_off[p]), "batch: offsets not monotone");
     }
     Carver measure;
-    carve_batch(b, measure, (size_t)b->T, ncoord, alnb, (size_t)b->h_packed_off[n], G, C);
+    carve_batch(b, measure, (size_t)b->T, ncoord, alnb, (size_t)b->h_packed_off[n], G, C, pin);
     const size_t bytes = measure.top + 512;
     char *base = nullptr;
     if (persistent) {
@@ -448,7 +468,7 @@ static int batch_build(mdf_ctx *ctx, mdf_batch *b, bool persistent, int n, const
     b->block = base;
     Carver carve;
     carve.base = base;
-    carve_batch(b, carve, (size_t)b->T, ncoord, alnb, (size_t)b->h_packed_off[n], G, C);
+    carve_batch(b, carve, (size_t)b->T, ncoord, alnb, (size_t)b->h_packed_off[n], G, C, pin);
     cudaStream_t s = ctx->stream;
     b->slot = slot;
     // small metadata: through the slot's pinned staging when there is one (asynchronous), else from the pageable vectors (+ sync below)
@@ -480,11 +500,23 @@ static int batch_build(mdf_ctx *ctx, mdf_batch *b, bool persistent, int n, const
         }
         if (ncoord) MDF_CUDA(cudaMemcpyAsync(b->d_coords, coords, ncoord * 3 * sizeof(float), cudaMemcpyHostToDevice, cs));
         MDF_CUDA(cudaMemcpyAsync(b->d_coord_off, coord_off, (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, cs));
-        if (alnb) {
-            MDF_CUDA(cudaMemcpyAsync(b->d_qaln, q_aln, alnb, cudaMemcpyHostToDevice, cs));
-            MDF_CUDA(cudaMemcpyAsync(b->d_taln, t_aln, alnb, cudaMemcpyHostToDevice, cs));
+        if (pin) {
+            // pairs: the residue codes and the alignment table travel with the coordinates; the alignment stage reads them
+            const size_t codes = (size_t)pin->plan->off[n];
+            if (codes) MDF_CUDA(cudaMemcpyAsync(b->d_nw_codes, pin->codes, codes, cudaMemcpyHostToDevice, cs));
+            if (n) MDF_CUDA(cudaMemcpyAsync(b->d_nw_pairs, pin->table, (size_t)n * sizeof(NwPair), cudaMemcpyHostToDevice, cs));
+            MDF_CUDA(cudaMemcpyAsync(b->d_nw_matrix, pin->matrix32, 1024, cudaMemcpyHostToDevice, cs));
+            b->pairs = b->aln_pending = true;
+            std::copy(pin->plan->cls_at, pin->plan->cls_at + 5, b->nw_cls_at);
+            b->nw_A = pin->A; b->nw_open = pin->open; b->nw_ext = pin->ext;
+            b->h_nw_off = pin->plan->off;
+        } else {
+            if (alnb) {
+                MDF_CUDA(cudaMemcpyAsync(b->d_qaln, q_aln, alnb, cudaMemcpyHostToDevice, cs));
+                MDF_CUDA(cudaMemcpyAsync(b->d_taln, t_aln, alnb, cudaMemcpyHostToDevice, cs));
+            }
+            MDF_CUDA(cudaMemcpyAsync(b->d_aln_off, aln_off, (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, cs));
         }
-        MDF_CUDA(cudaMemcpyAsync(b->d_aln_off, aln_off, (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, cs));
         if (cs != s) {
             MDF_CUDA(cudaEventRecord(ctx->copy_done, cs));
             b->copy_pending = true;
@@ -514,9 +546,14 @@ static int run_cmap(mdf_ctx *ctx, mdf_batch *b, float thr2, int gen)
         MDF_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->copy_done, 0));
         b->copy_pending = false;
     }
+    if (b->aln_pending) {                       // pairs batch: the alignment traceback writes the query frame
+        MDF_TRY(nw_frame_stage(ctx, b));
+        b->aln_pending = false;
+    }
     ProfScope ps(ctx, "cmap_build_transfer", ctx->profiling ? cmap_algorithmic_bytes(b, b->n_coord_rows, b->n_aln_cols) : 0.0);
-    MDF_TRY(launch_aln_transfer(ctx, b->n, b->d_qaln, b->d_taln, b->d_aln_off, b->d_seq_off, b->d_coords,
-                                b->d_coord_off, b->d_qc));
+    if (!b->pairs)
+        MDF_TRY(launch_aln_transfer(ctx, b->n, b->d_qaln, b->d_taln, b->d_aln_off, b->d_seq_off, b->d_coords,
+                                    b->d_coord_off, b->d_qc));
     return launch_cmap_pair(ctx, b->n, b->nwork, b->d_work, b->d_qc, b->d_seq_off, thr2, gen, 1, b->d_packed, b->d_packed_off);
 }
 
@@ -580,6 +617,92 @@ extern "C" int mdf_batch_upload(mdf_ctx *ctx, int n, const char *seq, const int6
         return r;
     }
     *out = b;
+    return MDF_OK;
+}
+
+// The resident form of mdf_path_submit_pairs: flat (query, target, coordinates) of n pairs; the alignment stage runs once here
+// (the query frame depends on neither the threshold, the generated contacts nor the head) and mdf_path_run* reuse the frame.
+static int align_uploaded(mdf_ctx *ctx, mdf_batch *b, const NwPlan &plan)
+{
+    ArenaScope scope(ctx);
+    MDF_TRY(ctx->reserve(plan.scratch_bytes() + 1024));
+    MDF_TRY(ctx->alloc_n(&b->d_nw_dir, (size_t)plan.dir_words + 4));
+    MDF_TRY(ctx->alloc_n(&b->d_nw_bnd, (size_t)plan.bnd_ints + 4));
+    MDF_TRY(nw_frame_stage(ctx, b));
+    MDF_CUDA(cudaStreamSynchronize(ctx->stream));
+    b->d_nw_dir = nullptr; b->d_nw_bnd = nullptr;
+    b->aln_pending = false;
+    return MDF_OK;
+}
+
+extern "C" int mdf_batch_upload_pairs(mdf_ctx *ctx, int n, const char *seq, const int64_t *seq_off, const char *target,
+                                      const int64_t *target_off, const float *coords, const int64_t *coord_off, const int8_t *matrix,
+                                      const char *alphabet, int A, int gap_open, int gap_extend, mdf_batch **out)
+{
+    MDF_REQUIRE(ctx && out && n >= 0 && matrix && alphabet && A > 0 && A <= 32, "mdf_batch_upload_pairs: bad arguments");
+    MDF_REQUIRE(seq_off && target_off && coord_off && coords, "mdf_batch_upload_pairs: input arrays missing");
+    MDF_REQUIRE(gap_open >= 0 && gap_extend >= 0 && gap_open < (1 << 20) && gap_extend < (1 << 20), "mdf_batch_upload_pairs: gap penalties out of range");
+    MDF_REQUIRE(seq_off[0] == 0 && target_off[0] == 0, "mdf_batch_upload_pairs: offsets must start at 0");
+    MDF_CUDA(cudaSetDevice(ctx->device));
+    std::vector<const char *> qp((size_t)n), tp((size_t)n);
+    std::vector<int> ql((size_t)n), tl((size_t)n);
+    for (int p = 0; p < n; ++p) {
+        const int64_t lq = seq_off[p + 1] - seq_off[p], lt = target_off[p + 1] - target_off[p];
+        MDF_REQUIRE(lq >= 0 && lt >= 0 && lq < (1 << 20) && lt < (1 << 20), "mdf_batch_upload_pairs: pair %d has an invalid length", p);
+        ql[p] = (int)lq; tl[p] = (int)lt;
+        qp[p] = seq ? seq + seq_off[p] : nullptr;
+        tp[p] = target ? target + target_off[p] : nullptr;
+    }
+    NwPlan plan;
+    MDF_TRY(nw_plan("mdf_batch_upload_pairs", n, qp.data(), ql.data(), tp.data(), tl.data(), &plan));
+    uint8_t lut[256];
+    nw_lut(alphabet, A, lut);
+    std::vector<uint8_t> codes((size_t)plan.off[(size_t)n] + 16);
+    for (int p = 0; p < n; ++p) {
+        char c = 0;
+        if (const int which = nw_encode_pair(lut, qp[p], ql[p], tp[p], tl[p], codes.data() + plan.off[p], &c))
+            return nw_bad_letter("mdf_batch_upload_pairs", p, which, c);
+    }
+    int8_t m32[1024];
+    nw_matrix32(matrix, A, m32);
+    const PairInputs pin{&plan, codes.data(), plan.pairs.data(), m32, A, gap_open, gap_extend, true};
+    mdf_batch *b = new mdf_batch();
+    int r = batch_build(ctx, b, true, n, seq, seq_off, coords, coord_off, nullptr, nullptr, nullptr, nullptr, 0, 0, 0, nullptr, &pin);
+    if (r == MDF_OK) r = align_uploaded(ctx, b, plan);
+    if (r != MDF_OK) {
+        cudaStreamSynchronize(ctx->stream);
+        if (b->owns_memory && b->block) cudaFree(b->block);
+        delete b;
+        return r;
+    }
+    *out = b;
+    return MDF_OK;
+}
+
+// Per-pair outputs of the alignment stage of a batch uploaded with mdf_batch_upload_pairs (see mdf_path_submit_pairs).
+extern "C" int mdf_batch_fetch_alignment(mdf_batch *b, int32_t *nw_score, int32_t *aln_len, int32_t *n_match, char *ops,
+                                         const int64_t *ops_off, int *ops_len)
+{
+    MDF_REQUIRE(b && b->ctx && nw_score && aln_len && n_match, "mdf_batch_fetch_alignment: bad arguments");
+    MDF_REQUIRE(b->pairs && b->owns_memory, "mdf_batch_fetch_alignment: needs a batch uploaded with mdf_batch_upload_pairs");
+    MDF_REQUIRE(!ops || (ops_off && ops_len), "mdf_batch_fetch_alignment: ops_off / ops_len missing");
+    const int n = b->n;
+    if (n == 0) return MDF_OK;
+    mdf_ctx *ctx = b->ctx;
+    MDF_CUDA(cudaSetDevice(ctx->device));
+    std::vector<int32_t> st((size_t)n * 3);
+    std::vector<char> h(ops ? (size_t)b->h_nw_off[n] : 0);
+    MDF_CUDA(cudaMemcpyAsync(st.data(), b->d_nw_stats, st.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    if (!h.empty()) MDF_CUDA(cudaMemcpyAsync(h.data(), b->d_ops, h.size(), cudaMemcpyDeviceToHost, ctx->stream));
+    MDF_CUDA(cudaStreamSynchronize(ctx->stream));
+    memcpy(nw_score, st.data(), (size_t)n * 4);
+    memcpy(aln_len, st.data() + n, (size_t)n * 4);
+    memcpy(n_match, st.data() + 2 * (size_t)n, (size_t)n * 4);
+    if (ops)
+        for (int p = 0; p < n; ++p) {
+            memcpy(ops + ops_off[p], h.data() + b->h_nw_off[p], (size_t)aln_len[p]);
+            ops_len[p] = aln_len[p];
+        }
     return MDF_OK;
 }
 
@@ -732,6 +855,7 @@ static int slot_acquire(mdf_ctx *ctx, mdf_job **out)
     sl->h_err[0] = sl->h_err[1] = 0;
     sl->rc = MDF_OK;
     sl->meta_top = 0;
+    sl->n_pairs = 0;
     *out = sl;
     return MDF_OK;
 }
@@ -787,7 +911,7 @@ static void slot_match_peer(mdf_ctx *ctx, mdf_job *sl)
 // enqueue everything for flat inputs (already where they may be read asynchronously: pinned slot memory or caller buffers)
 static int job_enqueue(mdf_model *m, mdf_job *sl, int n, const char *seq, const int64_t *seq_off, const float *coords,
                        const int64_t *coord_off, const char *q_aln, const char *t_aln, const int64_t *aln_off, float thr2, int gen,
-                       float *scores)
+                       float *scores, const PairInputs *pin = nullptr)
 {
     mdf_ctx *ctx = m->ctx;
     ArenaScope scope(ctx);
@@ -796,7 +920,12 @@ static int job_enqueue(mdf_model *m, mdf_job *sl, int n, const char *seq, const 
     const auto t0 = std::chrono::steady_clock::now();
     slot_meta_reserve(sl, n, n > 0 ? seq_off[n] : 0);
     int rc = batch_build(ctx, b, false, n, seq, seq_off, coords, coord_off, q_aln, t_aln, aln_off, nullptr, m->G, m->C,
-                         engine_workspace(m, n, seq_off), sl);
+                         engine_workspace(m, n, seq_off) + (pin ? pin->plan->scratch_bytes() + 1024 : 0), sl, pin);
+    if (rc == MDF_OK && pin) {
+        // alignment scratch (~1 byte per DP cell) from the arena, ahead of the engine stages; released in stream order
+        rc = ctx->alloc_n(&b->d_nw_dir, (size_t)pin->plan->dir_words + 4);
+        if (rc == MDF_OK) rc = ctx->alloc_n(&b->d_nw_bnd, (size_t)pin->plan->bnd_ints + 4);
+    }
     const auto t1 = std::chrono::steady_clock::now();
     if (rc == MDF_OK) rc = run_path(m, b, thr2, gen, 4, true);
     cudaStream_t out_stream = ctx->stream;
@@ -812,6 +941,9 @@ static int job_enqueue(mdf_model *m, mdf_job *sl, int n, const char *seq, const 
         }
         if (e == cudaSuccess) e = cudaMemcpyAsync(scores, b->d_scores, (size_t)n * m->C * sizeof(float), cudaMemcpyDeviceToHost, out_stream);
         if (e == cudaSuccess) e = cudaMemcpyAsync(sl->h_err, ctx->d_err + 2 + slot, sizeof(int), cudaMemcpyDeviceToHost, out_stream);
+        if (e == cudaSuccess && pin) e = cudaMemcpyAsync(sl->pin_stats, b->d_nw_stats, (size_t)n * 12, cudaMemcpyDeviceToHost, out_stream);
+        if (e == cudaSuccess && pin && pin->ops && b->h_nw_off[n])
+            e = cudaMemcpyAsync(sl->pin_ops, b->d_ops, (size_t)b->h_nw_off[n], cudaMemcpyDeviceToHost, out_stream);
         if (e != cudaSuccess) { set_error("mdf_path_submit: result copy failed: %s", cudaGetErrorString(e)); rc = MDF_ECUDA; }
     }
     if (rc != MDF_OK && ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);   // no input copy may outlive a failed call
@@ -906,6 +1038,95 @@ extern "C" int mdf_path_submit_ragged(mdf_model *m, int n, const char *const *se
     return MDF_OK;
 }
 
+// n (query, target, target coordinates) pairs as arrays of per-pair pointers: the pairs are aligned on the device (nw_align.cu) and
+// the traceback writes the query frame of the contact-map stage, then as mdf_path_submit_ragged.  Residues are encoded into
+// scoring-matrix codes by the packing threads; the caller's buffers are no longer needed on return.
+extern "C" int mdf_path_submit_pairs(mdf_model *m, int n, const char *const *query, const int *q_len, const char *const *target,
+                                     const int *t_len, const float *const *coords, const int *coord_rows, const int8_t *matrix,
+                                     const char *alphabet, int A, int gap_open, int gap_extend, float thr2, int gen, float *scores,
+                                     int32_t *nw_score, int32_t *aln_len, int32_t *n_match, char *ops, const int64_t *ops_off,
+                                     int *ops_len, mdf_job **job)
+{
+    MDF_REQUIRE(m && scores && nw_score && aln_len && n_match && job && n >= 0 && matrix && alphabet && A > 0 && A <= 32,
+                "mdf_path_submit_pairs: bad arguments");
+    MDF_REQUIRE(n == 0 || (query && q_len && target && t_len && coords && coord_rows), "mdf_path_submit_pairs: input arrays missing");
+    MDF_REQUIRE(!ops || (ops_off && ops_len), "mdf_path_submit_pairs: ops_off / ops_len missing");
+    MDF_REQUIRE(gap_open >= 0 && gap_extend >= 0 && gap_open < (1 << 20) && gap_extend < (1 << 20), "mdf_path_submit_pairs: gap penalties out of range");
+    mdf_ctx *ctx = m->ctx;
+    MDF_CUDA(cudaSetDevice(ctx->device));
+    NwPlan plan;
+    MDF_TRY(nw_plan("mdf_path_submit_pairs", n, query, q_len, target, t_len, &plan));
+    int64_t T = 0, R = 0;
+    for (int p = 0; p < n; ++p) {
+        MDF_REQUIRE(coord_rows[p] >= 0 && (coords[p] || coord_rows[p] == 0),
+                    "mdf_path_submit_pairs: protein %d has no coordinates (filter structure-less queries first)", p);
+        T += q_len[p]; R += coord_rows[p];
+    }
+    const int64_t NC = plan.off[(size_t)n];
+    mdf_job *sl = nullptr;
+    MDF_TRY(slot_acquire(ctx, &sl));
+    const size_t off_b = align_up((size_t)(n + 1) * 8, 256);
+    const size_t seq_at = 2 * off_b, crd_at = seq_at + align_up((size_t)T + 16, 256), code_at = crd_at + align_up((size_t)R * 12 + 16, 256),
+                 tab_at = code_at + align_up((size_t)NC + 16, 256), mat_at = tab_at + align_up((size_t)n * sizeof(NwPair) + 16, 256),
+                 stat_at = mat_at + 1024, ops_at = stat_at + align_up((size_t)n * 12 + 16, 256),
+                 total = ops_at + (ops ? align_up((size_t)NC + 16, 256) : 0);
+    MDF_TRY(slot_pinned(sl, total));
+    int64_t *so = (int64_t *)sl->pin, *co = (int64_t *)(sl->pin + off_b);
+    so[0] = co[0] = 0;
+    for (int p = 0; p < n; ++p) { so[p + 1] = so[p] + q_len[p]; co[p + 1] = co[p] + coord_rows[p]; }
+    char *pseq = sl->pin + seq_at;
+    float *pc = (float *)(sl->pin + crd_at);
+    uint8_t *pcode = (uint8_t *)(sl->pin + code_at);
+    uint8_t lut[256];
+    nw_lut(alphabet, A, lut);
+    struct Bad { int p = -1, which = 0; char c = 0; };
+    auto pack = [&](int lo, int hi, Bad *bad) {
+        for (int p = lo; p < hi; ++p) {
+            if (q_len[p]) memcpy(pseq + so[p], query[p], (size_t)q_len[p]);
+            if (coord_rows[p]) memcpy(pc + co[p] * 3, coords[p], (size_t)coord_rows[p] * 12);
+            char c = 0;
+            const int which = nw_encode_pair(lut, query[p], q_len[p], target[p], t_len[p], pcode + plan.off[p], &c);
+            if (which && bad->p < 0) { bad->p = p; bad->which = which; bad->c = c; }
+        }
+    };
+    const int nt = std::max(1, std::min(ctx->host_threads, n / 256));
+    std::vector<Bad> bad((size_t)nt);
+    if (nt == 1) pack(0, n, &bad[0]);
+    else {
+        // ranges of equal bytes, not equal pair counts
+        std::vector<std::thread> th;
+        const int64_t per = (T + R * 12 + NC) / nt + 1;
+        int lo = 0;
+        for (int k = 0; k < nt; ++k) {
+            int hi = lo;
+            if (k == nt - 1) hi = n;
+            else while (hi < n && (so[hi] + co[hi] * 12 + plan.off[hi]) < per * (k + 1)) ++hi;
+            if (hi > lo) th.emplace_back(pack, lo, hi, &bad[k]);
+            lo = hi;
+        }
+        for (auto &t : th) t.join();
+    }
+    for (const Bad &b : bad)           // the thread ranges ascend: the first one that met a bad letter holds the first bad pair
+        if (b.p >= 0) return nw_bad_letter("mdf_path_submit_pairs", b.p, b.which, b.c);
+    if (n) memcpy(sl->pin + tab_at, plan.pairs.data(), (size_t)n * sizeof(NwPair));
+    nw_matrix32(matrix, A, (int8_t *)(sl->pin + mat_at));
+    const PairInputs pin{&plan, pcode, (const NwPair *)(sl->pin + tab_at), (const int8_t *)(sl->pin + mat_at), A, gap_open, gap_extend,
+                         ops != nullptr};
+    sl->pin_stats = (int32_t *)(sl->pin + stat_at);
+    sl->pin_ops = ops ? sl->pin + ops_at : nullptr;
+    sl->out_stats[0] = nw_score; sl->out_stats[1] = aln_len; sl->out_stats[2] = n_match;
+    sl->out_ops = ops;
+    sl->out_ops_len = ops_len;
+    if (ops) { sl->out_ops_off.assign(ops_off, ops_off + n); sl->nw_off = plan.off; }
+    const int rc = job_enqueue(m, sl, n, pseq, so, pc, co, nullptr, nullptr, nullptr, thr2, gen, scores, &pin);
+    if (rc != MDF_OK) return rc;
+    sl->n_pairs = n;
+    sl->busy = true;
+    *job = sl;
+    slot_match_peer(ctx, sl);
+    return MDF_OK;
+}
+
 extern "C" int mdf_path_wait(mdf_job *job)
 {
     MDF_REQUIRE(job && job->ctx, "mdf_path_wait: job is NULL");
@@ -913,6 +1134,16 @@ extern "C" int mdf_path_wait(mdf_job *job)
     MDF_CUDA(cudaSetDevice(job->ctx->device));
     job->busy = false;
     MDF_CUDA(cudaEventSynchronize(job->done));
+    if (const int n = job->n_pairs) {
+        for (int k = 0; k < 3; ++k) memcpy(job->out_stats[k], job->pin_stats + (size_t)k * n, (size_t)n * 4);
+        if (job->out_ops)
+            for (int p = 0; p < n; ++p) {
+                const int len = job->out_stats[1][p];
+                memcpy(job->out_ops + job->out_ops_off[p], job->pin_ops + job->nw_off[p], (size_t)len);
+                job->out_ops_len[p] = len;
+            }
+        job->n_pairs = 0;
+    }
     const int e = job->h_err[0];
     if (e == 0) return MDF_OK;
     set_error("path: %s", e == MDF_DERR_BAD_RESIDUE ? "Invalid character in sequence"

@@ -70,6 +70,20 @@ struct mdf_batch {
     void *lm_cache = nullptr;    // [Tp x H] fp16 operand image of the last LSTM layer
     size_t lm_cache_bytes = 0;
     unsigned long long lm_hash = 0;
+    // pairs batches (mdf_batch_upload_pairs / mdf_path_submit_pairs): (query, target, coordinates) in, the query frame d_qc is
+    // written by the Needleman-Wunsch traceback (nw_align.cu) instead of the alignment transfer of gapped strings
+    bool pairs = false;
+    bool aln_pending = false;    // the alignment stage has not run yet (jobs: it runs at the head of the contact-map stage)
+    int nw_cls_at[5] = {0, 0, 0, 0, 0};
+    int nw_A = 0, nw_open = 0, nw_ext = 0;
+    uint8_t *d_nw_codes = nullptr;    // scoring-matrix codes, pair p at h_nw_off[p]: query, then target
+    void *d_nw_pairs = nullptr;       // NwPair table (nw_align.cuh)
+    int8_t *d_nw_matrix = nullptr;    // [32][32]
+    int32_t *d_nw_stats = nullptr;    // [3][n]: NW score, alignment length, M columns
+    char *d_ops = nullptr;            // alignment strings (when asked for), pair p at h_nw_off[p]
+    uint32_t *d_nw_dir = nullptr;     // direction-code / boundary scratch of the alignment stage (arena, set by the caller)
+    int32_t *d_nw_bnd = nullptr;
+    std::vector<int64_t> h_nw_off;
 };
 
 namespace mdf {

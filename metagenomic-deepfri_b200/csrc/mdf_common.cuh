@@ -62,6 +62,15 @@ struct mdf_job {
     // pinned staging for the small per-batch metadata (work lists, offsets, tile tables): copied from here the H2D copies are
     // truly asynchronous, so a submit never blocks on the previous job and the GPU does not idle between jobs
     char *meta = nullptr; size_t meta_bytes = 0, meta_top = 0;
+    // pairs jobs (mdf_path_submit_pairs): the per-pair outputs arrive in this slot's pinned block; mdf_path_wait copies them to
+    // the caller's arrays (ops of pair p from nw_off[p] to out_ops + out_ops_off[p])
+    int n_pairs = 0;
+    int32_t *pin_stats = nullptr;         // [3][n]
+    char *pin_ops = nullptr;
+    int32_t *out_stats[3] = {nullptr, nullptr, nullptr};
+    char *out_ops = nullptr;
+    int *out_ops_len = nullptr;
+    std::vector<int64_t> out_ops_off, nw_off;
     const void *stage(const void *src, size_t bytes)
     {
         const size_t at = (meta_top + 63) & ~(size_t)63;

@@ -19,7 +19,8 @@
 #include <algorithm>
 #include <vector>
 
-#include "mdf_common.cuh"
+#include "gcn.cuh"
+#include "nw_align.cuh"
 
 namespace mdf {
 
@@ -27,15 +28,6 @@ namespace {
 
 constexpr int NW_NEG = -1000000000;
 constexpr int NW_WARPS = 4;                 // warps (= pairs) per block
-
-struct NwPair {
-    int64_t q_off, t_off;                   // into the packed residue codes
-    int lq, lt;
-    int64_t dir_off;                        // uint32 words: panel-major, then row, lane, word
-    int64_t bnd_off;                        // int32: 2 * (lq + 1) boundary values (H, F of the panel's last column)
-    int64_t ops_off;                        // output bytes
-    int out;                                // index in the caller's order
-};
 
 template <int W>
 __global__ void __launch_bounds__(NW_WARPS * 32) nw_fill_kernel(int n, const NwPair *__restrict__ pairs, const uint8_t *__restrict__ codes,
@@ -147,43 +139,106 @@ __global__ void __launch_bounds__(NW_WARPS * 32) nw_fill_kernel(int n, const NwP
     }
 }
 
+// 4-bit code of cell (i, j) (1-based) as nw_fill_kernel<W> stored it: bits 0-1 source of H (0 diagonal, 1 E, 2 F), bit 2
+// "E was extended", bit 3 "F was extended"
+template <int W>
+__device__ __forceinline__ uint32_t nw_cell_code(const uint32_t *__restrict__ d, int lq, int i, int j)
+{
+    constexpr int WL = W >= 8 ? W / 8 : 1;
+    const int col = j - 1, panel = col / (32 * W), lane = (col / W) & 31, k = col % W;
+    const uint32_t word = d[(((int64_t)panel * lq + (i - 1)) * 32 + lane) * WL + (k >> 3)];
+    return (word >> (4 * (k & 7))) & 15u;
+}
+
+// Walks the codes of one pair back from (Lq, Lt) and calls step(op, i, j, c) for the c-th column from the END of the alignment;
+// (i, j) is the 1-based cell the column leaves: M / X consume query residue i - 1 and target residue j - 1, D query residue i - 1,
+// I target residue j - 1.  Returns the number of columns.  Both tracebacks go through here.
+template <int W, typename Step>
+__device__ __forceinline__ int nw_walk(const NwPair &pr, const uint8_t *__restrict__ codes, const uint32_t *__restrict__ dir, Step &&step)
+{
+    const uint8_t *q = codes + pr.q_off, *t = codes + pr.t_off;
+    const uint32_t *d = dir + pr.dir_off;
+    int i = pr.lq, j = pr.lt, cnt = 0, state = 0;
+    while (i > 0 || j > 0) {
+        char op;
+        if (i == 0) op = 'I';
+        else if (j == 0) op = 'D';
+        else {
+            const uint32_t code = nw_cell_code<W>(d, pr.lq, i, j);
+            if (state == 0) {
+                const uint32_t src = code & 3u;
+                if (src != 0u) { state = (int)src; continue; }
+                op = q[i - 1] == t[j - 1] ? 'M' : 'X';
+            } else if (state == 1) {
+                op = 'D';
+                state = (code & 4u) ? 1 : 0;
+            } else {
+                op = 'I';
+                state = (code & 8u) ? 2 : 0;
+            }
+        }
+        step(op, i, j, cnt++);
+        if (op != 'I') --i;
+        if (op != 'D') --j;
+    }
+    return cnt;
+}
+
+__device__ __forceinline__ void reverse_ops(char *out, int cnt)
+{
+    for (int a = 0, b = cnt - 1; a < b; ++a, --b) { const char c = out[a]; out[a] = out[b]; out[b] = c; }
+}
+
 template <int W>
 __global__ void nw_trace_kernel(int n, const NwPair *__restrict__ pairs, const uint8_t *__restrict__ codes, const uint32_t *__restrict__ dir,
                                 char *__restrict__ ops, int *__restrict__ ops_len)
 {
-    constexpr int WL = W >= 8 ? W / 8 : 1;
     const int pi = blockIdx.x * blockDim.x + threadIdx.x;
     if (pi >= n) return;
     const NwPair pr = pairs[pi];
-    const uint8_t *q = codes + pr.q_off, *t = codes + pr.t_off;
     char *out = ops + pr.ops_off;
-    int i = pr.lq, j = pr.lt, cnt = 0, state = 0;
-    const uint32_t *d = dir + pr.dir_off;
-    while (i > 0 || j > 0) {
-        if (i == 0) { out[cnt++] = 'I'; --j; continue; }
-        if (j == 0) { out[cnt++] = 'D'; --i; continue; }
-        const int col = j - 1, panel = col / (32 * W), lane = (col / W) & 31, k = col % W;
-        const uint32_t word = d[(((int64_t)panel * pr.lq + (i - 1)) * 32 + lane) * WL + (k >> 3)];
-        const uint32_t code = (word >> (4 * (k & 7))) & 15u;
-        if (state == 0) {
-            const uint32_t src = code & 3u;
-            if (src == 0u) { out[cnt++] = q[i - 1] == t[j - 1] ? 'M' : 'X'; --i; --j; }
-            else state = (int)src;
-        } else if (state == 1) {
-            out[cnt++] = 'D'; --i;
-            state = (code & 4u) ? 1 : 0;
-        } else {
-            out[cnt++] = 'I'; --j;
-            state = (code & 8u) ? 2 : 0;
-        }
-    }
-    for (int a = 0, b = cnt - 1; a < b; ++a, --b) { const char c = out[a]; out[a] = out[b]; out[b] = c; }
+    const int cnt = nw_walk<W>(pr, codes, dir, [&](char op, int, int, int c) { out[c] = op; });
+    reverse_ops(out, cnt);
     ops_len[pr.out] = cnt;
+}
+
+// The traceback of nw_trace_kernel writing the query-frame table of cmap_pair_tri_kernel instead of characters (what
+// aln_transfer_kernel derives from the gapped strings): a diagonal column puts target residue j - 1 (NaN xyz when the structure
+// has no such row) over query residue i - 1, a D column leaves query residue i - 1 unmapped with flag 1 (it spawns generated
+// contacts), an I column writes nothing.  The walk runs backwards, so no string is needed and none is reversed unless asked for.
+template <int W>
+__global__ void nw_trace_frame_kernel(int n, const NwPair *__restrict__ pairs, const uint8_t *__restrict__ codes,
+                                      const uint32_t *__restrict__ dir, NwTrace tr)
+{
+    const int pi = blockIdx.x * blockDim.x + threadIdx.x;
+    if (pi >= n) return;
+    const NwPair pr = pairs[pi];
+    const int64_t s0 = tr.seq_off[pr.out], c0 = tr.coord_off[pr.out];
+    const int nc = (int)(tr.coord_off[pr.out + 1] - c0);
+    const float qnan = __int_as_float(0x7fc00000);
+    char *out = tr.ops ? tr.ops + pr.ops_off : nullptr;
+    int matches = 0;
+    const int cnt = nw_walk<W>(pr, codes, dir, [&](char op, int i, int j, int c) {
+        if (out) out[c] = op;
+        if (op == 'I') return;
+        float4 v = make_float4(qnan, qnan, qnan, __int_as_float(op == 'D' ? 1 : 0));
+        if (op != 'D') {
+            matches += op == 'M';
+            if (j - 1 < nc) {
+                const float *x = tr.coords + (c0 + j - 1) * 3;
+                v.x = x[0]; v.y = x[1]; v.z = x[2];
+            }
+        }
+        tr.qc[s0 + i - 1] = v;
+    });
+    if (out) reverse_ops(out, cnt);
+    tr.aln_len[pr.out] = cnt;
+    tr.n_match[pr.out] = matches;
 }
 
 template <int W>
 int launch_class(mdf_ctx *ctx, int n, const NwPair *d_pairs, const uint8_t *d_codes, const int8_t *d_matrix, int A, int open, int ext,
-                 uint32_t *d_dir, int32_t *d_bnd, int32_t *d_scores, char *d_ops, int *d_len, bool full)
+                 uint32_t *d_dir, int32_t *d_bnd, int32_t *d_scores, const NwTrace &tr)
 {
     if (n <= 0) return MDF_OK;
     const size_t smem = 1024 + (size_t)NW_WARPS * A * 32 * W;
@@ -191,14 +246,108 @@ int launch_class(mdf_ctx *ctx, int n, const NwPair *d_pairs, const uint8_t *d_co
     MDF_CUDA(cudaFuncSetAttribute(fill, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     fill<<<cdiv(n, NW_WARPS), NW_WARPS * 32, smem, ctx->stream>>>(n, d_pairs, d_codes, d_matrix, A, open, ext, d_dir, d_bnd, d_scores);
     MDF_LAUNCH_CHECK(ctx);
-    if (full) {
-        nw_trace_kernel<W><<<cdiv(n, 64), 64, 0, ctx->stream>>>(n, d_pairs, d_codes, d_dir, d_ops, d_len);
+    if (tr.qc) {
+        nw_trace_frame_kernel<W><<<cdiv(n, 64), 64, 0, ctx->stream>>>(n, d_pairs, d_codes, d_dir, tr);
+        MDF_LAUNCH_CHECK(ctx);
+    } else if (tr.ops) {
+        nw_trace_kernel<W><<<cdiv(n, 64), 64, 0, ctx->stream>>>(n, d_pairs, d_codes, d_dir, tr.ops, tr.ops_len);
         MDF_LAUNCH_CHECK(ctx);
     }
     return MDF_OK;
 }
 
 }  // namespace
+
+int nw_plan(const char *who, int n, const char *const *query, const int *q_len, const char *const *target, const int *t_len, NwPlan *plan)
+{
+    for (int p = 0; p < n; ++p) {
+        MDF_REQUIRE(q_len[p] >= 0 && t_len[p] >= 0 && q_len[p] < (1 << 20) && t_len[p] < (1 << 20), "%s: pair %d has an invalid length", who, p);
+        MDF_REQUIRE((query[p] || !q_len[p]) && (target[p] || !t_len[p]), "%s: pair %d has a NULL sequence", who, p);
+    }
+    plan->off.assign((size_t)n + 1, 0);
+    std::vector<NwPair> cls[4];
+    int64_t dir_words = 0, bnd_ints = 0;
+    for (int p = 0; p < n; ++p) {
+        NwPair pr;
+        pr.lq = q_len[p]; pr.lt = t_len[p]; pr.out = p;
+        pr.q_off = plan->off[p];
+        pr.t_off = pr.q_off + pr.lq;
+        pr.ops_off = pr.q_off;
+        plan->off[(size_t)p + 1] = pr.t_off + pr.lt;
+        const int k = pr.lt <= 128 ? 0 : pr.lt <= 256 ? 1 : pr.lt <= 512 ? 2 : 3;
+        const int W = 4 << k, WL = W >= 8 ? W / 8 : 1;
+        const int panels = std::max(1, (pr.lt + 32 * W - 1) / (32 * W));
+        pr.dir_off = dir_words;
+        // score-only calls still write the codes (one code path); their storage is recycled pair after pair is NOT possible
+        // with concurrent warps, so it is sized for real
+        dir_words += (int64_t)panels * pr.lq * 32 * WL;
+        pr.bnd_off = bnd_ints;
+        bnd_ints += 2 * ((int64_t)pr.lq + 1);
+        cls[k].push_back(pr);
+    }
+    // longest first inside a class: the tail of the launch is made of short pairs
+    for (auto &c : cls) std::stable_sort(c.begin(), c.end(), [](const NwPair &a, const NwPair &b) { return (int64_t)a.lq * a.lt > (int64_t)b.lq * b.lt; });
+    plan->pairs.clear();
+    plan->cls_at[0] = 0;
+    for (int k = 0; k < 4; ++k) { plan->pairs.insert(plan->pairs.end(), cls[k].begin(), cls[k].end()); plan->cls_at[k + 1] = (int)plan->pairs.size(); }
+    plan->dir_words = dir_words;
+    plan->bnd_ints = bnd_ints;
+    return MDF_OK;
+}
+
+void nw_lut(const char *alphabet, int A, uint8_t lut[256])
+{
+    memset(lut, 255, 256);
+    for (int a = 0; a < A; ++a) lut[(unsigned char)alphabet[a]] = (uint8_t)a;
+}
+
+int nw_encode_pair(const uint8_t lut[256], const char *q, int lq, const char *t, int lt, uint8_t *dst, char *bad)
+{
+    for (int i = 0; i < lq; ++i)
+        if ((dst[i] = lut[(unsigned char)q[i]]) == 255) { *bad = q[i]; return 1; }
+    dst += lq;
+    for (int i = 0; i < lt; ++i)
+        if ((dst[i] = lut[(unsigned char)t[i]]) == 255) { *bad = t[i]; return 2; }
+    return 0;
+}
+
+int nw_bad_letter(const char *who, int p, int which, char c)
+{
+    set_error("%s: %s %d holds '%c', which is not in the scoring matrix alphabet", who, which == 1 ? "query" : "target", p, c);
+    return MDF_EINVAL;
+}
+
+void nw_matrix32(const int8_t *matrix, int A, int8_t out[1024])
+{
+    memset(out, 0, 1024);
+    for (int r = 0; r < A; ++r) for (int c = 0; c < A; ++c) out[r * 32 + c] = matrix[r * A + c];
+}
+
+int nw_launch(mdf_ctx *ctx, const int cls_at[5], const NwPair *d_pairs, const uint8_t *d_codes, const int8_t *d_matrix, int A, int open,
+              int ext, uint32_t *d_dir, int32_t *d_bnd, int32_t *d_scores, const NwTrace &tr)
+{
+    ProfScope ps(ctx, "nw_align", 0.0);
+    MDF_TRY(launch_class<4>(ctx, cls_at[1] - cls_at[0], d_pairs + cls_at[0], d_codes, d_matrix, A, open, ext, d_dir, d_bnd, d_scores, tr));
+    MDF_TRY(launch_class<8>(ctx, cls_at[2] - cls_at[1], d_pairs + cls_at[1], d_codes, d_matrix, A, open, ext, d_dir, d_bnd, d_scores, tr));
+    MDF_TRY(launch_class<16>(ctx, cls_at[3] - cls_at[2], d_pairs + cls_at[2], d_codes, d_matrix, A, open, ext, d_dir, d_bnd, d_scores, tr));
+    MDF_TRY(launch_class<32>(ctx, cls_at[4] - cls_at[3], d_pairs + cls_at[3], d_codes, d_matrix, A, open, ext, d_dir, d_bnd, d_scores, tr));
+    return MDF_OK;
+}
+
+int nw_frame_stage(mdf_ctx *ctx, mdf_batch *b)
+{
+    NwTrace tr;
+    tr.qc = b->d_qc;
+    tr.seq_off = b->d_seq_off;
+    tr.coords = b->d_coords;
+    tr.coord_off = b->d_coord_off;
+    tr.aln_len = b->d_nw_stats + b->n;
+    tr.n_match = b->d_nw_stats + 2 * (size_t)b->n;
+    tr.ops = b->d_ops;
+    return nw_launch(ctx, b->nw_cls_at, (const NwPair *)b->d_nw_pairs, b->d_nw_codes, b->d_nw_matrix, b->nw_A, b->nw_open, b->nw_ext,
+                     b->d_nw_dir, b->d_nw_bnd, b->d_nw_stats, tr);
+}
+
 }  // namespace mdf
 
 using namespace mdf;
@@ -220,83 +369,47 @@ extern "C" int mdf_nw_align(mdf_ctx *ctx, int n, const char *const *query, const
     if (n == 0) return MDF_OK;
     MDF_CUDA(cudaSetDevice(ctx->device));
     uint8_t lut[256];
-    memset(lut, 255, sizeof lut);
-    for (int a = 0; a < A; ++a) lut[(unsigned char)alphabet[a]] = (uint8_t)a;
-    // ---- pack + encode on the host, classify by target length
-    int64_t total = 0;
-    for (int p = 0; p < n; ++p) {
-        MDF_REQUIRE(q_len[p] >= 0 && t_len[p] >= 0 && q_len[p] < (1 << 20) && t_len[p] < (1 << 20), "mdf_nw_align: pair %d has an invalid length", p);
-        MDF_REQUIRE((query[p] || !q_len[p]) && (target[p] || !t_len[p]), "mdf_nw_align: pair %d has a NULL sequence", p);
-        total += q_len[p] + t_len[p];
-    }
+    nw_lut(alphabet, A, lut);
+    NwPlan plan;
+    MDF_TRY(nw_plan("mdf_nw_align", n, query, q_len, target, t_len, &plan));
+    const int64_t total = plan.off[(size_t)n];
+    // ---- encode on the host
     std::vector<uint8_t> h_codes((size_t)total + 16);
-    std::vector<NwPair> cls[4];
-    int64_t at = 0, dir_words = 0, bnd_ints = 0;
-    const bool full = ops != nullptr;
     for (int p = 0; p < n; ++p) {
-        NwPair pr;
-        pr.lq = q_len[p]; pr.lt = t_len[p]; pr.out = p;
-        pr.q_off = at;
-        for (int i = 0; i < pr.lq; ++i) {
-            const uint8_t c = lut[(unsigned char)query[p][i]];
-            MDF_REQUIRE(c != 255, "mdf_nw_align: query %d holds '%c', which is not in the scoring matrix alphabet", p, query[p][i]);
-            h_codes[(size_t)at++] = c;
-        }
-        pr.t_off = at;
-        for (int i = 0; i < pr.lt; ++i) {
-            const uint8_t c = lut[(unsigned char)target[p][i]];
-            MDF_REQUIRE(c != 255, "mdf_nw_align: target %d holds '%c', which is not in the scoring matrix alphabet", p, target[p][i]);
-            h_codes[(size_t)at++] = c;
-        }
-        const int k = pr.lt <= 128 ? 0 : pr.lt <= 256 ? 1 : pr.lt <= 512 ? 2 : 3;
-        const int W = 4 << k, WL = W >= 8 ? W / 8 : 1;
-        const int panels = std::max(1, (pr.lt + 32 * W - 1) / (32 * W));
-        pr.dir_off = dir_words;
-        // score-only calls still write the codes (one code path); their storage is recycled pair after pair is NOT possible
-        // with concurrent warps, so it is sized for real
-        dir_words += (int64_t)panels * pr.lq * 32 * WL;
-        pr.bnd_off = bnd_ints;
-        bnd_ints += 2 * ((int64_t)pr.lq + 1);
-        pr.ops_off = full ? ops_off[p] : 0;
-        cls[k].push_back(pr);
+        char bad = 0;
+        if (const int which = nw_encode_pair(lut, query[p], q_len[p], target[p], t_len[p], h_codes.data() + plan.off[p], &bad))
+            return nw_bad_letter("mdf_nw_align", p, which, bad);
     }
+    const bool full = ops != nullptr;
     int64_t ops_bytes = 0;
-    if (full)
+    if (full) {
+        for (auto &pr : plan.pairs) pr.ops_off = ops_off[pr.out];
         for (int p = 0; p < n; ++p) ops_bytes = std::max(ops_bytes, ops_off[p] + q_len[p] + t_len[p]);
-    // longest first inside a class: the tail of the launch is made of short pairs
-    for (auto &c : cls) std::stable_sort(c.begin(), c.end(), [](const NwPair &a, const NwPair &b) { return (int64_t)a.lq * a.lt > (int64_t)b.lq * b.lt; });
-    std::vector<NwPair> all;
-    int cls_at[5] = {0, 0, 0, 0, 0};
-    for (int k = 0; k < 4; ++k) { all.insert(all.end(), cls[k].begin(), cls[k].end()); cls_at[k + 1] = (int)all.size(); }
+    }
+    const auto &all = plan.pairs;
     ArenaScope scope(ctx);
-    MDF_TRY(ctx->reserve((size_t)total + 16 + all.size() * sizeof(NwPair) + 1024 + (size_t)dir_words * 4 + (size_t)bnd_ints * 4 + (size_t)n * 8 +
+    MDF_TRY(ctx->reserve((size_t)total + 16 + all.size() * sizeof(NwPair) + 1024 + plan.scratch_bytes() + (size_t)n * 8 +
                          (size_t)ops_bytes + (1 << 16)));
-    uint8_t *d_codes; NwPair *d_pairs; int8_t *d_matrix; uint32_t *d_dir; int32_t *d_bnd, *d_scores; char *d_ops = nullptr; int *d_len = nullptr;
+    uint8_t *d_codes; NwPair *d_pairs; int8_t *d_matrix; uint32_t *d_dir; int32_t *d_bnd, *d_scores;
+    NwTrace tr;
     MDF_TRY(ctx->alloc_n(&d_codes, (size_t)total + 16));
     MDF_TRY(ctx->alloc_n(&d_pairs, all.size()));
     MDF_TRY(ctx->alloc_n(&d_matrix, 1024));
-    MDF_TRY(ctx->alloc_n(&d_dir, (size_t)dir_words + 4));
-    MDF_TRY(ctx->alloc_n(&d_bnd, (size_t)bnd_ints + 4));
+    MDF_TRY(ctx->alloc_n(&d_dir, (size_t)plan.dir_words + 4));
+    MDF_TRY(ctx->alloc_n(&d_bnd, (size_t)plan.bnd_ints + 4));
     MDF_TRY(ctx->alloc_n(&d_scores, (size_t)n));
-    if (full) { MDF_TRY(ctx->alloc_n(&d_ops, (size_t)ops_bytes + 4)); MDF_TRY(ctx->alloc_n(&d_len, (size_t)n)); }
+    if (full) { MDF_TRY(ctx->alloc_n(&tr.ops, (size_t)ops_bytes + 4)); MDF_TRY(ctx->alloc_n(&tr.ops_len, (size_t)n)); }
     int8_t h_matrix[1024];
-    memset(h_matrix, 0, sizeof h_matrix);
-    for (int r = 0; r < A; ++r) for (int c = 0; c < A; ++c) h_matrix[r * 32 + c] = matrix[r * A + c];
+    nw_matrix32(matrix, A, h_matrix);
     cudaStream_t s = ctx->stream;
     MDF_CUDA(cudaMemcpyAsync(d_codes, h_codes.data(), (size_t)total, cudaMemcpyHostToDevice, s));
     MDF_CUDA(cudaMemcpyAsync(d_pairs, all.data(), all.size() * sizeof(NwPair), cudaMemcpyHostToDevice, s));
     MDF_CUDA(cudaMemcpyAsync(d_matrix, h_matrix, 1024, cudaMemcpyHostToDevice, s));
-    {
-        ProfScope ps(ctx, "nw_align", 0.0);
-        MDF_TRY(launch_class<4>(ctx, cls_at[1] - cls_at[0], d_pairs + cls_at[0], d_codes, d_matrix, A, gap_open, gap_extend, d_dir, d_bnd, d_scores, d_ops, d_len, full));
-        MDF_TRY(launch_class<8>(ctx, cls_at[2] - cls_at[1], d_pairs + cls_at[1], d_codes, d_matrix, A, gap_open, gap_extend, d_dir, d_bnd, d_scores, d_ops, d_len, full));
-        MDF_TRY(launch_class<16>(ctx, cls_at[3] - cls_at[2], d_pairs + cls_at[2], d_codes, d_matrix, A, gap_open, gap_extend, d_dir, d_bnd, d_scores, d_ops, d_len, full));
-        MDF_TRY(launch_class<32>(ctx, cls_at[4] - cls_at[3], d_pairs + cls_at[3], d_codes, d_matrix, A, gap_open, gap_extend, d_dir, d_bnd, d_scores, d_ops, d_len, full));
-    }
+    MDF_TRY(nw_launch(ctx, plan.cls_at, d_pairs, d_codes, d_matrix, A, gap_open, gap_extend, d_dir, d_bnd, d_scores, tr));
     MDF_CUDA(cudaMemcpyAsync(scores, d_scores, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
     if (full) {
-        MDF_CUDA(cudaMemcpyAsync(ops_len, d_len, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
-        if (ops_bytes) MDF_CUDA(cudaMemcpyAsync(ops, d_ops, (size_t)ops_bytes, cudaMemcpyDeviceToHost, s));
+        MDF_CUDA(cudaMemcpyAsync(ops_len, tr.ops_len, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
+        if (ops_bytes) MDF_CUDA(cudaMemcpyAsync(ops, tr.ops, (size_t)ops_bytes, cudaMemcpyDeviceToHost, s));
     }
     MDF_CUDA(cudaStreamSynchronize(s));
     return MDF_OK;

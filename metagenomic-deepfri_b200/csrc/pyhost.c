@@ -8,6 +8,7 @@
  * memory on worker threads with the GIL released.  No arithmetic happens here.
  *
  *   submit_ragged(fn_addr, model_addr, seqs, gapped_query, gapped_target, coords, thr2, gen, scores_addr) -> (rc, job_addr)
+ *   submit_pairs(fn_addr, model_addr, queries, targets, coords, matrix_addr, alphabet, ...) -> (rc, job_addr)
  *   pointers(strings) -> (bytes ptr-array, bytes len-array)      [used for the alignment / ingest entry points]
  *   cmap_ragged(fn_addr, ctx_addr, gapped_query, gapped_target, coords, thr2, gen, out_addr, out_words) -> (rc, packed_off, seq_off)
  *
@@ -47,6 +48,27 @@ static int text_of(PyObject *o, const char **ptr, Py_ssize_t *len, const char *w
     return -1;
 }
 
+/* data pointer and row count of coordinate item i (a C-contiguous float32 [rows, 3] buffer, kept in views[*nviews] until released) */
+static int coords_of(PyObject *c, Py_buffer *views, Py_ssize_t *nviews, Py_ssize_t i, const float **ptr, int *rows)
+{
+    Py_buffer *v = &views[*nviews];
+    if (PyObject_GetBuffer(c, v, PyBUF_C_CONTIGUOUS | PyBUF_FORMAT) < 0) {
+        PyErr_Clear();
+        PyErr_Format(PyExc_TypeError, "coords[%zd] is not a C-contiguous buffer", i);
+        return -1;
+    }
+    ++*nviews;
+    const char *f = v->format ? v->format : "";
+    if (*f == '<' || *f == '=' || *f == '@') ++f;
+    if (strcmp(f, "f") != 0 || v->itemsize != 4 || v->ndim != 2 || v->shape[1] != 3) {
+        PyErr_Format(PyExc_TypeError, "coords[%zd] is not a float32 array of shape (Lt, 3)", i);
+        return -1;
+    }
+    *ptr = (const float *)v->buf;
+    *rows = (int)v->shape[0];
+    return 0;
+}
+
 static PyObject *submit_ragged(PyObject *self, PyObject *args)
 {
     unsigned long long fn_addr, model_addr, scores_addr;
@@ -84,22 +106,7 @@ static PyObject *submit_ragged(PyObject *self, PyObject *args)
         if (lq != lt) { PyErr_Format(PyExc_ValueError, "alignment %zd: query and target alignments differ in length", i); goto done; }
         if (ls > INT32_MAX || lq > INT32_MAX) { PyErr_SetString(PyExc_OverflowError, "sequence too long"); goto done; }
         lseq[i] = (int)ls; laln[i] = (int)lq;
-        PyObject *c = PySequence_Fast_GET_ITEM(fc, i);
-        Py_buffer *v = &views[nviews];
-        if (PyObject_GetBuffer(c, v, PyBUF_C_CONTIGUOUS | PyBUF_FORMAT) < 0) {
-            PyErr_Clear();
-            PyErr_Format(PyExc_TypeError, "coords[%zd] is not a C-contiguous buffer", i);
-            goto done;
-        }
-        ++nviews;
-        const char *f = v->format ? v->format : "";
-        if (*f == '<' || *f == '=' || *f == '@') ++f;
-        if (strcmp(f, "f") != 0 || v->itemsize != 4 || v->ndim != 2 || v->shape[1] != 3) {
-            PyErr_Format(PyExc_TypeError, "coords[%zd] is not a float32 array of shape (Lt, 3)", i);
-            goto done;
-        }
-        pc[i] = (const float *)v->buf;
-        rows[i] = (int)v->shape[0];
+        if (coords_of(PySequence_Fast_GET_ITEM(fc, i), views, &nviews, i, &pc[i], &rows[i]) < 0) goto done;
     }
     {
         mdf_job *job = NULL;
@@ -115,6 +122,72 @@ done:
     for (Py_ssize_t i = 0; i < nviews; ++i) PyBuffer_Release(&views[i]);
     free(views); free(pseq); free(pq); free(pt); free(pc); free(lseq); free(laln); free(rows);
     Py_XDECREF(fs); Py_XDECREF(fq); Py_XDECREF(ft); Py_XDECREF(fc);
+    return result;
+}
+
+typedef int (*submit_pairs_fn)(mdf_model *, int, const char *const *, const int *, const char *const *, const int *, const float *const *,
+                               const int *, const int8_t *, const char *, int, int, int, float, int, float *, int32_t *, int32_t *, int32_t *,
+                               char *, const int64_t *, int *, mdf_job **);
+
+/* submit_pairs(fn_addr, model_addr, queries, targets, coords, matrix_addr, alphabet, gap_open, gap_extend, thr2, gen, scores_addr,
+ *              nw_score_addr, aln_len_addr, n_match_addr, ops_addr, ops_off_addr, ops_len_addr) -> (rc, job_addr)
+ * the pairs twin of submit_ragged: calls mdf_path_submit_pairs with the GIL released (ops_addr == 0: no alignment strings) */
+static PyObject *submit_pairs(PyObject *self, PyObject *args)
+{
+    unsigned long long fn_addr, model_addr, matrix_addr, scores_addr, nw_addr, len_addr, match_addr, ops_addr, ops_off_addr, ops_len_addr;
+    PyObject *queries, *targets, *coords;
+    const char *alphabet;
+    Py_ssize_t A;
+    int gap_open, gap_extend, gen;
+    double thr2;
+    if (!PyArg_ParseTuple(args, "KKOOOKy#iidiKKKKKKK", &fn_addr, &model_addr, &queries, &targets, &coords, &matrix_addr, &alphabet, &A,
+                          &gap_open, &gap_extend, &thr2, &gen, &scores_addr, &nw_addr, &len_addr, &match_addr, &ops_addr, &ops_off_addr,
+                          &ops_len_addr))
+        return NULL;
+    PyObject *fq = PySequence_Fast(queries, "queries must be a sequence"), *ft = NULL, *fc = NULL;
+    if (!fq) return NULL;
+    ft = PySequence_Fast(targets, "targets must be a sequence");
+    fc = ft ? PySequence_Fast(coords, "coords must be a sequence") : NULL;
+    const Py_ssize_t n = PySequence_Fast_GET_SIZE(fq);
+    const char **pq = NULL, **pt = NULL;
+    const float **pc = NULL;
+    int *lq = NULL, *lt = NULL, *rows = NULL;
+    Py_buffer *views = NULL;
+    Py_ssize_t nviews = 0;
+    PyObject *result = NULL;
+    if (!fc) goto done;
+    if (PySequence_Fast_GET_SIZE(ft) != n || PySequence_Fast_GET_SIZE(fc) != n) {
+        PyErr_SetString(PyExc_ValueError, "queries, targets and coords must have the same length");
+        goto done;
+    }
+    pq = malloc(sizeof(char *) * (n + 1)); pt = malloc(sizeof(char *) * (n + 1)); pc = malloc(sizeof(float *) * (n + 1));
+    lq = malloc(sizeof(int) * (n + 1)); lt = malloc(sizeof(int) * (n + 1)); rows = malloc(sizeof(int) * (n + 1));
+    views = calloc((size_t)n + 1, sizeof(Py_buffer));
+    if (!pq || !pt || !pc || !lq || !lt || !rows || !views) { PyErr_NoMemory(); goto done; }
+    for (Py_ssize_t i = 0; i < n; ++i) {
+        Py_ssize_t a, b;
+        if (text_of(PySequence_Fast_GET_ITEM(fq, i), &pq[i], &a, "queries", i) < 0) goto done;
+        if (text_of(PySequence_Fast_GET_ITEM(ft, i), &pt[i], &b, "targets", i) < 0) goto done;
+        if (a > INT32_MAX || b > INT32_MAX) { PyErr_SetString(PyExc_OverflowError, "sequence too long"); goto done; }
+        lq[i] = (int)a; lt[i] = (int)b;
+        if (coords_of(PySequence_Fast_GET_ITEM(fc, i), views, &nviews, i, &pc[i], &rows[i]) < 0) goto done;
+    }
+    {
+        mdf_job *job = NULL;
+        int rc;
+        submit_pairs_fn fn = (submit_pairs_fn)(uintptr_t)fn_addr;
+        Py_BEGIN_ALLOW_THREADS
+        rc = fn((mdf_model *)(uintptr_t)model_addr, (int)n, pq, lq, pt, lt, pc, rows, (const int8_t *)(uintptr_t)matrix_addr, alphabet, (int)A,
+                gap_open, gap_extend, (float)thr2, gen, (float *)(uintptr_t)scores_addr, (int32_t *)(uintptr_t)nw_addr,
+                (int32_t *)(uintptr_t)len_addr, (int32_t *)(uintptr_t)match_addr, (char *)(uintptr_t)ops_addr,
+                (const int64_t *)(uintptr_t)ops_off_addr, (int *)(uintptr_t)ops_len_addr, &job);
+        Py_END_ALLOW_THREADS
+        result = Py_BuildValue("iK", rc, (unsigned long long)(uintptr_t)job);
+    }
+done:
+    for (Py_ssize_t i = 0; i < nviews; ++i) PyBuffer_Release(&views[i]);
+    free(views); free(pq); free(pt); free(pc); free(lq); free(lt); free(rows);
+    Py_XDECREF(fq); Py_XDECREF(ft); Py_XDECREF(fc);
     return result;
 }
 
@@ -191,22 +264,7 @@ static PyObject *cmap_ragged(PyObject *self, PyObject *args)
         if (sizes_only) continue;
         if (text_of(PySequence_Fast_GET_ITEM(ft, i), &pt[i], &lt, "gapped_target", i) < 0) goto done;
         if (lq != lt) { PyErr_Format(PyExc_ValueError, "alignment %zd: query and target alignments differ in length", i); goto done; }
-        PyObject *c = PySequence_Fast_GET_ITEM(fc, i);
-        Py_buffer *v = &views[nviews];
-        if (PyObject_GetBuffer(c, v, PyBUF_C_CONTIGUOUS | PyBUF_FORMAT) < 0) {
-            PyErr_Clear();
-            PyErr_Format(PyExc_TypeError, "coords[%zd] is not a C-contiguous buffer", i);
-            goto done;
-        }
-        ++nviews;
-        const char *f = v->format ? v->format : "";
-        if (*f == '<' || *f == '=' || *f == '@') ++f;
-        if (strcmp(f, "f") != 0 || v->itemsize != 4 || v->ndim != 2 || v->shape[1] != 3) {
-            PyErr_Format(PyExc_TypeError, "coords[%zd] is not a float32 array of shape (Lt, 3)", i);
-            goto done;
-        }
-        pc[i] = (const float *)v->buf;
-        rows[i] = (int)v->shape[0];
+        if (coords_of(PySequence_Fast_GET_ITEM(fc, i), views, &nviews, i, &pc[i], &rows[i]) < 0) goto done;
     }
     {
         int rc;
@@ -229,6 +287,7 @@ done:
 static PyMethodDef methods[] = {
     {"cmap_ragged", cmap_ragged, METH_VARARGS, "collect per-alignment pointers and call mdf_cmap_build_transfer_ragged (GIL released)"},
     {"submit_ragged", submit_ragged, METH_VARARGS, "collect per-protein pointers and call mdf_path_submit_ragged (GIL released)"},
+    {"submit_pairs", submit_pairs, METH_VARARGS, "collect per-pair pointers and call mdf_path_submit_pairs (GIL released)"},
     {"pointers", pointers, METH_O, "pointer / length arrays of a list of str or bytes"},
     {NULL, NULL, 0, NULL}};
 

@@ -9,6 +9,9 @@ row per call.  Here the same rows come out of a few batched launches:
 * `predict_structures` is the fast path: alignments in, one score matrix per mode out.  A chunk of
   proteins is uploaded once; the contact maps are built once; the LSTM language model - identical in all
   four heads - runs once, and every further head only runs its embedding, GraphConv stack and classifier.
+* `predict_pairs` does the same from (query, best-hit target, target coordinates) pairs: the alignment step
+  (`align_mmseqs_results`, `alignment.py:266-322`) runs on the device once per chunk and its traceback builds the
+  contact-map input directly, so no alignment string or gapped sequence passes through Python.
 
 Nothing here falls back to the CPU; sequences without structure (`alignment.coords is None`,
 `bio_utils.py:381-383`) are reported back so the caller can route them to the sequence-only branch
@@ -96,3 +99,40 @@ def predict_structures(predictors: Dict[str, Predictor], alignments: Sequence, t
                 for a, vec in zip(part, out[mode][lo:hi]):
                     w.writerow([a.query_name, "gcn"] + vec.tolist())
     return out, kept, skipped
+
+
+def predict_pairs(predictors: Dict[str, Predictor], query_ids: Sequence[str], queries: Sequence[str], target_ids: Sequence[str],
+                  targets: Sequence[str], coords: Sequence[np.ndarray], scoring_matrix="VTML80", gap_open: int = 10, gap_extend: int = 1,
+                  threshold: float = 6, generated_contacts: int = 2, max_residues: int = DEFAULT_MAX_RESIDUES,
+                  writers: Optional[Dict[str, "csv.writer"]] = None):
+    """`predict_structures` from (query, best-hit target, target coordinates) pairs: `align_mmseqs_results` +
+    `build_align_contact_map` + `forward_pass` of every mode in `predictors` (all on one context).  Per chunk the pairs are
+    uploaded and aligned once (`Predictor.upload_pairs`), then every head runs on the batch with `share=True`.
+
+    Returns `(scores, stats)`: `scores[mode]` is float32 `[n, C_mode]` in input order; `stats` holds per pair the `target_id`,
+    the int32 `nw_score`, `aln_len` and `n_match` arrays and `identity` = n_match / aln_len (PyOpal's `identity()`).  With
+    `writers`, rows `[query_id, "gcn"] + scores` are written per mode in input order, as `pipeline.py:318-319` writes them."""
+    if not predictors:
+        raise ValueError("predict_pairs: no predictors")
+    n = len(queries)
+    if not len(query_ids) == len(target_ids) == len(targets) == len(coords) == n:
+        raise ValueError("predict_pairs: query_ids, queries, target_ids, targets and coords must have the same length")
+    first = next(iter(predictors.values()))
+    out = {mode: np.empty((n, p.n_terms), np.float32) for mode, p in predictors.items()}
+    stats = {k: np.empty(n, np.int32) for k in ("nw_score", "aln_len", "n_match")}
+    for lo, hi in _chunks([len(q) for q in queries], max_residues):
+        batch = first.upload_pairs(queries[lo:hi], targets[lo:hi], coords[lo:hi], scoring_matrix, gap_open, gap_extend)
+        try:
+            for mode, pred in predictors.items():
+                pred.run(batch, threshold, generated_contacts, share=True)   # maps and LM output come from the first head
+                pred.fetch_scores(batch, out[mode][lo:hi])
+            stats["nw_score"][lo:hi], stats["aln_len"][lo:hi], stats["n_match"][lo:hi] = batch.alignment()
+        finally:
+            batch.close()
+        if writers:
+            for mode, w in writers.items():
+                for qid, vec in zip(query_ids[lo:hi], out[mode][lo:hi]):
+                    w.writerow([qid, "gcn"] + vec.tolist())
+    stats["identity"] = np.where(stats["aln_len"] > 0, stats["n_match"] / np.maximum(stats["aln_len"], 1), 0.0)
+    stats["target_id"] = list(target_ids)
+    return out, stats

@@ -54,6 +54,17 @@ def _pack_checked(seqs: Sequence[str]):
     return b, off
 
 
+def _float32_coords(coords) -> list:
+    """Structures as C-contiguous float32 [Lt, 3] arrays, converted like the reference's astype(np.float32) (contact_map.py:25)."""
+    conv = []
+    for i, c in enumerate(coords):
+        c = np.ascontiguousarray(c, dtype=np.float32)
+        if c.ndim != 2 or c.shape[1] != 3:
+            raise ValueError(f"structure {i}: coordinates must have shape (Lt, 3)")
+        conv.append(c)
+    return conv
+
+
 def seq2onehot(seq: str) -> np.ndarray:
     """`predict.pyx:17-48`: float32 [L, 26] one-hot over "-DGULNTKHYWCPVSOIEFXQABZRM"."""
     b = _encode(seq)
@@ -173,6 +184,85 @@ class PathBatch:
             self.close()
         except Exception:
             pass
+
+
+class PairBatch(PathBatch):
+    """A `PathBatch` made from (query, target, coordinates) pairs (`mdf_batch_upload_pairs`): the pairs are aligned on the device
+    once, at upload, and the alignment traceback writes the query frame of the contact-map stage; `Predictor.run` / `fetch` /
+    `unpack_dense` work on it as on any uploaded batch."""
+
+    def __init__(self, ctx: _lib.Context, queries: Sequence[str], targets: Sequence[str], coords: Sequence[np.ndarray],
+                 scoring_matrix="VTML80", gap_open: int = 10, gap_extend: int = 1):
+        from .alignment import resolve_matrix
+        if not len(queries) == len(targets) == len(coords):
+            raise ValueError("queries, targets and coords must have the same length")
+        alphabet, m = resolve_matrix(scoring_matrix)
+        qs, ts = [q.upper() for q in queries], [t.upper() for t in targets]
+        seq_bytes, seq_off = _pack_checked(qs)
+        t_bytes = "".join(ts).encode("ascii")
+        t_off = np.zeros(len(ts) + 1, np.int64)
+        np.cumsum(np.fromiter(map(len, ts), np.int64, len(ts)), out=t_off[1:])
+        cs = _float32_coords(coords)
+        c_off = np.zeros(len(cs) + 1, np.int64)
+        np.cumsum(np.fromiter((c.shape[0] for c in cs), np.int64, len(cs)), out=c_off[1:])
+        flat = np.ascontiguousarray(np.concatenate(cs) if cs else np.zeros((0, 3), np.float32))
+        self.n = len(qs)
+        self.ctx = ctx
+        self.handle = None
+        h = C.c_void_p()
+        _lib.check(_lib.lib().mdf_batch_upload_pairs(
+            ctx.handle, self.n, seq_bytes, _lib.lp(seq_off), t_bytes, _lib.lp(t_off), flat.ctypes.data, _lib.lp(c_off),
+            m.ctypes.data, alphabet.encode("ascii"), len(alphabet), int(gap_open), int(gap_extend), C.byref(h)))
+        self.handle = h
+        self.seq_off = seq_off
+        self.packed_off = packed_offsets(np.diff(seq_off))
+        self._ops_off = np.zeros(self.n + 1, np.int64)
+        self._ops_off[1:] = seq_off[1:] + t_off[1:]
+        self.h2d_bytes = 2 * len(seq_bytes) + len(t_bytes) + flat.nbytes + 8 * (seq_off.size + c_off.size)   # queries: ASCII + codes
+
+    def alignment(self, ops: bool = False):
+        """Per pair: (int32 NW score, alignment length, M columns[, alignment strings over M / X / I / D])."""
+        stats = np.empty((3, self.n), np.int32)
+        buf = np.empty(int(self._ops_off[-1]) + 1, np.uint8) if ops else None
+        ops_len = np.empty(self.n, np.int32) if ops else None
+        _lib.check(_lib.lib().mdf_batch_fetch_alignment(
+            self.handle, stats[0].ctypes.data, stats[1].ctypes.data, stats[2].ctypes.data, buf.ctypes.data if ops else None,
+            self._ops_off.ctypes.data if ops else None, ops_len.ctypes.data if ops else None))
+        out = (stats[0], stats[1], stats[2])
+        return out + (_decode_ops(buf, self._ops_off, ops_len),) if ops else out
+
+
+def _decode_ops(buf: np.ndarray, off: np.ndarray, lens: np.ndarray) -> List[str]:
+    b = buf.tobytes()
+    return [b[off[p]:off[p] + lens[p]].decode("ascii") for p in range(len(lens))]
+
+
+class PairJob:
+    """An in-flight `Predictor.submit_pairs` call: `wait()` returns `(scores, nw_score, aln_len, n_match)`, plus the alignment
+    strings when they were asked for."""
+
+    def __init__(self, handle: Optional[int], out: np.ndarray, stats: np.ndarray, ops, queries):
+        self._handle, self._out, self._stats, self._ops, self._queries = handle, out, stats, ops, queries
+        self._result = None
+
+    def wait(self):
+        if self._handle is not None:
+            h, self._handle = self._handle, None
+            try:
+                _lib.check(_lib.lib().mdf_path_wait(C.c_void_p(h)))
+            except ValueError as e:
+                if "Invalid character" in str(e):      # name the residue the way the reference does (predict.pyx:45-46)
+                    for s in self._queries:
+                        _encode(s)
+                raise
+            finally:
+                self._queries = None
+        if self._result is None:
+            self._result = (self._out, self._stats[0], self._stats[1], self._stats[2])
+            if self._ops is not None:
+                buf, off, lens = self._ops
+                self._result += (_decode_ops(buf, off, lens),)
+        return self._result
 
 
 class PathJob:
@@ -337,15 +427,8 @@ class Predictor:
         try:
             rc, job = host.submit_ragged(*args, coords, *tail)
         except TypeError:
-            # some structure is not a C-contiguous float32 [Lt, 3] array (lists, float64 ...): convert like the reference's
-            # astype(np.float32) (contact_map.py:25) and retry once
-            conv = []
-            for i, c in enumerate(coords):
-                c = np.ascontiguousarray(c, dtype=np.float32)
-                if c.ndim != 2 or c.shape[1] != 3:
-                    raise ValueError(f"structure {i}: coordinates must have shape (Lt, 3)")
-                conv.append(c)
-            rc, job = host.submit_ragged(*args, conv, *tail)
+            # some structure is not a C-contiguous float32 [Lt, 3] array (lists, float64 ...): convert and retry once
+            rc, job = host.submit_ragged(*args, _float32_coords(coords), *tail)
         _lib.check(rc)
         return PathJob(self, job, out, (seqs, gapped_query, gapped_target))
 
@@ -355,6 +438,55 @@ class Predictor:
         """The whole path for n proteins (contact map build + alignment transfer + GCN), host
         buffers in, host scores out: what `pipeline.py:476-481` + `:301-319` compute together."""
         return self.submit_structures(seqs, gapped_query, gapped_target, coords, threshold, generated_contacts, out).wait()
+
+    def submit_pairs(self, queries: Sequence[str], targets: Sequence[str], coords: Sequence[np.ndarray], scoring_matrix="VTML80",
+                     gap_open: int = 10, gap_extend: int = 1, threshold: float = 6, generated_contacts: int = 2,
+                     out: Optional[np.ndarray] = None, alignments: bool = False) -> PairJob:
+        """Align and predict in one asynchronous job: pair p is (query, best-hit target sequence, target C-alpha coordinates).
+        The pairs are aligned on the device (global alignment as `alignment.nw_align`: same matrices, gap penalties, scores
+        and alignment strings; sequences upper-cased) and the traceback builds the contact-map input directly, so the result
+        equals `submit_structures(queries, *insert_gaps(query, target, ops), coords)` with no alignment string passing through
+        the host.  `job.wait()` returns `(scores, nw_score, aln_len, n_match)` - identity = n_match / aln_len - and the
+        alignment strings as a fifth item with `alignments=True`.  Jobs share the two slots of `submit_structures`."""
+        from .alignment import resolve_matrix
+        from .bio_utils import threshold_sq
+        self._require_gcn("submit_pairs")
+        n = len(queries)
+        if len(targets) != n or len(coords) != n:
+            raise ValueError("queries, targets and coords must have the same length")
+        if out is None:
+            out = np.empty((n, self.n_terms), np.float32)
+        if out.shape != (n, self.n_terms) or out.dtype != np.float32 or not out.flags["C_CONTIGUOUS"]:
+            raise ValueError("out must be a C-contiguous float32 array of shape (n, n_terms)")
+        alphabet, m = resolve_matrix(scoring_matrix)
+        qs, ts = [q.upper() for q in queries], [t.upper() for t in targets]
+        stats = np.empty((3, n), np.int32)
+        ops = None
+        if alignments:
+            off = np.zeros(n + 1, np.int64)
+            if n:
+                np.cumsum(np.fromiter((len(q) + len(t) for q, t in zip(qs, ts)), np.int64, n), out=off[1:])
+            ops = (np.empty(int(off[-1]) + 1, np.uint8), off, np.empty(n, np.int32))
+        if n == 0:
+            return PairJob(None, out, stats, ops, None)
+        host = _lib.pyhost()
+        head = (_lib.fn_addr("mdf_path_submit_pairs"), self._handle.value, qs, ts)
+        tail = (m.ctypes.data, alphabet.encode("ascii"), int(gap_open), int(gap_extend), float(threshold_sq(threshold)),
+                int(generated_contacts), out.ctypes.data, stats[0].ctypes.data, stats[1].ctypes.data, stats[2].ctypes.data,
+                *((ops[0].ctypes.data, ops[1].ctypes.data, ops[2].ctypes.data) if alignments else (0, 0, 0)))
+        try:
+            rc, job = host.submit_pairs(*head, coords, *tail)
+        except TypeError:
+            rc, job = host.submit_pairs(*head, _float32_coords(coords), *tail)
+        _lib.check(rc)
+        return PairJob(job, out, stats, ops, qs)
+
+    def forward_pairs(self, queries: Sequence[str], targets: Sequence[str], coords: Sequence[np.ndarray], scoring_matrix="VTML80",
+                      gap_open: int = 10, gap_extend: int = 1, threshold: float = 6, generated_contacts: int = 2,
+                      out: Optional[np.ndarray] = None, alignments: bool = False):
+        """`submit_pairs(...).wait()`."""
+        return self.submit_pairs(queries, targets, coords, scoring_matrix, gap_open, gap_extend, threshold, generated_contacts, out,
+                                 alignments).wait()
 
     def forward_inputs(self, inputs: PathInputs, threshold: float = 6, generated_contacts: int = 2,
                        out: Optional[np.ndarray] = None) -> np.ndarray:
@@ -374,6 +506,11 @@ class Predictor:
     def upload(self, seqs, gapped_query, gapped_target, coords) -> PathBatch:
         self._require_gcn("upload")
         return PathBatch(self._ctx, seqs, gapped_query, gapped_target, coords)
+
+    def upload_pairs(self, queries, targets, coords, scoring_matrix="VTML80", gap_open: int = 10, gap_extend: int = 1) -> PairBatch:
+        """Resident form of `submit_pairs`: aligns once at upload; `run(batch, ..., share=True)` then serves every head."""
+        self._require_gcn("upload_pairs")
+        return PairBatch(self._ctx, queries, targets, coords, scoring_matrix, gap_open, gap_extend)
 
     def run(self, batch: PathBatch, threshold: float = 6, generated_contacts: int = 2, upto: int = 4,
             share: bool = False) -> None:
