@@ -58,6 +58,26 @@ def pack_structures(gapped_query: Sequence[str], gapped_target: Sequence[str],
                             seq_off, packed_offsets(lens))
 
 
+def float32_coords(coords) -> list:
+    """Structures as C-contiguous float32 [Lt, 3] arrays, converted like the reference's astype(np.float32) (contact_map.py:25)."""
+    conv = []
+    for i, c in enumerate(coords):
+        c = np.ascontiguousarray(c, dtype=np.float32)
+        if c.ndim != 2 or c.shape[1] != 3:
+            raise ValueError(f"structure {i}: coordinates must have shape (Lt, 3)")
+        conv.append(c)
+    return conv
+
+
+def with_float32_coords(call, coords):
+    """`call(coords)` into the CPython glue, which takes structures only as C-contiguous float32 [Lt, 3] arrays and raises
+    TypeError for any other (lists, float64 ...): then once more with every structure converted by `float32_coords`."""
+    try:
+        return call(coords)
+    except TypeError:
+        return call(float32_coords(coords))
+
+
 def pack_sequences(seqs: Sequence[str]):
     sb = [s.encode("ascii") for s in seqs]
     off = np.zeros(len(sb) + 1, np.int64)

@@ -13,7 +13,7 @@ from typing import List, Optional, Sequence, Tuple
 import numpy as np
 
 from . import _lib
-from .batching import pack_structures
+from .batching import pack_structures, with_float32_coords
 from .contact_map_utils import pairwise_sqeuclidean
 
 logger = logging.getLogger(__name__)
@@ -86,15 +86,8 @@ def _packed_ragged(gq: Sequence[str], gt: Sequence[str], coords: Sequence[np.nda
         buf = arena
     else:
         buf = np.empty(total, np.uint32)
-    try:
-        rc, _, _ = host.cmap_ragged(fn, ctx.handle.value, gq, gt, coords, thr, gen, buf.ctypes.data, buf.size)
-    except TypeError:
-        # some structure is not a C-contiguous float32 [Lt, 3] array: convert like the reference's astype (contact_map.py:25)
-        conv = [np.ascontiguousarray(c, dtype=np.float32) for c in coords]
-        for i, c in enumerate(conv):
-            if c.ndim != 2 or c.shape[1] != 3:
-                raise ValueError(f"structure {i}: coordinates must have shape (Lt, 3)")
-        rc, _, _ = host.cmap_ragged(fn, ctx.handle.value, gq, gt, conv, thr, gen, buf.ctypes.data, buf.size)
+    rc, _, _ = with_float32_coords(lambda cs: host.cmap_ragged(fn, ctx.handle.value, gq, gt, cs, thr, gen, buf.ctypes.data, buf.size),
+                                   coords)
     _lib.check(rc)
     return buf, packed_off, seq_off
 

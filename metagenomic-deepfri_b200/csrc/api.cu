@@ -3,6 +3,7 @@
 #include <functional>
 #include <stdarg.h>
 #include <algorithm>
+#include <atomic>
 #include <numeric>
 #include <thread>
 
@@ -359,11 +360,24 @@ struct PairInputs {
     bool ops;                   // also write the alignment strings
 };
 
-static void carve_batch(mdf_batch *b, Carver &c, size_t seq_bytes, size_t ncoord_rows, size_t aln_bytes,
-                        size_t packed_words, int G, int C, const PairInputs *pin)
+// What a batch is built from, in host memory its copies may read (pinned for jobs).  A structure batch has coordinates and either
+// the alignment strings or, for pairs, `pairs`; a batch without coordinates may bring its contact maps packed.  G / C size the
+// pooled features and scores (0: allocated by the first run); `extra_reserve` is arena room kept above the batch for its run.
+struct BatchInputs {
+    int n = 0;
+    const char *seq = nullptr;    const int64_t *seq_off = nullptr;
+    const float *coords = nullptr; const int64_t *coord_off = nullptr;
+    const char *q_aln = nullptr, *t_aln = nullptr; const int64_t *aln_off = nullptr;
+    const PairInputs *pairs = nullptr;
+    const uint32_t *packed = nullptr;
+    int G = 0, C = 0;
+    size_t extra_reserve = 0;
+};
+
+static void carve_batch(mdf_batch *b, Carver &c, size_t ncoord_rows, size_t aln_bytes, const BatchInputs &in)
 {
     const size_t n = b->n, T = (size_t)b->T;
-    b->d_seq = c.take<char>(seq_bytes + 16);
+    b->d_seq = c.take<char>(T + 16);
     b->d_seq_off = c.take<int64_t>(n + 1);
     b->d_coords = c.take<float>(ncoord_rows * 3 + 4);
     b->d_coord_off = c.take<int64_t>(n + 1);
@@ -375,15 +389,15 @@ static void carve_batch(mdf_batch *b, Carver &c, size_t seq_bytes, size_t ncoord
     b->d_order = c.take<int>(n + 1);
     b->d_res_prot = c.take<int>(T + 1);
     b->d_qc = c.take<float4>(T + 1);
-    b->d_packed = c.take<uint32_t>(packed_words + 4);
+    b->d_packed = c.take<uint32_t>((size_t)b->h_packed_off[n] + 4);
     b->d_deg = c.take<float>(T + 1);
     b->d_idx = c.take<uint8_t>(T + 16);
-    if (G > 0) {
-        b->d_pooled = c.take<float>(n * (size_t)G + 1);
-        b->d_scores = c.take<float>(n * (size_t)C + 1);
-        b->out_G = G; b->out_C = C;
+    if (in.G > 0) {
+        b->d_pooled = c.take<float>(n * (size_t)in.G + 1);
+        b->d_scores = c.take<float>(n * (size_t)in.C + 1);
+        b->out_G = in.G; b->out_C = in.C;
     }
-    if (pin) {
+    if (const PairInputs *pin = in.pairs) {
         const size_t codes = (size_t)pin->plan->off[n];
         b->d_nw_codes = c.take<uint8_t>(codes + 16);
         b->d_nw_pairs = c.take<NwPair>(n + 1);
@@ -393,7 +407,133 @@ static void carve_batch(mdf_batch *b, Carver &c, size_t seq_bytes, size_t ncoord
     }
 }
 
-// Builds host metadata, allocates (cudaMalloc when `persistent`, arena otherwise) and uploads.
+// ------------------------------------------------------------------------------------------- host staging
+// Grow-only block of pinned host or device memory: when `need` bytes do not fit, it is freed and `size` bytes are allocated (default:
+// `need` + 25 % headroom in 2 MiB steps).  On failure the block is left empty and the (cleared) CUDA error is returned.
+static size_t with_headroom(size_t need) { return align_up(need + need / 4, 2u << 20); }
+static cudaError_t grow_block(char *&p, size_t &cap, size_t need, bool device, size_t size = 0)
+{
+    if (cap >= need) return cudaSuccess;
+    if (!size) size = with_headroom(need);
+    cudaError_t e = !p ? cudaSuccess : device ? cudaFree(p) : cudaFreeHost(p);
+    p = nullptr; cap = 0;
+    if (e == cudaSuccess) e = device ? cudaMalloc((void **)&p, size) : cudaHostAlloc((void **)&p, size, cudaHostAllocDefault);
+    if (e != cudaSuccess) { cudaGetLastError(); p = nullptr; return e; }
+    cap = size;
+    return cudaSuccess;
+}
+
+static int pinned_block(char *&p, size_t &cap, size_t need, const char *what)
+{
+    const cudaError_t e = grow_block(p, cap, need, false);
+    if (e != cudaSuccess) { set_error("cudaHostAlloc(%zu bytes)%s failed: %s", with_headroom(need), what, cudaGetErrorString(e)); return MDF_ENOMEM; }
+    return MDF_OK;
+}
+
+// threads that pack an n-item batch: MDF_HOST_THREADS (default 4), at most one per 256 items
+static int pack_threads(const mdf_ctx *ctx, int n) { return std::max(1, std::min(ctx ? ctx->host_threads : 4, n / 256)); }
+
+// Runs fn(lo, hi) on nt threads over consecutive ranges of [0, n) that hold equal bytes (item p: bytes(p)), not equal item counts.
+template <typename Bytes, typename Fn>
+static void run_split(int n, int nt, Bytes bytes, Fn fn)
+{
+    if (nt <= 1) { fn(0, n); return; }
+    int64_t total = 0, before = 0;              // before: bytes of the items in front of `hi`
+    for (int p = 0; p < n; ++p) total += bytes(p);
+    const int64_t per = total / nt + 1;
+    std::vector<std::thread> th;
+    for (int k = 0, lo = 0, hi = 0; k < nt; ++k, lo = hi) {
+        if (k == nt - 1) hi = n;
+        else while (hi < n && before < per * (k + 1)) before += bytes(hi++);
+        if (hi > lo) th.emplace_back(fn, lo, hi);
+    }
+    for (auto &t : th) t.join();
+}
+
+// n ragged host items packed into one block.  A column holds, for item p, rows off[p] .. off[p + 1) of `row` bytes (coordinates:
+// 12) copied from src[p]; its int64 [n + 1] offsets go into the block, one array for all columns with the same `len`.  A column
+// given offsets instead of lengths is filled by the hook of pack(); a region has neither and is left to the caller (or is an output
+// the job writes).  Every part is 256-byte aligned with 16 bytes of slack.
+struct RaggedPack {
+    struct Col { const int *len; const int64_t *off; size_t row; const void *const *src; size_t bytes; char *at; };
+    int n;
+    std::vector<Col> cols;
+
+    explicit RaggedPack(int n_) : n(n_) {}
+    template <typename T>
+    int column(const int *len, size_t row, const T *const *src)
+    {
+        int64_t rows = 0;
+        for (int p = 0; p < n; ++p) rows += len[p];
+        return add({len, nullptr, row, reinterpret_cast<const void *const *>(src), (size_t)rows * row, nullptr});
+    }
+    int column(const int64_t *off) { return add({nullptr, off, 1, nullptr, (size_t)off[n], nullptr}); }
+    int region(size_t bytes) { return add({nullptr, nullptr, 0, nullptr, bytes, nullptr}); }
+    int add(const Col &col) { cols.push_back(col); return (int)cols.size() - 1; }
+    char *at(int c) const { return cols[c].at; }
+    const int64_t *off(int c) const { return cols[c].off; }
+
+    // Lays the block out from `base` and fills the offset arrays; with base == nullptr only measures.  Returns the block's bytes.
+    size_t place(char *base)
+    {
+        Carver carve;
+        carve.base = base;
+        for (size_t c = 0; c < cols.size(); ++c) {
+            Col &col = cols[c];
+            size_t same = 0;
+            while (col.len && same < c && cols[same].len != col.len) ++same;
+            if (col.len && same < c) col.off = cols[same].off;
+            else if (col.len) {
+                int64_t *o = carve.take<int64_t>((size_t)n + 1);
+                if (o) { o[0] = 0; for (int p = 0; p < n; ++p) o[p + 1] = o[p] + col.len[p]; }
+                col.off = o;
+            }
+            col.at = carve.take<char>(col.bytes + 16);
+        }
+        return carve.top;
+    }
+
+    // Copies every item into the placed block on nt threads; hook(p), when given, runs after the copies of item p and returns
+    // false for a bad item, which ends its thread's range.  Returns the lowest bad item over all threads, or -1.
+    int pack(int nt, const std::function<bool(int)> &hook = {})
+    {
+        std::atomic<int> bad(n);
+        auto bytes = [&](int p) {
+            int64_t b = 0;
+            for (const Col &col : cols) if (col.off) b += (col.off[p + 1] - col.off[p]) * (int64_t)col.row;
+            return b;
+        };
+        run_split(n, nt, bytes, [&](int lo, int hi) {
+            for (int p = lo; p < hi; ++p) {
+                for (const Col &col : cols)
+                    if (col.src && col.len[p]) memcpy(col.at + col.off[p] * col.row, col.src[p], (size_t)col.len[p] * col.row);
+                if (hook && !hook(p)) {
+                    for (int first = bad.load(); p < first && !bad.compare_exchange_weak(first, p);) {}
+                    return;
+                }
+            }
+        });
+        return bad < n ? bad.load() : -1;
+    }
+};
+
+// Packs `pk` with, as its hook, the residues of pair p encoded into scoring-matrix codes at column `codes` + plan.off[p]; a letter
+// outside the alphabet fails with the message of nw_bad_letter for the first bad pair.
+static int pack_pairs(const char *who, RaggedPack &pk, int codes, int nt, const NwPlan &plan, const char *alphabet, int A,
+                      const char *const *query, const int *q_len, const char *const *target, const int *t_len)
+{
+    uint8_t lut[256];
+    nw_lut(alphabet, A, lut);
+    uint8_t *dst = (uint8_t *)pk.at(codes);
+    auto encode = [&](int p, char *c) { return nw_encode_pair(lut, query[p], q_len[p], target[p], t_len[p], dst + plan.off[p], c); };
+    const int bad = pk.pack(nt, [&](int p) { char c; return encode(p, &c) == 0; });
+    if (bad < 0) return MDF_OK;
+    char c = 0;
+    const int which = encode(bad, &c);
+    return nw_bad_letter(who, bad, which, c);
+}
+
+// Builds host metadata, allocates (cudaMalloc when `persistent`, the slot's block for a job, arena otherwise) and uploads.
 __global__ void fill_res_prot_kernel(int n, const int64_t *__restrict__ seq_off, int *__restrict__ res_prot)
 {
     for (int p = blockIdx.x; p < n; p += gridDim.x) {
@@ -402,12 +542,12 @@ __global__ void fill_res_prot_kernel(int n, const int64_t *__restrict__ seq_off,
     }
 }
 
-static int batch_build(mdf_ctx *ctx, mdf_batch *b, bool persistent, int n, const char *seq, const int64_t *seq_off,
-                       const float *coords, const int64_t *coord_off, const char *q_aln, const char *t_aln,
-                       const int64_t *aln_off, const uint32_t *packed_host, int G, int C, size_t extra_reserve, mdf_job *slot = nullptr,
-                       const PairInputs *pin = nullptr)
+static int batch_build(mdf_ctx *ctx, mdf_batch *b, bool persistent, const BatchInputs &in, mdf_job *slot = nullptr)
 {
-    MDF_REQUIRE(n >= 0 && seq_off && (n == 0 || seq), "batch: sequences missing");
+    const int n = in.n;
+    const int64_t *seq_off = in.seq_off, *coord_off = in.coord_off, *aln_off = in.aln_off;
+    const PairInputs *pin = in.pairs;
+    MDF_REQUIRE(n >= 0 && seq_off && (n == 0 || in.seq), "batch: sequences missing");
     b->ctx = ctx;
     b->n = n;
     b->h_seq_off.assign(seq_off, seq_off + n + 1);
@@ -430,12 +570,12 @@ static int batch_build(mdf_ctx *ctx, mdf_batch *b, bool persistent, int n, const
     std::stable_sort(b->h_order.begin(), b->h_order.end(), [&](int x, int y) {
         return (b->h_seq_off[x + 1] - b->h_seq_off[x]) > (b->h_seq_off[y + 1] - b->h_seq_off[y]);
     });
-    b->has_structure = coords != nullptr;
+    b->has_structure = in.coords != nullptr;
     size_t ncoord = 0, alnb = 0;
-    b->n_coord_rows = coords ? coord_off[n] : 0;
-    b->n_aln_cols = coords && !pin ? aln_off[n] : 0;
+    b->n_coord_rows = in.coords ? coord_off[n] : 0;
+    b->n_aln_cols = in.coords && !pin ? aln_off[n] : 0;
     if (b->has_structure) {
-        MDF_REQUIRE(coord_off && (pin || (q_aln && t_aln && aln_off)), "batch: structure inputs incomplete");
+        MDF_REQUIRE(coord_off && (pin || (in.q_aln && in.t_aln && aln_off)), "batch: structure inputs incomplete");
         MDF_REQUIRE(coord_off[0] == 0 && (pin || aln_off[0] == 0), "batch: offsets must start at 0");
         ncoord = (size_t)coord_off[n];
         alnb = pin ? 0 : (size_t)aln_off[n];
@@ -443,7 +583,7 @@ static int batch_build(mdf_ctx *ctx, mdf_batch *b, bool persistent, int n, const
             MDF_REQUIRE(coord_off[p + 1] >= coord_off[p] && (pin || aln_off[p + 1] >= aln_off[p]), "batch: offsets not monotone");
     }
     Carver measure;
-    carve_batch(b, measure, (size_t)b->T, ncoord, alnb, (size_t)b->h_packed_off[n], G, C, pin);
+    carve_batch(b, measure, ncoord, alnb, in);
     const size_t bytes = measure.top + 512;
     char *base = nullptr;
     if (persistent) {
@@ -451,35 +591,26 @@ static int batch_build(mdf_ctx *ctx, mdf_batch *b, bool persistent, int n, const
         b->owns_memory = true;
     } else if (slot) {
         // job slot: a device block of its own, so the inputs of this job may arrive while the previous job still computes
-        if (slot->dev_bytes < bytes) {
-            if (slot->dev) MDF_CUDA(cudaFree(slot->dev));
-            slot->dev = nullptr; slot->dev_bytes = 0;
-            const size_t want = align_up(bytes + bytes / 4, 2u << 20);
-            cudaError_t e = cudaMalloc((void **)&slot->dev, want);
-            if (e != cudaSuccess) { cudaGetLastError(); set_error("cudaMalloc(%zu bytes) for a job slot failed: %s", want, cudaGetErrorString(e)); return MDF_ENOMEM; }
-            slot->dev_bytes = want;
+        if (const cudaError_t e = grow_block(slot->dev, slot->dev_bytes, bytes, true)) {
+            set_error("cudaMalloc(%zu bytes) for a job slot failed: %s", with_headroom(bytes), cudaGetErrorString(e));
+            return MDF_ENOMEM;
         }
-        MDF_TRY(ctx->reserve(extra_reserve));
+        MDF_TRY(ctx->reserve(in.extra_reserve));
         base = slot->dev;
     } else {
-        MDF_TRY(ctx->reserve(bytes + extra_reserve));
+        MDF_TRY(ctx->reserve(bytes + in.extra_reserve));
         MDF_TRY(ctx->alloc((void **)&base, bytes));
     }
     b->block = base;
     Carver carve;
     carve.base = base;
-    carve_batch(b, carve, (size_t)b->T, ncoord, alnb, (size_t)b->h_packed_off[n], G, C, pin);
+    carve_batch(b, carve, ncoord, alnb, in);
     cudaStream_t s = ctx->stream;
     b->slot = slot;
     // small metadata: through the slot's pinned staging when there is one (asynchronous), else from the pageable vectors (+ sync below)
     bool staged = slot != nullptr;
-    auto src_of = [&](const void *p, size_t bytes) -> const void * {
-        if (!staged) return p;
-        const void *q = slot->stage(p, bytes);
-        if (!q) { staged = false; return p; }
-        return q;
-    };
-    if (b->T) MDF_CUDA(cudaMemcpyAsync(b->d_seq, seq, (size_t)b->T, cudaMemcpyHostToDevice, s));
+    auto src_of = [&](const void *p, size_t bytes) { return mdf_job::src_of(slot, p, bytes, &staged); };
+    if (b->T) MDF_CUDA(cudaMemcpyAsync(b->d_seq, in.seq, (size_t)b->T, cudaMemcpyHostToDevice, s));
     MDF_CUDA(cudaMemcpyAsync(b->d_seq_off, src_of(b->h_seq_off.data(), (n + 1) * sizeof(int64_t)), (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, s));
     MDF_CUDA(cudaMemcpyAsync(b->d_packed_off, src_of(b->h_packed_off.data(), (n + 1) * sizeof(int64_t)), (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, s));
     if (b->nwork) MDF_CUDA(cudaMemcpyAsync(b->d_work, src_of(work.data(), work.size() * sizeof(int2)), work.size() * sizeof(int2), cudaMemcpyHostToDevice, s));
@@ -498,7 +629,7 @@ static int batch_build(mdf_ctx *ctx, mdf_batch *b, bool persistent, int n, const
             MDF_CUDA(cudaEventRecord(ctx->copy_done, s));
             MDF_CUDA(cudaStreamWaitEvent(cs, ctx->copy_done, 0));
         }
-        if (ncoord) MDF_CUDA(cudaMemcpyAsync(b->d_coords, coords, ncoord * 3 * sizeof(float), cudaMemcpyHostToDevice, cs));
+        if (ncoord) MDF_CUDA(cudaMemcpyAsync(b->d_coords, in.coords, ncoord * 3 * sizeof(float), cudaMemcpyHostToDevice, cs));
         MDF_CUDA(cudaMemcpyAsync(b->d_coord_off, coord_off, (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, cs));
         if (pin) {
             // pairs: the residue codes and the alignment table travel with the coordinates; the alignment stage reads them
@@ -512,8 +643,8 @@ static int batch_build(mdf_ctx *ctx, mdf_batch *b, bool persistent, int n, const
             b->h_nw_off = pin->plan->off;
         } else {
             if (alnb) {
-                MDF_CUDA(cudaMemcpyAsync(b->d_qaln, q_aln, alnb, cudaMemcpyHostToDevice, cs));
-                MDF_CUDA(cudaMemcpyAsync(b->d_taln, t_aln, alnb, cudaMemcpyHostToDevice, cs));
+                MDF_CUDA(cudaMemcpyAsync(b->d_qaln, in.q_aln, alnb, cudaMemcpyHostToDevice, cs));
+                MDF_CUDA(cudaMemcpyAsync(b->d_taln, in.t_aln, alnb, cudaMemcpyHostToDevice, cs));
             }
             MDF_CUDA(cudaMemcpyAsync(b->d_aln_off, aln_off, (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, cs));
         }
@@ -521,8 +652,8 @@ static int batch_build(mdf_ctx *ctx, mdf_batch *b, bool persistent, int n, const
             MDF_CUDA(cudaEventRecord(ctx->copy_done, cs));
             b->copy_pending = true;
         }
-    } else if (packed_host && b->h_packed_off[n]) {
-        MDF_CUDA(cudaMemcpyAsync(b->d_packed, packed_host, (size_t)b->h_packed_off[n] * 4, cudaMemcpyHostToDevice, s));
+    } else if (in.packed && b->h_packed_off[n]) {
+        MDF_CUDA(cudaMemcpyAsync(b->d_packed, in.packed, (size_t)b->h_packed_off[n] * 4, cudaMemcpyHostToDevice, s));
     }
     // pageable sources (work / order vectors) must be consumed before they go out of scope; pinned staging needs no wait
     if (!staged) MDF_CUDA(cudaStreamSynchronize(s));
@@ -610,10 +741,10 @@ extern "C" int mdf_batch_upload(mdf_ctx *ctx, int n, const char *seq, const int6
     MDF_CUDA(cudaSetDevice(ctx->device));
     mdf_batch *b = new mdf_batch();
     // pooled / scores depend on the model head: allocated lazily by the first run
-    int r = batch_build(ctx, b, true, n, seq, seq_off, coords, coord_off, q_aln, t_aln, aln_off, nullptr, 0, 0, 0);
+    const int r = batch_build(ctx, b, true, {.n = n, .seq = seq, .seq_off = seq_off, .coords = coords, .coord_off = coord_off,
+                                             .q_aln = q_aln, .t_aln = t_aln, .aln_off = aln_off});
     if (r != MDF_OK) {
-        if (b->owns_memory && b->block) cudaFree(b->block);
-        delete b;
+        mdf_batch_destroy(b);
         return r;
     }
     *out = b;
@@ -655,24 +786,20 @@ extern "C" int mdf_batch_upload_pairs(mdf_ctx *ctx, int n, const char *seq, cons
     }
     NwPlan plan;
     MDF_TRY(nw_plan("mdf_batch_upload_pairs", n, qp.data(), ql.data(), tp.data(), tl.data(), &plan));
-    uint8_t lut[256];
-    nw_lut(alphabet, A, lut);
-    std::vector<uint8_t> codes((size_t)plan.off[(size_t)n] + 16);
-    for (int p = 0; p < n; ++p) {
-        char c = 0;
-        if (const int which = nw_encode_pair(lut, qp[p], ql[p], tp[p], tl[p], codes.data() + plan.off[p], &c))
-            return nw_bad_letter("mdf_batch_upload_pairs", p, which, c);
-    }
+    RaggedPack pk(n);
+    const int codes = pk.column(plan.off.data());
+    std::vector<char> block(pk.place(nullptr));
+    pk.place(block.data());
+    MDF_TRY(pack_pairs("mdf_batch_upload_pairs", pk, codes, pack_threads(ctx, n), plan, alphabet, A, qp.data(), ql.data(), tp.data(),
+                       tl.data()));
     int8_t m32[1024];
     nw_matrix32(matrix, A, m32);
-    const PairInputs pin{&plan, codes.data(), plan.pairs.data(), m32, A, gap_open, gap_extend, true};
+    const PairInputs pin{&plan, (const uint8_t *)pk.at(codes), plan.pairs.data(), m32, A, gap_open, gap_extend, true};
     mdf_batch *b = new mdf_batch();
-    int r = batch_build(ctx, b, true, n, seq, seq_off, coords, coord_off, nullptr, nullptr, nullptr, nullptr, 0, 0, 0, nullptr, &pin);
+    int r = batch_build(ctx, b, true, {.n = n, .seq = seq, .seq_off = seq_off, .coords = coords, .coord_off = coord_off, .pairs = &pin});
     if (r == MDF_OK) r = align_uploaded(ctx, b, plan);
     if (r != MDF_OK) {
-        cudaStreamSynchronize(ctx->stream);
-        if (b->owns_memory && b->block) cudaFree(b->block);
-        delete b;
+        mdf_batch_destroy(b);
         return r;
     }
     *out = b;
@@ -860,31 +987,6 @@ static int slot_acquire(mdf_ctx *ctx, mdf_job **out)
     return MDF_OK;
 }
 
-// room for the metadata of an n-protein / T-residue batch in the slot's pinned staging (only grows while the slot is idle)
-static int slot_meta_reserve(mdf_job *sl, int n, int64_t T)
-{
-    const size_t want = (size_t)n * 96 + (size_t)T + (2u << 20);
-    if (sl->meta_bytes >= want) return MDF_OK;
-    if (sl->meta) MDF_CUDA(cudaFreeHost(sl->meta));
-    sl->meta = nullptr; sl->meta_bytes = 0;
-    cudaError_t e = cudaHostAlloc((void **)&sl->meta, want + want / 4, cudaHostAllocDefault);
-    if (e != cudaSuccess) { cudaGetLastError(); return MDF_OK; }      // without it the copies fall back to pageable sources + a sync
-    sl->meta_bytes = want + want / 4;
-    return MDF_OK;
-}
-
-static int slot_pinned(mdf_job *sl, size_t bytes)
-{
-    if (sl->pin_bytes >= bytes) return MDF_OK;
-    if (sl->pin) MDF_CUDA(cudaFreeHost(sl->pin));
-    sl->pin = nullptr; sl->pin_bytes = 0;
-    const size_t want = align_up(bytes + bytes / 4, 2u << 20);
-    cudaError_t e = cudaHostAlloc((void **)&sl->pin, want, cudaHostAllocDefault);
-    if (e != cudaSuccess) { cudaGetLastError(); set_error("cudaHostAlloc(%zu bytes) for a job slot failed: %s", want, cudaGetErrorString(e)); return MDF_ENOMEM; }
-    sl->pin_bytes = want;
-    return MDF_OK;
-}
-
 // After a job has been enqueued from slot `sl`, bring the idle peer slot to the same buffer sizes while the GPU is busy with that
 // job: page-locking ~100 MB and a first cudaMalloc cost 50-75 ms of host time, which the second job of a stream of chunks would
 // otherwise pay in front of an idle GPU.
@@ -892,35 +994,28 @@ static void slot_match_peer(mdf_ctx *ctx, mdf_job *sl)
 {
     mdf_job *peer = &ctx->slots[(sl - ctx->slots) ^ 1];
     if (peer->busy || (peer->done && cudaEventQuery(peer->done) != cudaSuccess)) { cudaGetLastError(); return; }
-    if (peer->pin_bytes < sl->pin_bytes) {
-        if (peer->pin) cudaFreeHost(peer->pin);
-        peer->pin = nullptr; peer->pin_bytes = 0;
-        if (cudaHostAlloc((void **)&peer->pin, sl->pin_bytes, cudaHostAllocDefault) == cudaSuccess) peer->pin_bytes = sl->pin_bytes;
-    }
-    if (peer->meta_bytes < sl->meta_bytes) {
-        if (peer->meta) cudaFreeHost(peer->meta);
-        peer->meta = nullptr; peer->meta_bytes = 0;
-        if (cudaHostAlloc((void **)&peer->meta, sl->meta_bytes, cudaHostAllocDefault) == cudaSuccess) peer->meta_bytes = sl->meta_bytes;
-    }
-    if (peer->dev_bytes < sl->dev_bytes && peer->dev == nullptr) {     // (growing an existing block would need a cudaFree = a device sync)
-        if (cudaMalloc((void **)&peer->dev, sl->dev_bytes) == cudaSuccess) peer->dev_bytes = sl->dev_bytes;
-    }
-    cudaGetLastError();
+    grow_block(peer->pin, peer->pin_bytes, sl->pin_bytes, false, sl->pin_bytes);
+    grow_block(peer->meta, peer->meta_bytes, sl->meta_bytes, false, sl->meta_bytes);
+    if (!peer->dev)                     // (growing an existing block would need a cudaFree = a device sync)
+        grow_block(peer->dev, peer->dev_bytes, sl->dev_bytes, true, sl->dev_bytes);
 }
 
-// enqueue everything for flat inputs (already where they may be read asynchronously: pinned slot memory or caller buffers)
-static int job_enqueue(mdf_model *m, mdf_job *sl, int n, const char *seq, const int64_t *seq_off, const float *coords,
-                       const int64_t *coord_off, const char *q_aln, const char *t_aln, const int64_t *aln_off, float thr2, int gen,
-                       float *scores, const PairInputs *pin = nullptr)
+// enqueue everything for flat inputs (already where they may be read asynchronously: pinned slot memory or caller buffers) and
+// hand the slot out as *job
+static int job_enqueue(mdf_model *m, mdf_job *sl, BatchInputs in, float thr2, int gen, float *scores, mdf_job **job)
 {
     mdf_ctx *ctx = m->ctx;
     ArenaScope scope(ctx);
     mdf_batch *b = sl->batch;
+    const int n = in.n;
+    const PairInputs *pin = in.pairs;
     static const bool timing = getenv("MDF_TIMING") != nullptr;       // host-side breakdown of one call on stderr
     const auto t0 = std::chrono::steady_clock::now();
-    slot_meta_reserve(sl, n, n > 0 ? seq_off[n] : 0);
-    int rc = batch_build(ctx, b, false, n, seq, seq_off, coords, coord_off, q_aln, t_aln, aln_off, nullptr, m->G, m->C,
-                         engine_workspace(m, n, seq_off) + (pin ? pin->plan->scratch_bytes() + 1024 : 0), sl, pin);
+    // pinned staging of the small metadata; without it the copies fall back to pageable sources + a synchronise
+    grow_block(sl->meta, sl->meta_bytes, (size_t)n * 96 + (size_t)(n > 0 ? in.seq_off[n] : 0) + (2u << 20), false);
+    in.G = m->G; in.C = m->C;
+    in.extra_reserve = engine_workspace(m, n, in.seq_off) + (pin ? pin->plan->scratch_bytes() + 1024 : 0);
+    int rc = batch_build(ctx, b, false, in, sl);
     if (rc == MDF_OK && pin) {
         // alignment scratch (~1 byte per DP cell) from the arena, ahead of the engine stages; released in stream order
         rc = ctx->alloc_n(&b->d_nw_dir, (size_t)pin->plan->dir_words + 4);
@@ -953,7 +1048,12 @@ static int job_enqueue(mdf_model *m, mdf_job *sl, int n, const char *seq, const 
         auto ms = [](auto a, auto b2) { return std::chrono::duration<double, std::milli>(b2 - a).count(); };
         fprintf(stderr, "[mdf_path_submit] n=%d: batch build + H2D %.2f ms, enqueue (host) %.2f ms\n", n, ms(t0, t1), ms(t1, t2));
     }
-    return rc;
+    if (rc != MDF_OK) return rc;
+    sl->n_pairs = pin ? n : 0;
+    sl->busy = true;
+    *job = sl;
+    slot_match_peer(ctx, sl);
+    return MDF_OK;
 }
 
 extern "C" int mdf_path_submit(mdf_model *m, int n, const char *seq, const int64_t *seq_off, const float *coords,
@@ -965,12 +1065,8 @@ extern "C" int mdf_path_submit(mdf_model *m, int n, const char *seq, const int64
     MDF_CUDA(cudaSetDevice(ctx->device));
     mdf_job *sl = nullptr;
     MDF_TRY(slot_acquire(ctx, &sl));
-    const int rc = job_enqueue(m, sl, n, seq, seq_off, coords, coord_off, q_aln, t_aln, aln_off, thr2, gen, scores);
-    if (rc != MDF_OK) return rc;
-    sl->busy = true;
-    *job = sl;
-    slot_match_peer(ctx, sl);
-    return MDF_OK;
+    return job_enqueue(m, sl, {.n = n, .seq = seq, .seq_off = seq_off, .coords = coords, .coord_off = coord_off, .q_aln = q_aln,
+                               .t_aln = t_aln, .aln_off = aln_off}, thr2, gen, scores, job);
 }
 
 // n proteins given as arrays of per-protein pointers (what a host holding n separate strings and coordinate arrays has): packed
@@ -984,58 +1080,28 @@ extern "C" int mdf_path_submit_ragged(mdf_model *m, int n, const char *const *se
     mdf_ctx *ctx = m->ctx;
     MDF_CUDA(cudaSetDevice(ctx->device));
     const auto t0 = std::chrono::steady_clock::now();
-    int64_t T = 0, R = 0, A = 0;
     for (int p = 0; p < n; ++p) {
         MDF_REQUIRE(seq_len[p] >= 0 && coord_rows[p] >= 0 && aln_len[p] >= 0, "mdf_path_submit_ragged: protein %d has a negative length", p);
         MDF_REQUIRE(seq[p] || seq_len[p] == 0, "mdf_path_submit_ragged: protein %d has no sequence", p);
         MDF_REQUIRE(coords[p] || coord_rows[p] == 0, "mdf_path_submit_ragged: protein %d has no coordinates (filter structure-less queries first)", p);
         MDF_REQUIRE((q_aln[p] && t_aln[p]) || aln_len[p] == 0, "mdf_path_submit_ragged: protein %d has no alignment", p);
-        T += seq_len[p]; R += coord_rows[p]; A += aln_len[p];
     }
     mdf_job *sl = nullptr;
     MDF_TRY(slot_acquire(ctx, &sl));
-    const size_t off_b = align_up((size_t)(n + 1) * 8, 256);
-    const size_t seq_at = 3 * off_b, crd_at = seq_at + align_up((size_t)T + 16, 256), qa_at = crd_at + align_up((size_t)R * 12 + 16, 256),
-                 ta_at = qa_at + align_up((size_t)A + 16, 256), total = ta_at + align_up((size_t)A + 16, 256);
-    MDF_TRY(slot_pinned(sl, total));
-    int64_t *so = (int64_t *)sl->pin, *co = (int64_t *)(sl->pin + off_b), *ao = (int64_t *)(sl->pin + 2 * off_b);
-    so[0] = co[0] = ao[0] = 0;
-    for (int p = 0; p < n; ++p) { so[p + 1] = so[p] + seq_len[p]; co[p + 1] = co[p] + coord_rows[p]; ao[p + 1] = ao[p] + aln_len[p]; }
-    char *pseq = sl->pin + seq_at, *pq = sl->pin + qa_at, *pt = sl->pin + ta_at;
-    float *pc = (float *)(sl->pin + crd_at);
-    auto pack = [&](int lo, int hi) {
-        for (int p = lo; p < hi; ++p) {
-            if (seq_len[p]) memcpy(pseq + so[p], seq[p], (size_t)seq_len[p]);
-            if (coord_rows[p]) memcpy(pc + co[p] * 3, coords[p], (size_t)coord_rows[p] * 12);
-            if (aln_len[p]) { memcpy(pq + ao[p], q_aln[p], (size_t)aln_len[p]); memcpy(pt + ao[p], t_aln[p], (size_t)aln_len[p]); }
-        }
-    };
-    const int nt = std::max(1, std::min(ctx->host_threads, n / 256));
-    if (nt == 1) pack(0, n);
-    else {
-        // ranges of equal bytes, not equal protein counts
-        std::vector<std::thread> th;
-        const int64_t per = (T + R * 12 + 2 * A) / nt + 1;
-        int lo = 0;
-        for (int k = 0; k < nt; ++k) {
-            int hi = lo;
-            if (k == nt - 1) hi = n;
-            else while (hi < n && (so[hi] + co[hi] * 12 + 2 * ao[hi]) < per * (k + 1)) ++hi;
-            if (hi > lo) th.emplace_back(pack, lo, hi);
-            lo = hi;
-        }
-        for (auto &t : th) t.join();
-    }
+    RaggedPack pk(n);
+    const int S = pk.column(seq_len, 1, seq), R = pk.column(coord_rows, 12, coords), Q = pk.column(aln_len, 1, q_aln),
+              T = pk.column(aln_len, 1, t_aln);
+    MDF_TRY(pinned_block(sl->pin, sl->pin_bytes, pk.place(nullptr), " for a job slot"));
+    pk.place(sl->pin);
+    const int nt = pack_threads(ctx, n);
+    pk.pack(nt);
     static const bool timing = getenv("MDF_TIMING") != nullptr;
     if (timing)
-        fprintf(stderr, "[mdf_path_submit_ragged] n=%d: packed %.1f MB with %d threads in %.2f ms\n", n, (T + R * 12 + 2 * A) / 1e6, nt,
+        fprintf(stderr, "[mdf_path_submit_ragged] n=%d: packed %.1f MB with %d threads in %.2f ms\n", n,
+                (double)(pk.cols[S].bytes + pk.cols[R].bytes + pk.cols[Q].bytes + pk.cols[T].bytes) / 1e6, nt,
                 std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count());
-    const int rc = job_enqueue(m, sl, n, pseq, so, pc, co, pq, pt, ao, thr2, gen, scores);
-    if (rc != MDF_OK) return rc;
-    sl->busy = true;
-    *job = sl;
-    slot_match_peer(ctx, sl);
-    return MDF_OK;
+    return job_enqueue(m, sl, {.n = n, .seq = pk.at(S), .seq_off = pk.off(S), .coords = (const float *)pk.at(R), .coord_off = pk.off(R),
+                               .q_aln = pk.at(Q), .t_aln = pk.at(T), .aln_off = pk.off(Q)}, thr2, gen, scores, job);
 }
 
 // n (query, target, target coordinates) pairs as arrays of per-pair pointers: the pairs are aligned on the device (nw_align.cu) and
@@ -1056,75 +1122,30 @@ extern "C" int mdf_path_submit_pairs(mdf_model *m, int n, const char *const *que
     MDF_CUDA(cudaSetDevice(ctx->device));
     NwPlan plan;
     MDF_TRY(nw_plan("mdf_path_submit_pairs", n, query, q_len, target, t_len, &plan));
-    int64_t T = 0, R = 0;
-    for (int p = 0; p < n; ++p) {
+    for (int p = 0; p < n; ++p)
         MDF_REQUIRE(coord_rows[p] >= 0 && (coords[p] || coord_rows[p] == 0),
                     "mdf_path_submit_pairs: protein %d has no coordinates (filter structure-less queries first)", p);
-        T += q_len[p]; R += coord_rows[p];
-    }
-    const int64_t NC = plan.off[(size_t)n];
     mdf_job *sl = nullptr;
     MDF_TRY(slot_acquire(ctx, &sl));
-    const size_t off_b = align_up((size_t)(n + 1) * 8, 256);
-    const size_t seq_at = 2 * off_b, crd_at = seq_at + align_up((size_t)T + 16, 256), code_at = crd_at + align_up((size_t)R * 12 + 16, 256),
-                 tab_at = code_at + align_up((size_t)NC + 16, 256), mat_at = tab_at + align_up((size_t)n * sizeof(NwPair) + 16, 256),
-                 stat_at = mat_at + 1024, ops_at = stat_at + align_up((size_t)n * 12 + 16, 256),
-                 total = ops_at + (ops ? align_up((size_t)NC + 16, 256) : 0);
-    MDF_TRY(slot_pinned(sl, total));
-    int64_t *so = (int64_t *)sl->pin, *co = (int64_t *)(sl->pin + off_b);
-    so[0] = co[0] = 0;
-    for (int p = 0; p < n; ++p) { so[p + 1] = so[p] + q_len[p]; co[p + 1] = co[p] + coord_rows[p]; }
-    char *pseq = sl->pin + seq_at;
-    float *pc = (float *)(sl->pin + crd_at);
-    uint8_t *pcode = (uint8_t *)(sl->pin + code_at);
-    uint8_t lut[256];
-    nw_lut(alphabet, A, lut);
-    struct Bad { int p = -1, which = 0; char c = 0; };
-    auto pack = [&](int lo, int hi, Bad *bad) {
-        for (int p = lo; p < hi; ++p) {
-            if (q_len[p]) memcpy(pseq + so[p], query[p], (size_t)q_len[p]);
-            if (coord_rows[p]) memcpy(pc + co[p] * 3, coords[p], (size_t)coord_rows[p] * 12);
-            char c = 0;
-            const int which = nw_encode_pair(lut, query[p], q_len[p], target[p], t_len[p], pcode + plan.off[p], &c);
-            if (which && bad->p < 0) { bad->p = p; bad->which = which; bad->c = c; }
-        }
-    };
-    const int nt = std::max(1, std::min(ctx->host_threads, n / 256));
-    std::vector<Bad> bad((size_t)nt);
-    if (nt == 1) pack(0, n, &bad[0]);
-    else {
-        // ranges of equal bytes, not equal pair counts
-        std::vector<std::thread> th;
-        const int64_t per = (T + R * 12 + NC) / nt + 1;
-        int lo = 0;
-        for (int k = 0; k < nt; ++k) {
-            int hi = lo;
-            if (k == nt - 1) hi = n;
-            else while (hi < n && (so[hi] + co[hi] * 12 + plan.off[hi]) < per * (k + 1)) ++hi;
-            if (hi > lo) th.emplace_back(pack, lo, hi, &bad[k]);
-            lo = hi;
-        }
-        for (auto &t : th) t.join();
-    }
-    for (const Bad &b : bad)           // the thread ranges ascend: the first one that met a bad letter holds the first bad pair
-        if (b.p >= 0) return nw_bad_letter("mdf_path_submit_pairs", b.p, b.which, b.c);
-    if (n) memcpy(sl->pin + tab_at, plan.pairs.data(), (size_t)n * sizeof(NwPair));
-    nw_matrix32(matrix, A, (int8_t *)(sl->pin + mat_at));
-    const PairInputs pin{&plan, pcode, (const NwPair *)(sl->pin + tab_at), (const int8_t *)(sl->pin + mat_at), A, gap_open, gap_extend,
+    RaggedPack pk(n);
+    const int S = pk.column(q_len, 1, query), R = pk.column(coord_rows, 12, coords), K = pk.column(plan.off.data()),
+              TAB = pk.region((size_t)n * sizeof(NwPair)), MAT = pk.region(1024), STAT = pk.region((size_t)n * 12),
+              OPS = pk.region(ops ? (size_t)plan.off[n] : 0);
+    MDF_TRY(pinned_block(sl->pin, sl->pin_bytes, pk.place(nullptr), " for a job slot"));
+    pk.place(sl->pin);
+    MDF_TRY(pack_pairs("mdf_path_submit_pairs", pk, K, pack_threads(ctx, n), plan, alphabet, A, query, q_len, target, t_len));
+    if (n) memcpy(pk.at(TAB), plan.pairs.data(), (size_t)n * sizeof(NwPair));
+    nw_matrix32(matrix, A, (int8_t *)pk.at(MAT));
+    const PairInputs pin{&plan, (const uint8_t *)pk.at(K), (const NwPair *)pk.at(TAB), (const int8_t *)pk.at(MAT), A, gap_open, gap_extend,
                          ops != nullptr};
-    sl->pin_stats = (int32_t *)(sl->pin + stat_at);
-    sl->pin_ops = ops ? sl->pin + ops_at : nullptr;
+    sl->pin_stats = (int32_t *)pk.at(STAT);
+    sl->pin_ops = ops ? pk.at(OPS) : nullptr;
     sl->out_stats[0] = nw_score; sl->out_stats[1] = aln_len; sl->out_stats[2] = n_match;
     sl->out_ops = ops;
     sl->out_ops_len = ops_len;
     if (ops) { sl->out_ops_off.assign(ops_off, ops_off + n); sl->nw_off = plan.off; }
-    const int rc = job_enqueue(m, sl, n, pseq, so, pc, co, nullptr, nullptr, nullptr, thr2, gen, scores, &pin);
-    if (rc != MDF_OK) return rc;
-    sl->n_pairs = n;
-    sl->busy = true;
-    *job = sl;
-    slot_match_peer(ctx, sl);
-    return MDF_OK;
+    return job_enqueue(m, sl, {.n = n, .seq = pk.at(S), .seq_off = pk.off(S), .coords = (const float *)pk.at(R), .coord_off = pk.off(R),
+                               .pairs = &pin}, thr2, gen, scores, job);
 }
 
 extern "C" int mdf_path_wait(mdf_job *job)
@@ -1177,8 +1198,8 @@ extern "C" int mdf_gcn_forward_packed(mdf_model *m, int n, const char *seq, cons
         const int64_t L = seq_off[p + 1] - seq_off[p];
         off += L * mdf_packed_row_words((int)L);
     }
-    MDF_TRY(batch_build(ctx, &b, false, n, seq, seq_off, nullptr, nullptr, nullptr, nullptr, nullptr, packed, m->G, m->C,
-                        engine_workspace(m, n, seq_off)));
+    MDF_TRY(batch_build(ctx, &b, false, {.n = n, .seq = seq, .seq_off = seq_off, .packed = packed, .G = m->G, .C = m->C,
+                                         .extra_reserve = engine_workspace(m, n, seq_off)}));
     MDF_TRY(run_path(m, &b, 0.f, 0, 4, false));
     return fetch_scores(m, &b, scores);
 }
@@ -1192,8 +1213,8 @@ extern "C" int mdf_gcn_forward_dense(mdf_model *m, const char *seq, int L, const
     mdf_batch b;
     const int64_t seq_off[2] = {0, L};
     const size_t dense_bytes = (size_t)L * L * 4;
-    MDF_TRY(batch_build(ctx, &b, false, 1, seq, seq_off, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, m->G, m->C,
-                        engine_workspace(m, 1, seq_off) + dense_bytes + 4096));
+    MDF_TRY(batch_build(ctx, &b, false, {.n = 1, .seq = seq, .seq_off = seq_off, .G = m->G, .C = m->C,
+                                         .extra_reserve = engine_workspace(m, 1, seq_off) + dense_bytes + 4096}));
     int32_t *dd;
     MDF_TRY(ctx->alloc_n(&dd, (size_t)L * L + 1));
     if (L) MDF_CUDA(cudaMemcpyAsync(dd, cmap, dense_bytes, cudaMemcpyHostToDevice, ctx->stream));
@@ -1233,8 +1254,9 @@ extern "C" int mdf_cmap_build_transfer(mdf_ctx *ctx, int n, const float *coords,
             dense_total += (size_t)(L * L);
         }
     }
-    MDF_TRY(batch_build(ctx, &b, false, n, dummy.data(), seq_off, coords, coord_off, q_aln, t_aln, aln_off, nullptr, 1, 1,
-                        dense_total * 4 + (size_t)(n + 1) * 8 + 8192));
+    MDF_TRY(batch_build(ctx, &b, false, {.n = n, .seq = dummy.data(), .seq_off = seq_off, .coords = coords, .coord_off = coord_off,
+                                         .q_aln = q_aln, .t_aln = t_aln, .aln_off = aln_off, .G = 1, .C = 1,
+                                         .extra_reserve = dense_total * 4 + (size_t)(n + 1) * 8 + 8192}));
     if (packed_off)
         for (int p = 0; p <= n; ++p)
             if (packed_off[p] != b.h_packed_off[p]) {
@@ -1273,16 +1295,10 @@ extern "C" int mdf_cmap_build_transfer_ragged(mdf_ctx *ctx, int n, const float *
 {
     MDF_REQUIRE((ctx || !packed_out) && n >= 0 && packed_off_out && seq_off_out, "mdf_cmap_build_transfer_ragged: bad arguments");
     MDF_REQUIRE(n == 0 || (q_aln && aln_len), "mdf_cmap_build_transfer_ragged: alignment arrays missing");
-    const int nt = std::max(1, std::min(ctx ? ctx->host_threads : 4, n / 256));         // (sizes only: host work, no context needed)
-    auto run_threads = [&](auto &&fn) {
-        if (nt == 1) { fn(0, n); return; }
-        std::vector<std::thread> th;
-        for (int k = 0; k < nt; ++k) th.emplace_back(fn, (int)((int64_t)n * k / nt), (int)((int64_t)n * (k + 1) / nt));
-        for (auto &t : th) t.join();
-    };
     for (int p = 0; p < n; ++p) MDF_REQUIRE(aln_len[p] >= 0 && (q_aln[p] || aln_len[p] == 0), "mdf_cmap_build_transfer_ragged: alignment %d is missing", p);
+    const int nt = pack_threads(ctx, n);          // (sizes only: host work, no context needed)
     std::vector<int> lq((size_t)n, 0);
-    run_threads([&](int lo, int hi) {
+    run_split(n, nt, [&](int p) { return (int64_t)aln_len[p]; }, [&](int lo, int hi) {
         for (int p = lo; p < hi; ++p) {
             const char *q = q_aln[p];
             int c = 0;
@@ -1300,35 +1316,17 @@ extern "C" int mdf_cmap_build_transfer_ragged(mdf_ctx *ctx, int n, const float *
     MDF_REQUIRE((int64_t)packed_capacity_words >= packed_off_out[n], "mdf_cmap_build_transfer_ragged: output holds %zu words, %lld needed",
                 packed_capacity_words, (long long)packed_off_out[n]);
     MDF_CUDA(cudaSetDevice(ctx->device));
-    int64_t R = 0, A = 0;
     for (int p = 0; p < n; ++p) {
         MDF_REQUIRE(coord_rows[p] >= 0 && (coords[p] || coord_rows[p] == 0), "mdf_cmap_build_transfer_ragged: alignment %d has no coordinates", p);
         MDF_REQUIRE(t_aln[p] || aln_len[p] == 0, "mdf_cmap_build_transfer_ragged: alignment %d has no target string", p);
-        R += coord_rows[p]; A += aln_len[p];
     }
-    const size_t off_b = align_up((size_t)(n + 1) * 8, 256);
-    const size_t crd_at = 2 * off_b, qa_at = crd_at + align_up((size_t)R * 12 + 16, 256), ta_at = qa_at + align_up((size_t)A + 16, 256),
-                 total = ta_at + align_up((size_t)A + 16, 256);
-    if (ctx->rag_pin_bytes < total) {
-        if (ctx->rag_pin) MDF_CUDA(cudaFreeHost(ctx->rag_pin));
-        ctx->rag_pin = nullptr; ctx->rag_pin_bytes = 0;
-        const size_t want = align_up(total + total / 4, 2u << 20);
-        cudaError_t e = cudaHostAlloc((void **)&ctx->rag_pin, want, cudaHostAllocDefault);
-        if (e != cudaSuccess) { cudaGetLastError(); set_error("cudaHostAlloc(%zu bytes) failed: %s", want, cudaGetErrorString(e)); return MDF_ENOMEM; }
-        ctx->rag_pin_bytes = want;
-    }
-    int64_t *co = (int64_t *)ctx->rag_pin, *ao = (int64_t *)(ctx->rag_pin + off_b);
-    co[0] = ao[0] = 0;
-    for (int p = 0; p < n; ++p) { co[p + 1] = co[p] + coord_rows[p]; ao[p + 1] = ao[p] + aln_len[p]; }
-    float *pc = (float *)(ctx->rag_pin + crd_at);
-    char *pq = ctx->rag_pin + qa_at, *pt = ctx->rag_pin + ta_at;
-    run_threads([&](int lo, int hi) {
-        for (int p = lo; p < hi; ++p) {
-            if (coord_rows[p]) memcpy(pc + co[p] * 3, coords[p], (size_t)coord_rows[p] * 12);
-            if (aln_len[p]) { memcpy(pq + ao[p], q_aln[p], (size_t)aln_len[p]); memcpy(pt + ao[p], t_aln[p], (size_t)aln_len[p]); }
-        }
-    });
-    return mdf_cmap_build_transfer(ctx, n, pc, co, pq, pt, ao, seq_off_out, thr2, gen, packed_out, packed_off_out, nullptr, nullptr);
+    RaggedPack pk(n);
+    const int R = pk.column(coord_rows, 12, coords), Q = pk.column(aln_len, 1, q_aln), T = pk.column(aln_len, 1, t_aln);
+    MDF_TRY(pinned_block(ctx->rag_pin, ctx->rag_pin_bytes, pk.place(nullptr), ""));
+    pk.place(ctx->rag_pin);
+    pk.pack(nt);
+    return mdf_cmap_build_transfer(ctx, n, (const float *)pk.at(R), pk.off(R), pk.at(Q), pk.at(T), pk.off(Q), seq_off_out, thr2, gen,
+                                   packed_out, packed_off_out, nullptr, nullptr);
 }
 
 // ------------------------------------------------------------------------------------------- model

@@ -79,6 +79,14 @@ struct mdf_job {
         meta_top = at + bytes;
         return meta + at;
     }
+    // source of a small host -> device copy: staged in `slot` while *staged holds and there is room, else `src` itself with
+    // *staged = false - the caller then synchronises before its pageable sources go out of scope
+    static const void *src_of(mdf_job *slot, const void *src, size_t bytes, bool *staged)
+    {
+        const void *q = *staged ? slot->stage(src, bytes) : nullptr;
+        if (!q) *staged = false;
+        return q ? q : src;
+    }
 };
 
 // Device workspace: one big allocation, bump-allocated, reset per API call (stack discipline).

@@ -69,6 +69,82 @@ static int coords_of(PyObject *c, Py_buffer *views, Py_ssize_t *nviews, Py_ssize
     return 0;
 }
 
+enum { TEXT, SAME_LEN, COORDS };      /* SAME_LEN: text items as long as those of the column before (paired alignment strings) */
+
+/* One argument of n items, collected into pointer / length arrays: str or bytes items (their buffers and lengths), or coordinate
+ * items (their float32 data and row counts, with the buffer views held until release) */
+typedef struct {
+    const char *name;
+    int kind;
+    PyObject *obj, *fast;
+    const void **ptr;
+    int *len;
+    Py_buffer *views;
+    Py_ssize_t nviews;
+} Column;
+
+/* Collects k columns that must hold the same number *n of items (else ValueError `mismatch`; OverflowError `too_long` for an item
+ * of 2^31 characters or more).  Returns -1 with an exception set on failure; release() the columns in either case. */
+static int collect(Column *c, int k, const char *mismatch, const char *too_long, Py_ssize_t *n)
+{
+    char msg[64];
+    for (int j = 0; j < k; ++j) {
+        snprintf(msg, sizeof msg, "%s must be a sequence", c[j].name);
+        if (!(c[j].fast = PySequence_Fast(c[j].obj, msg))) return -1;
+    }
+    *n = PySequence_Fast_GET_SIZE(c[0].fast);
+    for (int j = 1; j < k; ++j)
+        if (PySequence_Fast_GET_SIZE(c[j].fast) != *n) {
+            PyErr_SetString(PyExc_ValueError, mismatch);
+            return -1;
+        }
+    for (int j = 0; j < k; ++j) {
+        c[j].ptr = malloc(sizeof(void *) * (*n + 1));
+        c[j].len = malloc(sizeof(int) * (*n + 1));
+        if (c[j].kind == COORDS) c[j].views = calloc((size_t)*n + 1, sizeof(Py_buffer));
+        if (!c[j].ptr || !c[j].len || (c[j].kind == COORDS && !c[j].views)) {
+            PyErr_NoMemory();
+            return -1;
+        }
+    }
+    for (Py_ssize_t i = 0; i < *n; ++i)
+        for (int j = 0; j < k; ++j) {
+            Column *col = &c[j];
+            PyObject *o = PySequence_Fast_GET_ITEM(col->fast, i);
+            if (col->kind == COORDS) {
+                const float *data;
+                if (coords_of(o, col->views, &col->nviews, i, &data, &col->len[i]) < 0) return -1;
+                col->ptr[i] = data;
+                continue;
+            }
+            const char *text;
+            Py_ssize_t len;
+            if (text_of(o, &text, &len, col->name, i) < 0) return -1;
+            if (col->kind == SAME_LEN && len != c[j - 1].len[i]) {
+                PyErr_Format(PyExc_ValueError, "alignment %zd: query and target alignments differ in length", i);
+                return -1;
+            }
+            if (len > INT32_MAX) {
+                PyErr_SetString(PyExc_OverflowError, too_long);
+                return -1;
+            }
+            col->ptr[i] = text;
+            col->len[i] = (int)len;
+        }
+    return 0;
+}
+
+static void release(Column *c, int k)
+{
+    for (int j = 0; j < k; ++j) {
+        for (Py_ssize_t i = 0; i < c[j].nviews; ++i) PyBuffer_Release(&c[j].views[i]);
+        free(c[j].views);
+        free(c[j].ptr);
+        free(c[j].len);
+        Py_XDECREF(c[j].fast);
+    }
+}
+
 static PyObject *submit_ragged(PyObject *self, PyObject *args)
 {
     unsigned long long fn_addr, model_addr, scores_addr;
@@ -76,52 +152,21 @@ static PyObject *submit_ragged(PyObject *self, PyObject *args)
     double thr2;
     int gen;
     if (!PyArg_ParseTuple(args, "KKOOOOdiK", &fn_addr, &model_addr, &seqs, &gq, &gt, &coords, &thr2, &gen, &scores_addr)) return NULL;
-    PyObject *fs = PySequence_Fast(seqs, "seqs must be a sequence"), *fq = NULL, *ft = NULL, *fc = NULL;
-    if (!fs) return NULL;
-    fq = PySequence_Fast(gq, "gapped_query must be a sequence");
-    ft = fq ? PySequence_Fast(gt, "gapped_target must be a sequence") : NULL;
-    fc = ft ? PySequence_Fast(coords, "coords must be a sequence") : NULL;
-    const Py_ssize_t n = PySequence_Fast_GET_SIZE(fs);
-    const char **pseq = NULL, **pq = NULL, **pt = NULL;
-    const float **pc = NULL;
-    int *lseq = NULL, *laln = NULL, *rows = NULL;
-    Py_buffer *views = NULL;
-    Py_ssize_t nviews = 0;
+    Column c[4] = {{"seqs", TEXT, seqs}, {"gapped_query", TEXT, gq}, {"gapped_target", SAME_LEN, gt}, {"coords", COORDS, coords}};
+    Py_ssize_t n;
     PyObject *result = NULL;
-    if (!fc) goto done;
-    if (PySequence_Fast_GET_SIZE(fq) != n || PySequence_Fast_GET_SIZE(ft) != n || PySequence_Fast_GET_SIZE(fc) != n) {
-        PyErr_SetString(PyExc_ValueError, "seqs, gapped_query, gapped_target and coords must have the same length");
-        goto done;
-    }
-    pseq = malloc(sizeof(char *) * (n + 1)); pq = malloc(sizeof(char *) * (n + 1)); pt = malloc(sizeof(char *) * (n + 1));
-    pc = malloc(sizeof(float *) * (n + 1));
-    lseq = malloc(sizeof(int) * (n + 1)); laln = malloc(sizeof(int) * (n + 1)); rows = malloc(sizeof(int) * (n + 1));
-    views = calloc((size_t)n + 1, sizeof(Py_buffer));
-    if (!pseq || !pq || !pt || !pc || !lseq || !laln || !rows || !views) { PyErr_NoMemory(); goto done; }
-    for (Py_ssize_t i = 0; i < n; ++i) {
-        Py_ssize_t ls, lq, lt;
-        if (text_of(PySequence_Fast_GET_ITEM(fs, i), &pseq[i], &ls, "seqs", i) < 0) goto done;
-        if (text_of(PySequence_Fast_GET_ITEM(fq, i), &pq[i], &lq, "gapped_query", i) < 0) goto done;
-        if (text_of(PySequence_Fast_GET_ITEM(ft, i), &pt[i], &lt, "gapped_target", i) < 0) goto done;
-        if (lq != lt) { PyErr_Format(PyExc_ValueError, "alignment %zd: query and target alignments differ in length", i); goto done; }
-        if (ls > INT32_MAX || lq > INT32_MAX) { PyErr_SetString(PyExc_OverflowError, "sequence too long"); goto done; }
-        lseq[i] = (int)ls; laln[i] = (int)lq;
-        if (coords_of(PySequence_Fast_GET_ITEM(fc, i), views, &nviews, i, &pc[i], &rows[i]) < 0) goto done;
-    }
-    {
+    if (collect(c, 4, "seqs, gapped_query, gapped_target and coords must have the same length", "sequence too long", &n) == 0) {
         mdf_job *job = NULL;
         int rc;
         submit_ragged_fn fn = (submit_ragged_fn)(uintptr_t)fn_addr;
         Py_BEGIN_ALLOW_THREADS
-        rc = fn((mdf_model *)(uintptr_t)model_addr, (int)n, pseq, lseq, pc, rows, pq, pt, laln, (float)thr2, gen,
+        rc = fn((mdf_model *)(uintptr_t)model_addr, (int)n, (const char *const *)c[0].ptr, c[0].len, (const float *const *)c[3].ptr,
+                c[3].len, (const char *const *)c[1].ptr, (const char *const *)c[2].ptr, c[1].len, (float)thr2, gen,
                 (float *)(uintptr_t)scores_addr, &job);
         Py_END_ALLOW_THREADS
         result = Py_BuildValue("iK", rc, (unsigned long long)(uintptr_t)job);
     }
-done:
-    for (Py_ssize_t i = 0; i < nviews; ++i) PyBuffer_Release(&views[i]);
-    free(views); free(pseq); free(pq); free(pt); free(pc); free(lseq); free(laln); free(rows);
-    Py_XDECREF(fs); Py_XDECREF(fq); Py_XDECREF(ft); Py_XDECREF(fc);
+    release(c, 4);
     return result;
 }
 
@@ -144,50 +189,23 @@ static PyObject *submit_pairs(PyObject *self, PyObject *args)
                           &gap_open, &gap_extend, &thr2, &gen, &scores_addr, &nw_addr, &len_addr, &match_addr, &ops_addr, &ops_off_addr,
                           &ops_len_addr))
         return NULL;
-    PyObject *fq = PySequence_Fast(queries, "queries must be a sequence"), *ft = NULL, *fc = NULL;
-    if (!fq) return NULL;
-    ft = PySequence_Fast(targets, "targets must be a sequence");
-    fc = ft ? PySequence_Fast(coords, "coords must be a sequence") : NULL;
-    const Py_ssize_t n = PySequence_Fast_GET_SIZE(fq);
-    const char **pq = NULL, **pt = NULL;
-    const float **pc = NULL;
-    int *lq = NULL, *lt = NULL, *rows = NULL;
-    Py_buffer *views = NULL;
-    Py_ssize_t nviews = 0;
+    Column c[3] = {{"queries", TEXT, queries}, {"targets", TEXT, targets}, {"coords", COORDS, coords}};
+    Py_ssize_t n;
     PyObject *result = NULL;
-    if (!fc) goto done;
-    if (PySequence_Fast_GET_SIZE(ft) != n || PySequence_Fast_GET_SIZE(fc) != n) {
-        PyErr_SetString(PyExc_ValueError, "queries, targets and coords must have the same length");
-        goto done;
-    }
-    pq = malloc(sizeof(char *) * (n + 1)); pt = malloc(sizeof(char *) * (n + 1)); pc = malloc(sizeof(float *) * (n + 1));
-    lq = malloc(sizeof(int) * (n + 1)); lt = malloc(sizeof(int) * (n + 1)); rows = malloc(sizeof(int) * (n + 1));
-    views = calloc((size_t)n + 1, sizeof(Py_buffer));
-    if (!pq || !pt || !pc || !lq || !lt || !rows || !views) { PyErr_NoMemory(); goto done; }
-    for (Py_ssize_t i = 0; i < n; ++i) {
-        Py_ssize_t a, b;
-        if (text_of(PySequence_Fast_GET_ITEM(fq, i), &pq[i], &a, "queries", i) < 0) goto done;
-        if (text_of(PySequence_Fast_GET_ITEM(ft, i), &pt[i], &b, "targets", i) < 0) goto done;
-        if (a > INT32_MAX || b > INT32_MAX) { PyErr_SetString(PyExc_OverflowError, "sequence too long"); goto done; }
-        lq[i] = (int)a; lt[i] = (int)b;
-        if (coords_of(PySequence_Fast_GET_ITEM(fc, i), views, &nviews, i, &pc[i], &rows[i]) < 0) goto done;
-    }
-    {
+    if (collect(c, 3, "queries, targets and coords must have the same length", "sequence too long", &n) == 0) {
         mdf_job *job = NULL;
         int rc;
         submit_pairs_fn fn = (submit_pairs_fn)(uintptr_t)fn_addr;
         Py_BEGIN_ALLOW_THREADS
-        rc = fn((mdf_model *)(uintptr_t)model_addr, (int)n, pq, lq, pt, lt, pc, rows, (const int8_t *)(uintptr_t)matrix_addr, alphabet, (int)A,
-                gap_open, gap_extend, (float)thr2, gen, (float *)(uintptr_t)scores_addr, (int32_t *)(uintptr_t)nw_addr,
+        rc = fn((mdf_model *)(uintptr_t)model_addr, (int)n, (const char *const *)c[0].ptr, c[0].len, (const char *const *)c[1].ptr,
+                c[1].len, (const float *const *)c[2].ptr, c[2].len, (const int8_t *)(uintptr_t)matrix_addr, alphabet, (int)A, gap_open,
+                gap_extend, (float)thr2, gen, (float *)(uintptr_t)scores_addr, (int32_t *)(uintptr_t)nw_addr,
                 (int32_t *)(uintptr_t)len_addr, (int32_t *)(uintptr_t)match_addr, (char *)(uintptr_t)ops_addr,
                 (const int64_t *)(uintptr_t)ops_off_addr, (int *)(uintptr_t)ops_len_addr, &job);
         Py_END_ALLOW_THREADS
         result = Py_BuildValue("iK", rc, (unsigned long long)(uintptr_t)job);
     }
-done:
-    for (Py_ssize_t i = 0; i < nviews; ++i) PyBuffer_Release(&views[i]);
-    free(views); free(pq); free(pt); free(pc); free(lq); free(lt); free(rows);
-    Py_XDECREF(fq); Py_XDECREF(ft); Py_XDECREF(fc);
+    release(c, 3);
     return result;
 }
 
@@ -230,57 +248,28 @@ static PyObject *cmap_ragged(PyObject *self, PyObject *args)
     double thr2;
     int gen;
     if (!PyArg_ParseTuple(args, "KKOOOdiKK", &fn_addr, &ctx_addr, &gq, &gt, &coords, &thr2, &gen, &out_addr, &out_cap)) return NULL;
-    const int sizes_only = out_addr == 0;
-    PyObject *fq = PySequence_Fast(gq, "gapped_query must be a sequence"), *ft = NULL, *fc = NULL;
-    if (!fq) return NULL;
-    const Py_ssize_t n = PySequence_Fast_GET_SIZE(fq);
-    const char **pq = NULL, **pt = NULL;
-    const float **pc = NULL;
-    int *laln = NULL, *rows = NULL;
-    Py_buffer *views = NULL;
-    Py_ssize_t nviews = 0;
+    /* out_addr == 0: sizes only, from the query alignments alone */
+    const int k = out_addr == 0 ? 1 : 3;
+    Column c[3] = {{"gapped_query", TEXT, gq}, {"gapped_target", SAME_LEN, gt}, {"coords", COORDS, coords}};
+    Py_ssize_t n;
     PyObject *result = NULL, *poff = NULL, *soff = NULL;
-    if (!sizes_only) {
-        ft = PySequence_Fast(gt, "gapped_target must be a sequence");
-        fc = ft ? PySequence_Fast(coords, "coords must be a sequence") : NULL;
-        if (!fc) goto done;
-        if (PySequence_Fast_GET_SIZE(ft) != n || PySequence_Fast_GET_SIZE(fc) != n) {
-            PyErr_SetString(PyExc_ValueError, "gapped_query, gapped_target and coords must have the same length");
-            goto done;
-        }
+    if (collect(c, k, "gapped_query, gapped_target and coords must have the same length", "alignment too long", &n) == 0) {
+        poff = PyBytes_FromStringAndSize(NULL, (n + 1) * 8);
+        soff = PyBytes_FromStringAndSize(NULL, (n + 1) * 8);
     }
-    pq = malloc(sizeof(char *) * (n + 1)); pt = malloc(sizeof(char *) * (n + 1)); pc = malloc(sizeof(float *) * (n + 1));
-    laln = malloc(sizeof(int) * (n + 1)); rows = malloc(sizeof(int) * (n + 1));
-    views = calloc((size_t)n + 1, sizeof(Py_buffer));
-    poff = PyBytes_FromStringAndSize(NULL, (n + 1) * 8);
-    soff = PyBytes_FromStringAndSize(NULL, (n + 1) * 8);
-    if (!pq || !pt || !pc || !laln || !rows || !views || !poff || !soff) { PyErr_NoMemory(); goto done; }
-    for (Py_ssize_t i = 0; i < n; ++i) {
-        Py_ssize_t lq, lt;
-        if (text_of(PySequence_Fast_GET_ITEM(fq, i), &pq[i], &lq, "gapped_query", i) < 0) goto done;
-        if (lq > INT32_MAX) { PyErr_SetString(PyExc_OverflowError, "alignment too long"); goto done; }
-        laln[i] = (int)lq;
-        pt[i] = NULL; pc[i] = NULL; rows[i] = 0;
-        if (sizes_only) continue;
-        if (text_of(PySequence_Fast_GET_ITEM(ft, i), &pt[i], &lt, "gapped_target", i) < 0) goto done;
-        if (lq != lt) { PyErr_Format(PyExc_ValueError, "alignment %zd: query and target alignments differ in length", i); goto done; }
-        if (coords_of(PySequence_Fast_GET_ITEM(fc, i), views, &nviews, i, &pc[i], &rows[i]) < 0) goto done;
-    }
-    {
+    if (poff && soff) {
         int rc;
         cmap_ragged_fn fn = (cmap_ragged_fn)(uintptr_t)fn_addr;
         int64_t *po = (int64_t *)PyBytes_AS_STRING(poff), *so = (int64_t *)PyBytes_AS_STRING(soff);
         Py_BEGIN_ALLOW_THREADS
-        rc = fn((mdf_ctx *)(uintptr_t)ctx_addr, (int)n, pc, rows, pq, pt, laln, (float)thr2, gen, (uint32_t *)(uintptr_t)out_addr,
-                (size_t)out_cap, po, so);
+        rc = fn((mdf_ctx *)(uintptr_t)ctx_addr, (int)n, (const float *const *)c[2].ptr, c[2].len, (const char *const *)c[0].ptr,
+                (const char *const *)c[1].ptr, c[0].len, (float)thr2, gen, (uint32_t *)(uintptr_t)out_addr, (size_t)out_cap, po, so);
         Py_END_ALLOW_THREADS
         result = Py_BuildValue("iOO", rc, poff, soff);
     }
-done:
-    for (Py_ssize_t i = 0; i < nviews; ++i) PyBuffer_Release(&views[i]);
-    free(views); free(pq); free(pt); free(pc); free(laln); free(rows);
-    Py_XDECREF(poff); Py_XDECREF(soff);
-    Py_XDECREF(fq); Py_XDECREF(ft); Py_XDECREF(fc);
+    Py_XDECREF(poff);
+    Py_XDECREF(soff);
+    release(c, k);
     return result;
 }
 

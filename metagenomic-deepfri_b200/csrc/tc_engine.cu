@@ -613,12 +613,7 @@ static int build_meta(mdf_ctx *ctx, mdf_batch *b, TcBatchMeta &meta, bool want_e
     cudaStream_t s = ctx->stream;
     // asynchronous jobs stage these tables through the slot's pinned memory: the copies then never block the submitting thread
     bool staged = b->slot != nullptr;
-    auto src_of = [&](const void *p, size_t bytes) -> const void * {
-        if (!staged) return p;
-        const void *q = b->slot->stage(p, bytes);
-        if (!q) { staged = false; return p; }
-        return q;
-    };
+    auto src_of = [&](const void *p, size_t bytes) { return mdf_job::src_of(b->slot, p, bytes, &staged); };
     // the [Tp] row map (24 MB for a 16k-protein batch) is filled on the device; only the per-tile / per-protein arrays travel
     MDF_CUDA(cudaMemcpyAsync(meta.seg_off, src_of(seg_off.data(), (size_t)(n + 1) * 8), (size_t)(n + 1) * 8, cudaMemcpyHostToDevice, s));
     MDF_CUDA(cudaMemsetAsync(meta.rowmap, 0xFF, (size_t)Tp * 4, s));

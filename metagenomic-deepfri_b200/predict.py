@@ -22,7 +22,7 @@ from typing import List, Optional, Sequence
 import numpy as np
 
 from . import _lib
-from .batching import pack_structures, packed_offsets
+from .batching import float32_coords, pack_structures, packed_offsets, with_float32_coords
 
 _ALPHABET = b"-DGULNTKHYWCPVSOIEFXQABZRM"          # predict.pyx:26
 _LUT = np.full(256, -1, np.int16)
@@ -52,17 +52,6 @@ def _pack_checked(seqs: Sequence[str]):
     if n:
         np.cumsum(np.fromiter(map(len, seqs), np.int64, n), out=off[1:])
     return b, off
-
-
-def _float32_coords(coords) -> list:
-    """Structures as C-contiguous float32 [Lt, 3] arrays, converted like the reference's astype(np.float32) (contact_map.py:25)."""
-    conv = []
-    for i, c in enumerate(coords):
-        c = np.ascontiguousarray(c, dtype=np.float32)
-        if c.ndim != 2 or c.shape[1] != 3:
-            raise ValueError(f"structure {i}: coordinates must have shape (Lt, 3)")
-        conv.append(c)
-    return conv
 
 
 def seq2onehot(seq: str) -> np.ndarray:
@@ -202,7 +191,7 @@ class PairBatch(PathBatch):
         t_bytes = "".join(ts).encode("ascii")
         t_off = np.zeros(len(ts) + 1, np.int64)
         np.cumsum(np.fromiter(map(len, ts), np.int64, len(ts)), out=t_off[1:])
-        cs = _float32_coords(coords)
+        cs = float32_coords(coords)
         c_off = np.zeros(len(cs) + 1, np.int64)
         np.cumsum(np.fromiter((c.shape[0] for c in cs), np.int64, len(cs)), out=c_off[1:])
         flat = np.ascontiguousarray(np.concatenate(cs) if cs else np.zeros((0, 3), np.float32))
@@ -424,11 +413,7 @@ class Predictor:
         host = _lib.pyhost()
         args = (_lib.fn_addr("mdf_path_submit_ragged"), self._handle.value, seqs, gapped_query, gapped_target)
         tail = (float(threshold_sq(threshold)), int(generated_contacts), out.ctypes.data)
-        try:
-            rc, job = host.submit_ragged(*args, coords, *tail)
-        except TypeError:
-            # some structure is not a C-contiguous float32 [Lt, 3] array (lists, float64 ...): convert and retry once
-            rc, job = host.submit_ragged(*args, _float32_coords(coords), *tail)
+        rc, job = with_float32_coords(lambda cs: host.submit_ragged(*args, cs, *tail), coords)
         _lib.check(rc)
         return PathJob(self, job, out, (seqs, gapped_query, gapped_target))
 
@@ -474,10 +459,7 @@ class Predictor:
         tail = (m.ctypes.data, alphabet.encode("ascii"), int(gap_open), int(gap_extend), float(threshold_sq(threshold)),
                 int(generated_contacts), out.ctypes.data, stats[0].ctypes.data, stats[1].ctypes.data, stats[2].ctypes.data,
                 *((ops[0].ctypes.data, ops[1].ctypes.data, ops[2].ctypes.data) if alignments else (0, 0, 0)))
-        try:
-            rc, job = host.submit_pairs(*head, coords, *tail)
-        except TypeError:
-            rc, job = host.submit_pairs(*head, _float32_coords(coords), *tail)
+        rc, job = with_float32_coords(lambda cs: host.submit_pairs(*head, cs, *tail), coords)
         _lib.check(rc)
         return PairJob(job, out, stats, ops, qs)
 
