@@ -193,6 +193,8 @@ int mdf_path_submit_ragged(mdf_model *model, int n,
                            const float *const *coords, const int *coord_rows,
                            const char *const *q_aln, const char *const *t_aln, const int *aln_len,
                            float thr2, int generated_contacts, float *scores, mdf_job **job);
+/* Waits for a job of either kind - mdf_path_submit* or mdf_cnn_submit_ragged - until its outputs are on the host, and reports
+ * device-side input errors (a residue outside the alphabet: "Invalid character in sequence"). */
 int mdf_path_wait(mdf_job *job);
 /* Alignment and prediction in one job: pair p is (query[p], target[p], coords[p]) - the GCN's query sequence (q_len[p] residues),
  * its best-hit target sequence (t_len[p]) and the target's C-alpha coordinates (float32 [coord_rows[p], 3]).  The pairs are
@@ -287,6 +289,13 @@ int mdf_cnn_forward(mdf_cnn_model *model, int n, const char *seq, const int64_t 
 int mdf_cnn_upload(mdf_cnn_model *model, int n, const char *seq, const int64_t *seq_off);
 int mdf_cnn_run(mdf_cnn_model *model);
 int mdf_cnn_fetch(mdf_cnn_model *model, float *scores /* host [n, C] */, float *pooled /* host [n, sum filters] or NULL */);
+/* Asynchronous mdf_cnn_forward from per-sequence pointers (pipeline.py:607-613 holds one str per unaligned query).  Takes one of
+ * the context's two job slots - the same slots mdf_path_submit* use, so CNN and GCN jobs may be in flight together - packs the
+ * sequences into the slot's pinned block on MDF_HOST_THREADS threads, enqueues H2D, encode, conv, head and the D2H of the
+ * scores, and returns; mdf_path_wait completes the job.  Every sequence needs >= 1 residue (MDF_EINVAL here, naming the index);
+ * a residue outside the alphabet is reported by mdf_path_wait ("Invalid character in sequence").  The caller's strings may be
+ * released when the call returns; `scores` (host float32 [n, C]) must stay valid until mdf_path_wait returns. */
+int mdf_cnn_submit_ragged(mdf_cnn_model *model, int n, const char *const *seq, const int *seq_len, float *scores, mdf_job **job);
 
 /* ---- pdb.py:130-162 extract_calpha_coords / bio_utils.py:230-302 extract_residues_coordinates: coordinate ingest (host only) ----
  * C-alpha coordinates of one PDB text with biotite's selection as the reference applies it: first model, ATOM records (HETATM =

@@ -134,6 +134,7 @@ def lib() -> C.CDLL:
         L.mdf_cnn_upload.argtypes = [vp, C.c_int, vp, c_i64p]
         L.mdf_cnn_run.argtypes = [vp]
         L.mdf_cnn_fetch.argtypes = [vp, vp, vp]
+        L.mdf_cnn_submit_ragged.argtypes = [vp, C.c_int, vp, vp, vp, C.POINTER(vp)]
         L.mdf_pdb_calpha.argtypes = [vp, C.c_size_t, C.c_char, vp, vp, vp, C.c_int, C.POINTER(C.c_int)]
         L.mdf_pdb_calpha_batch.argtypes = [C.c_int, vp, c_i64p, C.c_char, C.c_int, vp, vp, C.c_int64, c_i64p]
         L.mdf_coords_cache_create.argtypes = [C.c_char_p, C.c_int64, vp, vp, vp]
@@ -151,7 +152,7 @@ def lib() -> C.CDLL:
         for name in ("mdf_model_load", "mdf_cnn_model_load", "mdf_onnx_inspect", "mdf_model_info"):
             getattr(L, name).restype = C.c_int
         for name in ("mdf_cnn_model_create", "mdf_cnn_model_destroy", "mdf_cnn_forward", "mdf_cnn_upload", "mdf_cnn_run",
-                     "mdf_cnn_fetch"):
+                     "mdf_cnn_fetch", "mdf_cnn_submit_ragged"):
             getattr(L, name).restype = C.c_int
         for name in ("mdf_ctx_create", "mdf_ctx_destroy", "mdf_ctx_synchronize", "mdf_pairwise_sqeuclidean",
                      "mdf_contact_map_dense", "mdf_contact_map_sparse", "mdf_align_contact_map",
@@ -172,6 +173,7 @@ EXPORTED_SYMBOLS = [
     "mdf_batch_upload", "mdf_batch_destroy", "mdf_path_run", "mdf_path_run_stages", "mdf_path_run_shared",
     "mdf_batch_fetch_scores", "mdf_batch_fetch", "mdf_batch_scores_device", "mdf_batch_unpack_dense", "mdf_batch_invalidate",
     "mdf_cnn_model_create", "mdf_cnn_model_destroy", "mdf_cnn_forward", "mdf_cnn_upload", "mdf_cnn_run", "mdf_cnn_fetch",
+    "mdf_cnn_submit_ragged",
     "mdf_path_submit", "mdf_path_submit_ragged", "mdf_path_submit_pairs", "mdf_path_wait", "mdf_cmap_build_transfer_ragged",
     "mdf_batch_upload_pairs", "mdf_batch_fetch_alignment",
     "mdf_pdb_calpha", "mdf_pdb_calpha_batch", "mdf_coords_cache_create", "mdf_coords_cache_open", "mdf_coords_cache_close",

@@ -8,6 +8,7 @@
 #include <thread>
 
 #include "cmap_kernels.cuh"
+#include "cnn.cuh"
 #include "gcn.cuh"
 #include "nw_align.cuh"
 #include "tc_engine.cuh"
@@ -338,18 +339,6 @@ extern "C" int mdf_align_contact_map(mdf_ctx *ctx, const char *q_aln, const char
 }
 
 // ------------------------------------------------------------------------------------------- batches
-struct Carver {   // sub-allocates one block; first pass (base == nullptr) only measures
-    char *base = nullptr;
-    size_t top = 0;
-    template <typename T>
-    T *take(size_t count)
-    {
-        size_t off = align_up(top, 256);
-        top = off + count * sizeof(T);
-        return base ? reinterpret_cast<T *>(base + off) : nullptr;
-    }
-};
-
 // residue codes and alignment table of a pairs batch, in host memory its copies may read (pinned for jobs)
 struct PairInputs {
     const NwPlan *plan;
@@ -1000,6 +989,37 @@ static void slot_match_peer(mdf_ctx *ctx, mdf_job *sl)
         grow_block(peer->dev, peer->dev_bytes, sl->dev_bytes, true, sl->dev_bytes);
 }
 
+// The tail of every job kind, after its kernels have been enqueued on the compute stream: the scores (and the job's error word,
+// parked in a per-slot device word because the next job resets d_err) leave on the device-to-host stream behind an event, so the
+// next job's kernels do not queue behind this job's 32 MB result copy; `more` enqueues the job's other result copies on that
+// stream.  Both therefore live in the slot's device block, never in the arena.  On success the slot is handed out as *job.
+static int job_finish(mdf_job *sl, int rc, int n, const float *d_scores, size_t score_count, float *scores,
+                      const std::function<cudaError_t(cudaStream_t)> &more, mdf_job **job)
+{
+    mdf_ctx *ctx = sl->ctx;
+    cudaStream_t out_stream = ctx->stream;
+    if (rc == MDF_OK && n > 0) {
+        const int slot = (int)(sl - ctx->slots);
+        cudaError_t e = cudaMemcpyAsync(ctx->d_err + 2 + slot, ctx->d_err, sizeof(int), cudaMemcpyDeviceToDevice, ctx->stream);
+        if (e == cudaSuccess && ctx->d2h_stream) {
+            e = cudaEventRecord(ctx->path_done[slot], ctx->stream);
+            if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->d2h_stream, ctx->path_done[slot], 0);
+            if (e == cudaSuccess) out_stream = ctx->d2h_stream;
+        }
+        if (e == cudaSuccess) e = cudaMemcpyAsync(scores, d_scores, score_count * sizeof(float), cudaMemcpyDeviceToHost, out_stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(sl->h_err, ctx->d_err + 2 + slot, sizeof(int), cudaMemcpyDeviceToHost, out_stream);
+        if (e == cudaSuccess && more) e = more(out_stream);
+        if (e != cudaSuccess) { set_error("job: result copy failed: %s", cudaGetErrorString(e)); rc = MDF_ECUDA; }
+    }
+    if (rc != MDF_OK && ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);   // no input copy may outlive a failed call
+    cudaEventRecord(sl->done, out_stream);
+    if (rc != MDF_OK) return rc;
+    sl->busy = true;
+    *job = sl;
+    slot_match_peer(ctx, sl);
+    return MDF_OK;
+}
+
 // enqueue everything for flat inputs (already where they may be read asynchronously: pinned slot memory or caller buffers) and
 // hand the slot out as *job
 static int job_enqueue(mdf_model *m, mdf_job *sl, BatchInputs in, float thr2, int gen, float *scores, mdf_job **job)
@@ -1023,37 +1043,18 @@ static int job_enqueue(mdf_model *m, mdf_job *sl, BatchInputs in, float thr2, in
     }
     const auto t1 = std::chrono::steady_clock::now();
     if (rc == MDF_OK) rc = run_path(m, b, thr2, gen, 4, true);
-    cudaStream_t out_stream = ctx->stream;
-    if (rc == MDF_OK && n > 0) {
-        // the scores (and the job's error word, parked in a per-slot device word because the next job resets d_err) leave on the
-        // device-to-host stream behind an event: the next job's kernels do not queue behind this job's 32 MB result copy
-        const int slot = (int)(sl - ctx->slots);
-        cudaError_t e = cudaMemcpyAsync(ctx->d_err + 2 + slot, ctx->d_err, sizeof(int), cudaMemcpyDeviceToDevice, ctx->stream);
-        if (e == cudaSuccess && ctx->d2h_stream) {
-            e = cudaEventRecord(ctx->path_done[slot], ctx->stream);
-            if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->d2h_stream, ctx->path_done[slot], 0);
-            if (e == cudaSuccess) out_stream = ctx->d2h_stream;
-        }
-        if (e == cudaSuccess) e = cudaMemcpyAsync(scores, b->d_scores, (size_t)n * m->C * sizeof(float), cudaMemcpyDeviceToHost, out_stream);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(sl->h_err, ctx->d_err + 2 + slot, sizeof(int), cudaMemcpyDeviceToHost, out_stream);
-        if (e == cudaSuccess && pin) e = cudaMemcpyAsync(sl->pin_stats, b->d_nw_stats, (size_t)n * 12, cudaMemcpyDeviceToHost, out_stream);
-        if (e == cudaSuccess && pin && pin->ops && b->h_nw_off[n])
-            e = cudaMemcpyAsync(sl->pin_ops, b->d_ops, (size_t)b->h_nw_off[n], cudaMemcpyDeviceToHost, out_stream);
-        if (e != cudaSuccess) { set_error("mdf_path_submit: result copy failed: %s", cudaGetErrorString(e)); rc = MDF_ECUDA; }
-    }
-    if (rc != MDF_OK && ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);   // no input copy may outlive a failed call
-    cudaEventRecord(sl->done, out_stream);
     if (timing) {
         const auto t2 = std::chrono::steady_clock::now();
         auto ms = [](auto a, auto b2) { return std::chrono::duration<double, std::milli>(b2 - a).count(); };
         fprintf(stderr, "[mdf_path_submit] n=%d: batch build + H2D %.2f ms, enqueue (host) %.2f ms\n", n, ms(t0, t1), ms(t1, t2));
     }
-    if (rc != MDF_OK) return rc;
     sl->n_pairs = pin ? n : 0;
-    sl->busy = true;
-    *job = sl;
-    slot_match_peer(ctx, sl);
-    return MDF_OK;
+    auto pair_outputs = [&](cudaStream_t s) {
+        cudaError_t e = cudaMemcpyAsync(sl->pin_stats, b->d_nw_stats, (size_t)n * 12, cudaMemcpyDeviceToHost, s);
+        if (e == cudaSuccess && pin->ops && b->h_nw_off[n]) e = cudaMemcpyAsync(sl->pin_ops, b->d_ops, (size_t)b->h_nw_off[n], cudaMemcpyDeviceToHost, s);
+        return e;
+    };
+    return job_finish(sl, rc, n, b->d_scores, (size_t)n * m->C, scores, pin ? pair_outputs : std::function<cudaError_t(cudaStream_t)>(), job);
 }
 
 extern "C" int mdf_path_submit(mdf_model *m, int n, const char *seq, const int64_t *seq_off, const float *coords,
@@ -1146,6 +1147,55 @@ extern "C" int mdf_path_submit_pairs(mdf_model *m, int n, const char *const *que
     if (ops) { sl->out_ops_off.assign(ops_off, ops_off + n); sl->nw_off = plan.off; }
     return job_enqueue(m, sl, {.n = n, .seq = pk.at(S), .seq_off = pk.off(S), .coords = (const float *)pk.at(R), .coord_off = pk.off(R),
                                .pairs = &pin}, thr2, gen, scores, job);
+}
+
+// mdf_cnn_forward as a job from per-sequence pointers.  The sequences and the per-tile table are packed into the slot's pinned
+// block and copied on the copy stream into the slot's device block, which also holds the pooled features and the scores; the
+// head's temporaries come from the arena, in stream order.
+extern "C" int mdf_cnn_submit_ragged(mdf_cnn_model *m, int n, const char *const *seq, const int *seq_len, float *scores, mdf_job **job)
+{
+    MDF_REQUIRE(m && scores && job && n >= 0, "mdf_cnn_submit_ragged: bad arguments");
+    MDF_REQUIRE(n == 0 || (seq && seq_len), "mdf_cnn_submit_ragged: input arrays missing");
+    mdf_ctx *ctx = m->ctx;
+    MDF_CUDA(cudaSetDevice(ctx->device));
+    CnnBatch v;
+    v.n = n;
+    for (int p = 0; p < n; ++p) {
+        // ReduceMax over an empty residue axis is an error in the reference graph as well
+        MDF_REQUIRE(seq_len[p] >= 1, "mdf_cnn_submit_ragged: sequence %d is empty (the max-pool over residues needs at least one)", p);
+        MDF_REQUIRE(seq[p], "mdf_cnn_submit_ragged: sequence %d is missing", p);
+        v.T += seq_len[p];
+        v.n_tiles += cdiv(seq_len[p], 128);
+        MDF_REQUIRE(v.T < (int64_t)1 << 31, "mdf_cnn_submit_ragged: more than 2^31 residues in one batch");
+    }
+    mdf_job *sl = nullptr;
+    MDF_TRY(slot_acquire(ctx, &sl));
+    RaggedPack pk(n);
+    const int S = pk.column(seq_len, 1, seq), TILES = pk.region((size_t)v.n_tiles * sizeof(int4));
+    MDF_TRY(pinned_block(sl->pin, sl->pin_bytes, pk.place(nullptr), " for a job slot"));
+    pk.place(sl->pin);
+    pk.pack(pack_threads(ctx, n));
+    int4 *tiles = reinterpret_cast<int4 *>(pk.at(TILES));
+    cnn_tiles(n, pk.off(S), tiles);
+    const size_t bytes = cnn_carve(m, v, nullptr);
+    if (const cudaError_t e = grow_block(sl->dev, sl->dev_bytes, bytes, true)) {
+        set_error("cudaMalloc(%zu bytes) for a job slot failed: %s", with_headroom(bytes), cudaGetErrorString(e));
+        return MDF_ENOMEM;
+    }
+    cnn_carve(m, v, sl->dev);
+    ArenaScope scope(ctx);
+    int rc = MDF_OK;
+    if (n > 0) {
+        // the slot's previous job has finished (slot_acquire), so its block may be overwritten while the other slot's job computes
+        cudaStream_t cs = ctx->copy_stream;
+        cudaError_t e = cudaMemcpyAsync(v.d_seq, pk.at(S), (size_t)v.T, cudaMemcpyHostToDevice, cs);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(v.d_tile_info, tiles, (size_t)v.n_tiles * sizeof(int4), cudaMemcpyHostToDevice, cs);
+        if (e == cudaSuccess) e = cudaEventRecord(ctx->copy_done, cs);
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->stream, ctx->copy_done, 0);
+        if (e != cudaSuccess) { set_error("mdf_cnn_submit_ragged: input copy failed: %s", cudaGetErrorString(e)); rc = MDF_ECUDA; }
+        if (rc == MDF_OK) rc = cnn_run(m, v);
+    }
+    return job_finish(sl, rc, n, v.d_scores, (size_t)n * m->C, scores, {}, job);
 }
 
 extern "C" int mdf_path_wait(mdf_job *job)

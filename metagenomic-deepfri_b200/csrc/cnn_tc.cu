@@ -26,33 +26,9 @@
 // ints) per protein and channel.  HBM traffic: 1 byte per residue in, 4 * sum(F) bytes per protein out.
 #include <algorithm>
 
+#include "cnn.cuh"
 #include "gemm_tc.cuh"
 #include "tc_engine.cuh"
-
-struct mdf_cnn_model {
-    mdf_ctx *ctx = nullptr;
-    int n_conv = 0, width[MDF_MAX_CONV] = {0}, filters[MDF_MAX_CONV] = {0}, pl[MDF_MAX_CONV] = {0}, kb[MDF_MAX_CONV] = {0},
-        choff[MDF_MAX_CONV] = {0};
-    int Ctot = 0, C = 0, pl_max = 0, n_items = 0;
-    double macs_per_residue = 0.0;            // algorithmic: 26 * sum(w_c * F_c)
-    __half *W[MDF_MAX_CONV] = {nullptr};      // weight images [F_c rows x kb_c * 64]
-    uint4 *ktab = nullptr;                    // per conv kb_c entries: the four K steps of a k-block as {start / 16 | LBO / 16 << 16}
-    int ktab_off[MDF_MAX_CONV] = {0};
-    double issued_macs_per_row = 0.0;         // 16 * K steps * F summed over the convs (what the kernel issues per padded row)
-    float *scale = nullptr, *shift = nullptr;
-    __half *out_W[2] = {nullptr, nullptr};    // [2C rows x Ctot k] hi / residual * 2^11
-    float *out_b_pad = nullptr;
-    std::vector<void *> owned;
-    // resident batch (mdf_cnn_upload)
-    int n = 0, n_tiles = 0;
-    int64_t T = 0;
-    void *block = nullptr;
-    size_t block_bytes = 0;
-    char *d_seq = nullptr;
-    uint8_t *d_idx = nullptr;
-    int4 *d_tile_info = nullptr;
-    float *d_pooled = nullptr, *d_scores = nullptr;
-};
 
 namespace mdf {
 namespace tc {
@@ -353,7 +329,72 @@ static void cnn_free_batch(mdf_cnn_model *m)
     if (m->block) cudaFree(m->block);
     m->block = nullptr;
     m->block_bytes = 0;
-    m->n = 0; m->T = 0; m->n_tiles = 0;
+    m->batch = CnnBatch();
+}
+
+int cnn_tiles(int n, const int64_t *seq_off, int4 *tiles)
+{
+    int k = 0;
+    for (int p = 0; p < n; ++p) {
+        const int64_t L = seq_off[p + 1] - seq_off[p];
+        for (int r0 = 0; r0 < L; r0 += 128, ++k)
+            if (tiles) tiles[k] = make_int4(p, r0, (int)L, (int)seq_off[p]);
+    }
+    return k;
+}
+
+size_t cnn_carve(const mdf_cnn_model *m, CnnBatch &v, char *base)
+{
+    Carver carve;
+    carve.base = base;
+    v.d_seq = carve.take<char>((size_t)v.T);
+    v.d_idx = carve.take<uint8_t>((size_t)v.T);
+    v.d_tile_info = carve.take<int4>((size_t)v.n_tiles);
+    v.d_pooled = carve.take<float>((size_t)v.n * m->Ctot);
+    v.d_scores = carve.take<float>((size_t)v.n * m->C);
+    return align_up(carve.top, 256);
+}
+
+int cnn_run(mdf_cnn_model *m, const CnnBatch &v)
+{
+    mdf_ctx *ctx = m->ctx;
+    const int n = v.n;
+    const int ld = (2 * m->C + 3) / 4 * 4;
+    const size_t rows_pad = (size_t)cdiv(n, 128) * 128;
+    MDF_TRY(ctx->reserve(3 * align_up(rows_pad * m->Ctot * 2, 256) + align_up((size_t)n * ld * 4, 256) + 4096));
+    ArenaScope scope(ctx);
+    MDF_CUDA(cudaMemsetAsync(ctx->d_err, 0, sizeof(int), ctx->stream));
+    MDF_TRY(launch_seq_to_idx(ctx, v.T, v.d_seq, v.d_idx));
+    MDF_CUDA(cudaMemsetAsync(v.d_pooled, 0, (size_t)n * m->Ctot * 4, ctx->stream));
+    {
+        ProfScope ps(ctx, "cnn_conv", 2.0 * m->macs_per_residue * (double)v.T);
+        CnnArgs a;
+        memset(&a, 0, sizeof a);
+        a.n_tiles = v.n_tiles; a.n_groups = cdiv(v.n_tiles, CNN_TILES); a.n_items = m->n_items; a.pl_max = m->pl_max; a.Ctot = m->Ctot;
+        a.tile_info = v.d_tile_info; a.idx = v.d_idx; a.scale = m->scale; a.shift = m->shift; a.ktab = m->ktab;
+        a.pooled = reinterpret_cast<int *>(v.d_pooled);
+        int item = 0;
+        for (int c = 0; c < m->n_conv; ++c) {
+            a.W[c] = m->W[c]; a.kb[c] = (short)m->kb[c]; a.ktab_off[c] = m->ktab_off[c]; a.choff[c] = m->choff[c];
+            for (int fb = 0; fb < m->filters[c] / 128; ++fb, ++item) { a.item_conv[item] = (unsigned char)c; a.item_fb[item] = (unsigned char)fb; }
+        }
+        {
+            auto kern = cnn_conv_kernel<1>;
+            MDF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CNN_SMEM));
+            const int grid = std::min(a.n_groups, ctx->sm_count);
+            a.rounds = cdiv(a.n_groups, grid);
+            kern<<<grid, CNN_THREADS, CNN_SMEM, ctx->stream>>>(a);
+            MDF_LAUNCH_CHECK(ctx);
+        }
+    }
+    {
+        ProfScope ps(ctx, "cnn_head", 2.0 * n * (double)m->Ctot * 2 * m->C);
+        float *logits = nullptr;
+        MDF_TRY(ctx->alloc_n(&logits, (size_t)n * ld));
+        MDF_TRY(tc_dense_split(ctx, n, v.d_pooled, m->Ctot, m->out_W, 2 * m->C, ld, m->out_b_pad, 0, logits));
+        MDF_TRY(tc_softmax0_strided(ctx, n, m->C, ld, logits, v.d_scores));
+    }
+    return MDF_OK;
 }
 
 }  // namespace mdf
@@ -469,21 +510,18 @@ extern "C" int mdf_cnn_upload(mdf_cnn_model *m, int n, const char *seq, const in
     mdf_ctx *ctx = m->ctx;
     MDF_CUDA(cudaSetDevice(ctx->device));
     MDF_CUDA(cudaStreamSynchronize(ctx->stream));
-    m->n = 0; m->T = 0; m->n_tiles = 0;
+    m->batch = CnnBatch();
     if (n == 0) return MDF_OK;
     MDF_REQUIRE(seq_off[0] == 0, "mdf_cnn_upload: seq_off[0] must be 0");
     const int64_t T = seq_off[n];
     MDF_REQUIRE(T < (int64_t)1 << 31, "mdf_cnn_upload: more than 2^31 residues in one batch");
-    std::vector<int4> tiles;
-    for (int p = 0; p < n; ++p) {
-        const int64_t L = seq_off[p + 1] - seq_off[p];
-        // ReduceMax over an empty residue axis is an error in the reference graph as well
-        MDF_REQUIRE(L >= 1, "mdf_cnn_upload: sequence %d is empty (the max-pool over residues needs at least one)", p);
-        for (int r0 = 0; r0 < L; r0 += 128) tiles.push_back(make_int4(p, r0, (int)L, (int)seq_off[p]));
-    }
-    const size_t b_seq = align_up((size_t)T, 256), b_idx = align_up((size_t)T, 256), b_tiles = align_up(tiles.size() * sizeof(int4), 256),
-                 b_pool = align_up((size_t)n * m->Ctot * 4, 256), b_sc = align_up((size_t)n * m->C * 4, 256);
-    const size_t need = b_seq + b_idx + b_tiles + b_pool + b_sc;
+    for (int p = 0; p < n; ++p)          // ReduceMax over an empty residue axis is an error in the reference graph as well
+        MDF_REQUIRE(seq_off[p + 1] - seq_off[p] >= 1, "mdf_cnn_upload: sequence %d is empty (the max-pool over residues needs at least one)", p);
+    std::vector<int4> tiles(cnn_tiles(n, seq_off, nullptr));
+    cnn_tiles(n, seq_off, tiles.data());
+    CnnBatch v;
+    v.n = n; v.T = T; v.n_tiles = (int)tiles.size();
+    const size_t need = cnn_carve(m, v, nullptr);
     if (need > m->block_bytes) {            // the resident block only grows: back-to-back batches reuse it
         cnn_free_batch(m);
         const size_t want = need + need / 8;
@@ -491,15 +529,10 @@ extern "C" int mdf_cnn_upload(mdf_cnn_model *m, int n, const char *seq, const in
         if (e != cudaSuccess) { cudaGetLastError(); m->block = nullptr; set_error("mdf_cnn_upload: cudaMalloc(%zu) failed: %s", want, cudaGetErrorString(e)); return MDF_ENOMEM; }
         m->block_bytes = want;
     }
-    char *p = static_cast<char *>(m->block);
-    m->d_seq = p; p += b_seq;
-    m->d_idx = reinterpret_cast<uint8_t *>(p); p += b_idx;
-    m->d_tile_info = reinterpret_cast<int4 *>(p); p += b_tiles;
-    m->d_pooled = reinterpret_cast<float *>(p); p += b_pool;
-    m->d_scores = reinterpret_cast<float *>(p);
-    m->n = n; m->T = T; m->n_tiles = (int)tiles.size();
-    MDF_CUDA(cudaMemcpyAsync(m->d_seq, seq, (size_t)T, cudaMemcpyHostToDevice, ctx->stream));
-    MDF_CUDA(cudaMemcpyAsync(m->d_tile_info, tiles.data(), tiles.size() * sizeof(int4), cudaMemcpyHostToDevice, ctx->stream));
+    cnn_carve(m, v, static_cast<char *>(m->block));
+    m->batch = v;
+    MDF_CUDA(cudaMemcpyAsync(v.d_seq, seq, (size_t)T, cudaMemcpyHostToDevice, ctx->stream));
+    MDF_CUDA(cudaMemcpyAsync(v.d_tile_info, tiles.data(), tiles.size() * sizeof(int4), cudaMemcpyHostToDevice, ctx->stream));
     MDF_CUDA(cudaStreamSynchronize(ctx->stream));      // `tiles` is a local
     return MDF_OK;
 }
@@ -507,57 +540,21 @@ extern "C" int mdf_cnn_upload(mdf_cnn_model *m, int n, const char *seq, const in
 extern "C" int mdf_cnn_run(mdf_cnn_model *m)
 {
     MDF_REQUIRE(m, "mdf_cnn_run: bad arguments");
-    if (m->n == 0) return MDF_OK;
-    mdf_ctx *ctx = m->ctx;
-    MDF_CUDA(cudaSetDevice(ctx->device));
-    const int n = m->n;
-    const int ld = (2 * m->C + 3) / 4 * 4;
-    const size_t rows_pad = (size_t)cdiv(n, 128) * 128;
-    MDF_TRY(ctx->reserve(3 * align_up(rows_pad * m->Ctot * 2, 256) + align_up((size_t)n * ld * 4, 256) + 4096));
-    ArenaScope scope(ctx);
-    MDF_CUDA(cudaMemsetAsync(ctx->d_err, 0, sizeof(int), ctx->stream));
-    MDF_TRY(launch_seq_to_idx(ctx, m->T, m->d_seq, m->d_idx));
-    MDF_CUDA(cudaMemsetAsync(m->d_pooled, 0, (size_t)n * m->Ctot * 4, ctx->stream));
-    {
-        ProfScope ps(ctx, "cnn_conv", 2.0 * m->macs_per_residue * (double)m->T);
-        CnnArgs a;
-        memset(&a, 0, sizeof a);
-        a.n_tiles = m->n_tiles; a.n_groups = cdiv(m->n_tiles, CNN_TILES); a.n_items = m->n_items; a.pl_max = m->pl_max; a.Ctot = m->Ctot;
-        a.tile_info = m->d_tile_info; a.idx = m->d_idx; a.scale = m->scale; a.shift = m->shift; a.ktab = m->ktab;
-        a.pooled = reinterpret_cast<int *>(m->d_pooled);
-        int item = 0;
-        for (int c = 0; c < m->n_conv; ++c) {
-            a.W[c] = m->W[c]; a.kb[c] = (short)m->kb[c]; a.ktab_off[c] = m->ktab_off[c]; a.choff[c] = m->choff[c];
-            for (int fb = 0; fb < m->filters[c] / 128; ++fb, ++item) { a.item_conv[item] = (unsigned char)c; a.item_fb[item] = (unsigned char)fb; }
-        }
-        {
-            auto kern = cnn_conv_kernel<1>;
-            MDF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CNN_SMEM));
-            const int grid = std::min(a.n_groups, ctx->sm_count);
-            a.rounds = cdiv(a.n_groups, grid);
-            kern<<<grid, CNN_THREADS, CNN_SMEM, ctx->stream>>>(a);
-            MDF_LAUNCH_CHECK(ctx);
-        }
-    }
-    {
-        ProfScope ps(ctx, "cnn_head", 2.0 * n * (double)m->Ctot * 2 * m->C);
-        float *logits = nullptr;
-        MDF_TRY(ctx->alloc_n(&logits, (size_t)n * ld));
-        MDF_TRY(tc_dense_split(ctx, n, m->d_pooled, m->Ctot, m->out_W, 2 * m->C, ld, m->out_b_pad, 0, logits));
-        MDF_TRY(tc_softmax0_strided(ctx, n, m->C, ld, logits, m->d_scores));
-    }
-    return MDF_OK;
+    if (m->batch.n == 0) return MDF_OK;
+    MDF_CUDA(cudaSetDevice(m->ctx->device));
+    return cnn_run(m, m->batch);
 }
 
 extern "C" int mdf_cnn_fetch(mdf_cnn_model *m, float *scores, float *pooled)
 {
     MDF_REQUIRE(m, "mdf_cnn_fetch: bad arguments");
     mdf_ctx *ctx = m->ctx;
+    const CnnBatch &v = m->batch;
     MDF_CUDA(cudaSetDevice(ctx->device));
-    if (m->n && scores)
-        MDF_CUDA(cudaMemcpyAsync(scores, m->d_scores, (size_t)m->n * m->C * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    if (m->n && pooled)
-        MDF_CUDA(cudaMemcpyAsync(pooled, m->d_pooled, (size_t)m->n * m->Ctot * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    if (v.n && scores)
+        MDF_CUDA(cudaMemcpyAsync(scores, v.d_scores, (size_t)v.n * m->C * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    if (v.n && pooled)
+        MDF_CUDA(cudaMemcpyAsync(pooled, v.d_pooled, (size_t)v.n * m->Ctot * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     MDF_CUDA(cudaMemcpyAsync(ctx->h_err, ctx->d_err, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
     MDF_CUDA(cudaStreamSynchronize(ctx->stream));
     return ctx->check_device_error("cnn forward");

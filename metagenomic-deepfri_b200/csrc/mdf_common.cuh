@@ -43,6 +43,18 @@ __host__ __device__ __forceinline__ int packed_row_words(int L) { return ((L + 1
 static inline int cdiv(int a, int b) { return (a + b - 1) / b; }
 static inline int64_t cdiv64(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
+struct Carver {   // sub-allocates one block; first pass (base == nullptr) only measures
+    char *base = nullptr;
+    size_t top = 0;
+    template <typename T>
+    T *take(size_t count)
+    {
+        size_t off = align_up(top, 256);
+        top = off + count * sizeof(T);
+        return base ? reinterpret_cast<T *>(base + off) : nullptr;
+    }
+};
+
 }  // namespace mdf
 
 // One of the two job slots of a context (mdf_path_submit* / mdf_path_wait): the device block that holds a transient batch's inputs,

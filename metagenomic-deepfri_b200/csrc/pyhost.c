@@ -9,6 +9,7 @@
  *
  *   submit_ragged(fn_addr, model_addr, seqs, gapped_query, gapped_target, coords, thr2, gen, scores_addr) -> (rc, job_addr)
  *   submit_pairs(fn_addr, model_addr, queries, targets, coords, matrix_addr, alphabet, ...) -> (rc, job_addr)
+ *   submit_sequences(fn_addr, model_addr, seqs, scores_addr) -> (rc, job_addr)
  *   pointers(strings) -> (bytes ptr-array, bytes len-array)      [used for the alignment / ingest entry points]
  *   cmap_ragged(fn_addr, ctx_addr, gapped_query, gapped_target, coords, thr2, gen, out_addr, out_words) -> (rc, packed_off, seq_off)
  *
@@ -209,6 +210,33 @@ static PyObject *submit_pairs(PyObject *self, PyObject *args)
     return result;
 }
 
+typedef struct mdf_cnn_model mdf_cnn_model;
+typedef int (*submit_sequences_fn)(mdf_cnn_model *, int, const char *const *, const int *, float *, mdf_job **);
+
+/* submit_sequences(fn_addr, model_addr, seqs, scores_addr) -> (rc, job_addr)
+ * the sequence-only DeepCNN branch: calls mdf_cnn_submit_ragged with the GIL released */
+static PyObject *submit_sequences(PyObject *self, PyObject *args)
+{
+    unsigned long long fn_addr, model_addr, scores_addr;
+    PyObject *seqs;
+    if (!PyArg_ParseTuple(args, "KKOK", &fn_addr, &model_addr, &seqs, &scores_addr)) return NULL;
+    Column c[1] = {{"seqs", TEXT, seqs}};
+    Py_ssize_t n;
+    PyObject *result = NULL;
+    if (collect(c, 1, "", "sequence too long", &n) == 0) {
+        mdf_job *job = NULL;
+        int rc;
+        submit_sequences_fn fn = (submit_sequences_fn)(uintptr_t)fn_addr;
+        Py_BEGIN_ALLOW_THREADS
+        rc = fn((mdf_cnn_model *)(uintptr_t)model_addr, (int)n, (const char *const *)c[0].ptr, c[0].len, (float *)(uintptr_t)scores_addr,
+                &job);
+        Py_END_ALLOW_THREADS
+        result = Py_BuildValue("iK", rc, (unsigned long long)(uintptr_t)job);
+    }
+    release(c, 1);
+    return result;
+}
+
 /* pointers(list of str / bytes) -> (ptr-array as bytes [n x 8], int32 length array as bytes [n x 4]); the pointers stay valid as
  * long as the list's items live */
 static PyObject *pointers(PyObject *self, PyObject *arg)
@@ -277,6 +305,7 @@ static PyMethodDef methods[] = {
     {"cmap_ragged", cmap_ragged, METH_VARARGS, "collect per-alignment pointers and call mdf_cmap_build_transfer_ragged (GIL released)"},
     {"submit_ragged", submit_ragged, METH_VARARGS, "collect per-protein pointers and call mdf_path_submit_ragged (GIL released)"},
     {"submit_pairs", submit_pairs, METH_VARARGS, "collect per-pair pointers and call mdf_path_submit_pairs (GIL released)"},
+    {"submit_sequences", submit_sequences, METH_VARARGS, "collect per-sequence pointers and call mdf_cnn_submit_ragged (GIL released)"},
     {"pointers", pointers, METH_O, "pointer / length arrays of a list of str or bytes"},
     {NULL, NULL, 0, NULL}};
 

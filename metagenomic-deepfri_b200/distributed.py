@@ -5,44 +5,67 @@ collective on the compute path (SURVEY.md §8e; the reference's loop over protei
 from __future__ import annotations
 
 from collections import deque
-from typing import Callable, Iterable, List, Optional, Sequence, Tuple
+from typing import Callable, Iterable, List, Optional, Sequence, Tuple, Union
 
 import numpy as np
 
-from .sharding import chunks_by_residues, lpt_bins
+from .sharding import ALPHA, BETA, chunks_by_residues, lpt_bins
 
 #: one chunk = one launch of the whole path; bounded by proteins and residues (HBM workspace ~ 6 KB per residue)
 CHUNK_PROTEINS, CHUNK_RESIDUES = 16384, 5_200_000
 
 
 def shard_job(lengths: Sequence[int], world: int, max_proteins: int = CHUNK_PROTEINS,
-              max_residues: int = CHUNK_RESIDUES) -> List[List[np.ndarray]]:
-    """LPT bins over `world` ranks, each cut into launch-sized chunks: `result[rank]` = list of protein-index arrays."""
-    return [chunks_by_residues(b, lengths, max_residues, max_proteins) for b in lpt_bins(lengths, world)]
+              max_residues: int = CHUNK_RESIDUES, alpha: float = ALPHA, beta: float = BETA) -> List[List[np.ndarray]]:
+    """LPT bins over `world` ranks, each cut into launch-sized chunks: `result[rank]` = list of protein-index arrays.  The bins
+    balance the cost alpha L^2 + beta L (`sharding.cost`): the GCN path's fit by default; the sequence-only DeepCNN branch works
+    per residue tile, with no L^2 term, so it shards with `alpha=0`."""
+    return [chunks_by_residues(b, lengths, max_residues, max_proteins) for b in lpt_bins(lengths, world, alpha, beta)]
 
 
-def stream_chunks(submit: Callable[[object, np.ndarray], object], chunks: Iterable[Tuple[object, int]], out: np.ndarray,
-                  depth: int = 2, on_done: Optional[Callable[[int, np.ndarray], None]] = None) -> None:
+def stream_chunks(submit: Callable[[object, np.ndarray], object], chunks: Iterable[Tuple[object, int]],
+                  out: Union[np.ndarray, Sequence[np.ndarray]], depth: int = 2,
+                  on_done: Optional[Callable[[int, np.ndarray], None]] = None) -> None:
     """Software pipeline over chunks: `submit(chunk, out_rows)` returns a job with `.wait()`; at most `depth` jobs are in flight,
-    so chunk k + 1 is packed and copied while chunk k computes (`Predictor.submit_structures`).  `chunks` yields
-    `(chunk, n_proteins)`; the scores of the chunks land in consecutive rows of `out`.  `on_done(k, rows)` runs after chunk k's
-    scores are on the host, while the following chunks compute (e.g. `ScoreBoard.put`)."""
+    so chunk k + 1 is packed and copied while chunk k computes (`Predictor.submit_structures`, `Predictor.submit_sequences`).
+    `chunks` yields `(chunk, n_proteins)`.  With one array as `out`, the scores of the chunks land in consecutive rows of it; with a
+    list of `depth` arrays (each with at least as many rows as the largest chunk), chunk k's scores land in the first n rows of
+    `out[k % depth]`, so only the chunks in flight hold result memory.  `on_done(k, rows)` runs after chunk k's scores are on the
+    host, while the following chunks compute (e.g. `ScoreBoard.put`), and before chunk k + depth is submitted - with a ring the
+    rows are overwritten after that.  If a submit, wait or `on_done` raises, the jobs still in flight are waited for (their own
+    errors dropped) before the exception propagates: a job that is never waited for would keep its context's slot busy."""
+    ring = isinstance(out, (list, tuple))
+    if ring and len(out) != depth:
+        raise ValueError(f"stream_chunks: a ring of result buffers needs exactly depth = {depth} arrays, got {len(out)}")
     jobs = deque()
     row = 0
-    for k, (chunk, n) in enumerate(chunks):
-        rows = out[row:row + n]
-        jobs.append((submit(chunk, rows), k, rows))
-        row += n
-        if len(jobs) >= depth:
+    try:
+        for k, (chunk, n) in enumerate(chunks):
+            if ring:
+                if n > len(out[k % depth]):
+                    raise ValueError(f"stream_chunks: chunk {k} has {n} rows, its ring buffer {len(out[k % depth])}")
+                rows = out[k % depth][:n]
+            else:
+                rows = out[row:row + n]
+            jobs.append((submit(chunk, rows), k, rows))
+            row += n
+            if len(jobs) >= depth:
+                j, kk, rr = jobs.popleft()
+                j.wait()
+                if on_done is not None:
+                    on_done(kk, rr)
+        while jobs:
             j, kk, rr = jobs.popleft()
             j.wait()
             if on_done is not None:
                 on_done(kk, rr)
-    while jobs:
-        j, kk, rr = jobs.popleft()
-        j.wait()
-        if on_done is not None:
-            on_done(kk, rr)
+    except BaseException:
+        for j, _, _ in jobs:
+            try:
+                j.wait()
+            except Exception:
+                pass
+        raise
 
 
 class ScoreBoard:

@@ -15,7 +15,8 @@ row per call.  Here the same rows come out of a few batched launches:
 
 Nothing here falls back to the CPU; sequences without structure (`alignment.coords is None`,
 `bio_utils.py:381-383`) are reported back so the caller can route them to the sequence-only branch
-(`run_prediction_loop(..., net_type="cnn")` over a `DeepCNN-MERGED_*` Predictor).
+(`run_prediction_loop(..., net_type="cnn")` over a `DeepCNN-MERGED_*` Predictor, which streams its chunks through
+`Predictor.submit_sequences`).
 """
 from __future__ import annotations
 
@@ -25,6 +26,7 @@ from typing import Dict, Iterable, List, Optional, Sequence, Tuple
 import numpy as np
 
 from .batching import pack_bits
+from .distributed import stream_chunks
 from .predict import Predictor
 
 #: proteins per upload are bounded by residues so that the workspace stays within a few tens of GB
@@ -50,12 +52,22 @@ def run_prediction_loop(predictor: Predictor, data_iterable: Iterable, data_len:
     bit-packed on the host and pushed through `Predictor.forward_batch` chunk by chunk."""
     items = list(data_iterable)
     if net_type == "cnn":
-        # items are (query_id, sequence) pairs (`pipeline.py:313-316`): the sequence-only DeepCNN branch
-        lengths = [len(s) for _, s in items]
-        for lo, hi in _chunks(lengths, max_residues):
-            scores = predictor.forward_sequences([s for _, s in items[lo:hi]])
-            for (query_id, _), vec in zip(items[lo:hi], scores):
+        # items are (query_id, sequence) pairs (`pipeline.py:313-316`): the sequence-only DeepCNN branch, two chunks in flight so
+        # that the next chunk's packing and copies overlap this chunk's kernels; rows are written per chunk, in input order
+        chunks = _chunks([len(s) for _, s in items], max_residues)
+        # one page-locked buffer per job in flight, reused chunk after chunk (rows are written out in on_done, before the buffer's
+        # next chunk is submitted): a device-to-host copy into pageable memory returns only once it has completed, so every
+        # submit would wait for its own chunk's kernels and nothing would overlap
+        import torch
+        rows_max = max((hi - lo for lo, hi in chunks), default=0)
+        ring = [torch.empty((rows_max, predictor.n_terms), dtype=torch.float32, pin_memory=True).numpy() for _ in range(2)]
+
+        def write(k: int, rows: np.ndarray) -> None:
+            lo, hi = chunks[k]
+            for (query_id, _), vec in zip(items[lo:hi], rows):
                 tsv_writer.writerow([query_id, net_type] + vec.tolist())
+        stream_chunks(lambda c, rows: predictor.submit_sequences([s for _, s in items[c[0]:c[1]]], out=rows),
+                      ((c, c[1] - c[0]) for c in chunks), ring, depth=2, on_done=write)
         return
     if net_type != "gcn":
         raise ValueError(f"run_prediction_loop: unknown net_type {net_type!r}")

@@ -10,8 +10,8 @@ kernels over many proteins per launch; `forward_pass` is a batch of one.
 
 A single-input `.onnx` file (the `DeepCNN-MERGED_*` models) is the reference's sequence-only CNN
 branch: `forward_pass(seqres)` with `cmap=None` (`predict.pyx:91-95`) and the batched
-`forward_sequences` run it through the tcgen05 convolution kernel (`csrc/cnn_tc.cu`).  There is no
-CPU or library fallback on either branch.
+`forward_sequences` (or its asynchronous form `submit_sequences`) run it through the tcgen05 convolution kernel
+(`csrc/cnn_tc.cu`).  There is no CPU or library fallback on either branch.
 """
 from __future__ import annotations
 
@@ -255,7 +255,7 @@ class PairJob:
 
 
 class PathJob:
-    """An in-flight `Predictor.submit_structures` call."""
+    """An in-flight `Predictor.submit_structures` or `Predictor.submit_sequences` call."""
 
     def __init__(self, pred: "Predictor", handle: int, out: np.ndarray, inputs):
         self._pred, self._handle, self._out, self._inputs = pred, handle, out, inputs
@@ -320,6 +320,22 @@ class Predictor:
             return out
         _lib.check(_lib.lib().mdf_cnn_forward(self._handle, n, seq_bytes, _lib.lp(seq_off), out.ctypes.data))
         return out
+
+    def submit_sequences(self, seqs: Sequence[str], out: Optional[np.ndarray] = None) -> "PathJob":
+        """Asynchronous `forward_sequences`: packs the n sequences into pinned staging memory (C, worker threads, GIL released),
+        enqueues H2D + every kernel + the D2H of the scores and returns a `PathJob`; `job.wait()` returns the score matrix.
+        The jobs share the context's two slots with `submit_structures`, so the next chunk's packing and copies overlap this
+        chunk's kernels.  An empty sequence raises here; a residue outside the alphabet raises at `wait()`."""
+        if not self.is_cnn:
+            raise ValueError("submit_sequences needs a sequence-only DeepCNN model; this Predictor holds a GCN head")
+        n = len(seqs)
+        if out is None:
+            out = np.empty((n, self.n_terms), np.float32)
+        if out.shape != (n, self.n_terms) or out.dtype != np.float32 or not out.flags["C_CONTIGUOUS"]:
+            raise ValueError("out must be a C-contiguous float32 array of shape (n, n_terms)")
+        rc, job = _lib.pyhost().submit_sequences(_lib.fn_addr("mdf_cnn_submit_ragged"), self._handle.value, seqs, out.ctypes.data)
+        _lib.check(rc)
+        return PathJob(self, job, out, (seqs, None, None))
 
     def upload_sequences(self, seqs: Sequence[str]) -> int:
         """Keep n sequences resident in HBM for `run_sequences` / `fetch_sequences` (bench); returns the bytes copied."""
