@@ -82,7 +82,8 @@ int mdf_align_contact_map(mdf_ctx *ctx, const char *q_aln, const char *t_aln, in
  * alignment columns [aln_off[p], aln_off[p+1]) of q_aln / t_aln; output rows of Lq[p] =
  * seq_off[p+1]-seq_off[p] residues.  Exactly one of packed_out / dense_out may be non-NULL per
  * call: packed_out uint32 at word offset packed_off[p]; dense_out int32 [Lq,Lq] at element
- * offset dense_off[p]. */
+ * offset dense_off[p].  Synchronous: runs as a job in the context's synchronous slot and waits for
+ * it, so it works while two asynchronous jobs are in flight and leaves them undisturbed. */
 int mdf_cmap_build_transfer(mdf_ctx *ctx, int n,
                             const float *coords, const int64_t *coord_off,
                             const char *q_aln, const char *t_aln, const int64_t *aln_off,
@@ -95,7 +96,8 @@ int mdf_cmap_build_transfer(mdf_ctx *ctx, int n,
  * '-'), writes the canonical offsets seq_off_out[n+1] (residues) and packed_off_out[n+1] (uint32 words, row p: Lq *
  * mdf_packed_row_words(Lq)), packs the inputs into pinned staging memory on MDF_HOST_THREADS host threads and runs the fused
  * kernels.  packed_out == NULL: sizes only (host work, no GPU, ctx may be NULL) - call once to size the output, once to fill it;
- * packed_capacity_words < packed_off_out[n] is MDF_EINVAL.  packed_out may be pageable or pinned. */
+ * packed_capacity_words < packed_off_out[n] is MDF_EINVAL.  packed_out may be pageable or pinned.  Synchronous, like
+ * mdf_cmap_build_transfer. */
 int mdf_cmap_build_transfer_ragged(mdf_ctx *ctx, int n,
                                    const float *const *coords, const int *coord_rows,
                                    const char *const *q_aln, const char *const *t_aln, const int *aln_len,
@@ -157,7 +159,9 @@ int mdf_model_get_engine(const mdf_model *model);
 
 /* ---- predict.pyx:75-102  Predictor.forward_pass(seqres, cmap) ---------------------------------
  * seq: ASCII residues (alphabet "-DGULNTKHYWCPVSOIEFXQABZRM", anything else -> MDF_EINVAL);
- * cmap: host int32 [L, L] holding 0/1 (other values -> MDF_EINVAL); scores: host float32 [C]. */
+ * cmap: host int32 [L, L] holding 0/1 (other values -> MDF_EINVAL); scores: host float32 [C].
+ * A bad residue is reported before a bad map.  This and mdf_gcn_forward_packed are synchronous: each runs as a job in the
+ * context's synchronous slot and waits for it, so they work while two asynchronous jobs are in flight and leave them undisturbed. */
 int mdf_gcn_forward_dense(mdf_model *model, const char *seq, int L, const int32_t *cmap, float *scores);
 
 /* batched GCN forward on bit-packed maps (host buffers): scores host float32 [n, C] */
@@ -283,16 +287,19 @@ int mdf_cnn_model_create(mdf_ctx *ctx, const mdf_cnn_desc *desc, mdf_cnn_model *
 int mdf_cnn_model_destroy(mdf_cnn_model *model);
 /* same from a single-input `DeepCNN-*.onnx` file (conv bias + BatchNormalization folded into scale / shift while loading) */
 int mdf_cnn_model_load(mdf_ctx *ctx, const char *onnx_path, mdf_cnn_model **out);
-/* n sequences (ASCII residues, CSR offsets; every sequence needs >= 1 residue) -> scores host float32 [n, C] */
+/* n sequences (ASCII residues, CSR offsets; every sequence needs >= 1 residue) -> scores host float32 [n, C].  Synchronous:
+ * runs as a job in the context's synchronous slot and waits for it, so it works while two asynchronous jobs are in flight and
+ * leaves them undisturbed.  It does not touch the resident batch of mdf_cnn_upload: mdf_cnn_fetch after it returns the last
+ * mdf_cnn_run's results, not this call's. */
 int mdf_cnn_forward(mdf_cnn_model *model, int n, const char *seq, const int64_t *seq_off, float *scores);
 /* same with the sequences already resident: upload once, run many times (bench `value`), fetch */
 int mdf_cnn_upload(mdf_cnn_model *model, int n, const char *seq, const int64_t *seq_off);
 int mdf_cnn_run(mdf_cnn_model *model);
 int mdf_cnn_fetch(mdf_cnn_model *model, float *scores /* host [n, C] */, float *pooled /* host [n, sum filters] or NULL */);
 /* Asynchronous mdf_cnn_forward from per-sequence pointers (pipeline.py:607-613 holds one str per unaligned query).  Takes one of
- * the context's two job slots - the same slots mdf_path_submit* use, so CNN and GCN jobs may be in flight together - packs the
- * sequences into the slot's pinned block on MDF_HOST_THREADS threads, enqueues H2D, encode, conv, head and the D2H of the
- * scores, and returns; mdf_path_wait completes the job.  Every sequence needs >= 1 residue (MDF_EINVAL here, naming the index);
+ * the context's two asynchronous job slots - the same slots mdf_path_submit* use, so CNN and GCN jobs may be in flight
+ * together - packs the sequences into the slot's pinned block on MDF_HOST_THREADS threads, enqueues H2D, encode, conv, head
+ * and the D2H of the scores, and returns; mdf_path_wait completes the job.  Every sequence needs >= 1 residue (MDF_EINVAL here, naming the index);
  * a residue outside the alphabet is reported by mdf_path_wait ("Invalid character in sequence").  The caller's strings may be
  * released when the call returns; `scores` (host float32 [n, C]) must stay valid until mdf_path_wait returns. */
 int mdf_cnn_submit_ragged(mdf_cnn_model *model, int n, const char *const *seq, const int *seq_len, float *scores, mdf_job **job);

@@ -70,15 +70,13 @@ int mdf_ctx::alloc(void **out, size_t bytes)
     return MDF_OK;
 }
 
-int mdf_ctx::check_device_error(const char *where)
+int mdf::device_error(const char *where, int code)
 {
-    // caller has synchronised the stream after copying d_err into h_err
-    const int e = *h_err;
-    if (e == 0) return MDF_OK;
-    const char *what = e == MDF_DERR_BAD_RESIDUE ? "Invalid character in sequence"
-                     : e == MDF_DERR_BAD_CMAP    ? "contact map holds values other than 0/1"
-                     : e == MDF_DERR_LQ_MISMATCH ? "query sequence length does not match the gap-stripped query alignment"
-                                                 : "unknown device error";
+    if (code == 0) return MDF_OK;
+    const char *what = code == MDF_DERR_BAD_RESIDUE ? "Invalid character in sequence"
+                     : code == MDF_DERR_BAD_CMAP    ? "contact map holds values other than 0/1"
+                     : code == MDF_DERR_LQ_MISMATCH ? "query sequence length does not match the gap-stripped query alignment"
+                                                    : "unknown device error";
     set_error("%s: %s", where, what);
     return MDF_EINVAL;
 }
@@ -122,15 +120,17 @@ extern "C" int mdf_ctx_create(int device, void *arena, size_t arena_bytes, void 
     MDF_CUDA(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
     MDF_CUDA(cudaEventCreateWithFlags(&c->copy_done, cudaEventDisableTiming));
     MDF_CUDA(cudaStreamCreateWithFlags(&c->d2h_stream, cudaStreamNonBlocking));
-    for (int i = 0; i < 2; ++i) MDF_CUDA(cudaEventCreateWithFlags(&c->path_done[i], cudaEventDisableTiming));
+    for (auto &e : c->path_done) MDF_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     MDF_CUDA(cudaMalloc((void **)&c->d_err, 256));
     MDF_CUDA(cudaMemset(c->d_err, 0, 256));
     MDF_CUDA(cudaMallocHost((void **)&c->h_err, 256));
     *c->h_err = 0;
     for (auto &sl : c->slots) {
+        const int i = (int)(&sl - c->slots);
         sl.ctx = c;
         MDF_CUDA(cudaEventCreateWithFlags(&sl.done, cudaEventDisableTiming));
-        sl.h_err = c->h_err + 8 + 8 * (int)(&sl - c->slots);
+        sl.d_errs = c->d_err + 2 + 2 * i;
+        sl.h_err = c->h_err + 8 + 8 * i;
         sl.h_err[0] = sl.h_err[1] = 0;
     }
     if (const char *e = getenv("MDF_HOST_THREADS")) c->host_threads = std::max(1, std::min(64, atoi(e)));
@@ -156,8 +156,7 @@ extern "C" int mdf_ctx_destroy(mdf_ctx *c)
     if (c->copy_stream) { cudaStreamSynchronize(c->copy_stream); cudaStreamDestroy(c->copy_stream); }
     if (c->copy_done) cudaEventDestroy(c->copy_done);
     if (c->d2h_stream) { cudaStreamSynchronize(c->d2h_stream); cudaStreamDestroy(c->d2h_stream); }
-    if (c->rag_pin) cudaFreeHost(c->rag_pin);
-    for (int i = 0; i < 2; ++i) if (c->path_done[i]) cudaEventDestroy(c->path_done[i]);
+    for (auto e : c->path_done) if (e) cudaEventDestroy(e);
     if (c->own_stream) cudaStreamDestroy(c->stream);
     delete c;
     return MDF_OK;
@@ -350,8 +349,9 @@ struct PairInputs {
 };
 
 // What a batch is built from, in host memory its copies may read (pinned for jobs).  A structure batch has coordinates and either
-// the alignment strings or, for pairs, `pairs`; a batch without coordinates may bring its contact maps packed.  G / C size the
-// pooled features and scores (0: allocated by the first run); `extra_reserve` is arena room kept above the batch for its run.
+// the alignment strings or, for pairs, `pairs`; a batch without coordinates brings its contact maps, bit-packed (`packed`) or, for
+// a job with n == 1, as one dense int32 [L, L] map (`dense`).  A maps-only batch has no sequences.  G / C size the pooled
+// features and scores (0: allocated by the first run); `extra_reserve` is arena room kept above the batch for its run.
 struct BatchInputs {
     int n = 0;
     const char *seq = nullptr;    const int64_t *seq_off = nullptr;
@@ -359,6 +359,8 @@ struct BatchInputs {
     const char *q_aln = nullptr, *t_aln = nullptr; const int64_t *aln_off = nullptr;
     const PairInputs *pairs = nullptr;
     const uint32_t *packed = nullptr;
+    const int32_t *dense = nullptr;
+    bool maps_only = false;
     int G = 0, C = 0;
     size_t extra_reserve = 0;
 };
@@ -522,7 +524,6 @@ static int pack_pairs(const char *who, RaggedPack &pk, int codes, int nt, const 
     return nw_bad_letter(who, bad, which, c);
 }
 
-// Builds host metadata, allocates (cudaMalloc when `persistent`, the slot's block for a job, arena otherwise) and uploads.
 __global__ void fill_res_prot_kernel(int n, const int64_t *__restrict__ seq_off, int *__restrict__ res_prot)
 {
     for (int p = blockIdx.x; p < n; p += gridDim.x) {
@@ -531,12 +532,14 @@ __global__ void fill_res_prot_kernel(int n, const int64_t *__restrict__ seq_off,
     }
 }
 
-static int batch_build(mdf_ctx *ctx, mdf_batch *b, bool persistent, const BatchInputs &in, mdf_job *slot = nullptr)
+// Builds host metadata, allocates and uploads: a resident batch (slot == nullptr) into its own cudaMalloc block, a job's batch into
+// the slot's device block, its metadata staged through the slot's pinned memory and its structure inputs sent on the copy stream.
+static int batch_build(mdf_ctx *ctx, mdf_batch *b, const BatchInputs &in, mdf_job *slot = nullptr)
 {
     const int n = in.n;
     const int64_t *seq_off = in.seq_off, *coord_off = in.coord_off, *aln_off = in.aln_off;
     const PairInputs *pin = in.pairs;
-    MDF_REQUIRE(n >= 0 && seq_off && (n == 0 || in.seq), "batch: sequences missing");
+    MDF_REQUIRE(n >= 0 && seq_off && (n == 0 || in.seq || in.maps_only), "batch: sequences missing");
     b->ctx = ctx;
     b->n = n;
     b->h_seq_off.assign(seq_off, seq_off + n + 1);
@@ -575,10 +578,9 @@ static int batch_build(mdf_ctx *ctx, mdf_batch *b, bool persistent, const BatchI
     carve_batch(b, measure, ncoord, alnb, in);
     const size_t bytes = measure.top + 512;
     char *base = nullptr;
-    if (persistent) {
+    if (!slot) {
         MDF_CUDA(cudaMalloc((void **)&base, bytes));
-        b->owns_memory = true;
-    } else if (slot) {
+    } else {
         // job slot: a device block of its own, so the inputs of this job may arrive while the previous job still computes
         if (const cudaError_t e = grow_block(slot->dev, slot->dev_bytes, bytes, true)) {
             set_error("cudaMalloc(%zu bytes) for a job slot failed: %s", with_headroom(bytes), cudaGetErrorString(e));
@@ -586,9 +588,8 @@ static int batch_build(mdf_ctx *ctx, mdf_batch *b, bool persistent, const BatchI
         }
         MDF_TRY(ctx->reserve(in.extra_reserve));
         base = slot->dev;
-    } else {
-        MDF_TRY(ctx->reserve(bytes + in.extra_reserve));
-        MDF_TRY(ctx->alloc((void **)&base, bytes));
+        // pinned staging of the small metadata; without it the copies fall back to pageable sources + a synchronise
+        grow_block(slot->meta, slot->meta_bytes, (size_t)n * 96 + (size_t)b->T + (2u << 20), false);
     }
     b->block = base;
     Carver carve;
@@ -599,7 +600,7 @@ static int batch_build(mdf_ctx *ctx, mdf_batch *b, bool persistent, const BatchI
     // small metadata: through the slot's pinned staging when there is one (asynchronous), else from the pageable vectors (+ sync below)
     bool staged = slot != nullptr;
     auto src_of = [&](const void *p, size_t bytes) { return mdf_job::src_of(slot, p, bytes, &staged); };
-    if (b->T) MDF_CUDA(cudaMemcpyAsync(b->d_seq, in.seq, (size_t)b->T, cudaMemcpyHostToDevice, s));
+    if (b->T && in.seq) MDF_CUDA(cudaMemcpyAsync(b->d_seq, in.seq, (size_t)b->T, cudaMemcpyHostToDevice, s));
     MDF_CUDA(cudaMemcpyAsync(b->d_seq_off, src_of(b->h_seq_off.data(), (n + 1) * sizeof(int64_t)), (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, s));
     MDF_CUDA(cudaMemcpyAsync(b->d_packed_off, src_of(b->h_packed_off.data(), (n + 1) * sizeof(int64_t)), (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, s));
     if (b->nwork) MDF_CUDA(cudaMemcpyAsync(b->d_work, src_of(work.data(), work.size() * sizeof(int2)), work.size() * sizeof(int2), cudaMemcpyHostToDevice, s));
@@ -609,15 +610,9 @@ static int batch_build(mdf_ctx *ctx, mdf_batch *b, bool persistent, const BatchI
         MDF_LAUNCH_CHECK(ctx);
     }
     if (b->has_structure) {
-        // transient batches (mdf_path_forward): coordinates and alignments - nine tenths of the input bytes - travel on the copy
-        // stream and are only awaited by the contact-map stage, which run_path enqueues after the LSTM language model
-        cudaStream_t cs = (!persistent && ctx->copy_stream) ? ctx->copy_stream : s;
-        if (cs != s && !slot) {
-            // arena-backed transient batch: the bytes below may still be in use by kernels queued on the compute stream by an
-            // earlier call (the arena is reused in stream order) - the copy stream must not run ahead of them
-            MDF_CUDA(cudaEventRecord(ctx->copy_done, s));
-            MDF_CUDA(cudaStreamWaitEvent(cs, ctx->copy_done, 0));
-        }
+        // jobs: coordinates and alignments - nine tenths of the input bytes - travel on the copy stream into the slot's own block and
+        // are only awaited by the contact-map stage, which run_path enqueues after the LSTM language model
+        cudaStream_t cs = slot ? ctx->copy_stream : s;
         if (ncoord) MDF_CUDA(cudaMemcpyAsync(b->d_coords, in.coords, ncoord * 3 * sizeof(float), cudaMemcpyHostToDevice, cs));
         MDF_CUDA(cudaMemcpyAsync(b->d_coord_off, coord_off, (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, cs));
         if (pin) {
@@ -643,6 +638,14 @@ static int batch_build(mdf_ctx *ctx, mdf_batch *b, bool persistent, const BatchI
         }
     } else if (in.packed && b->h_packed_off[n]) {
         MDF_CUDA(cudaMemcpyAsync(b->d_packed, in.packed, (size_t)b->h_packed_off[n] * 4, cudaMemcpyHostToDevice, s));
+    } else if (in.dense) {
+        // packed on the device from arena scratch; the 0/1 check goes to the slot's second error word, as run_path resets d_err
+        int32_t *dd;
+        MDF_TRY(ctx->alloc_n(&dd, (size_t)b->T * b->T + 1));
+        if (b->T) MDF_CUDA(cudaMemcpyAsync(dd, in.dense, (size_t)b->T * b->T * 4, cudaMemcpyHostToDevice, s));
+        MDF_CUDA(cudaMemsetAsync(ctx->d_err, 0, sizeof(int), s));
+        MDF_TRY(launch_pack_dense(ctx, (int)b->T, dd, b->d_packed));
+        MDF_CUDA(cudaMemcpyAsync(slot->d_errs + 1, ctx->d_err, sizeof(int), cudaMemcpyDeviceToDevice, s));
     }
     // pageable sources (work / order vectors) must be consumed before they go out of scope; pinned staging needs no wait
     if (!staged) MDF_CUDA(cudaStreamSynchronize(s));
@@ -689,7 +692,7 @@ static int run_path(mdf_model *m, mdf_batch *b, float thr2, int gen, int upto, b
     mdf_ctx *ctx = m->ctx;
     MDF_CUDA(cudaMemsetAsync(ctx->d_err, 0, sizeof(int), ctx->stream));
     // a persistent batch that already holds the maps for this (threshold, generated contacts) keeps them for the next head
-    const bool maps_cached = with_cmap && b->owns_memory && b->reuse && b->cmap_valid && b->cmap_thr2 == thr2 && b->cmap_gen == gen &&
+    const bool maps_cached = with_cmap && !b->slot && b->reuse && b->cmap_valid && b->cmap_thr2 == thr2 && b->cmap_gen == gen &&
                              b->cmap_eps == m->eps && upto >= 2;
     // Transient batches on the tensor-core engine: the LSTM language model and the embedding only need the sequences, so they are
     // enqueued first and the contact-map stage (which waits for the coordinates still travelling on the copy stream) follows
@@ -706,20 +709,10 @@ static int run_path(mdf_model *m, mdf_batch *b, float thr2, int gen, int upto, b
     MDF_TRY(launch_seq_to_idx(ctx, b->T, b->d_seq, b->d_idx));
     if (!maps_cached && !defer_cmap) {
         MDF_TRY(launch_prep_adjacency(ctx, b, m->eps));
-        if (with_cmap && b->owns_memory) { b->cmap_valid = true; b->cmap_thr2 = thr2; b->cmap_gen = gen; b->cmap_eps = m->eps; }
+        if (with_cmap && !b->slot) { b->cmap_valid = true; b->cmap_thr2 = thr2; b->cmap_gen = gen; b->cmap_eps = m->eps; }
     }
     if (m->engine == 1) return tc_forward(m, b, upto, defer_cmap ? &cmap_stage : nullptr);
     return simt_forward(m, b, upto);
-}
-
-static int fetch_scores(mdf_model *m, mdf_batch *b, float *scores)
-{
-    mdf_ctx *ctx = m->ctx;
-    if (b->n && scores)
-        MDF_CUDA(cudaMemcpyAsync(scores, b->d_scores, (size_t)b->n * m->C * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    MDF_CUDA(cudaMemcpyAsync(ctx->h_err, ctx->d_err, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-    MDF_CUDA(cudaStreamSynchronize(ctx->stream));
-    return ctx->check_device_error("path");
 }
 
 extern "C" int mdf_batch_upload(mdf_ctx *ctx, int n, const char *seq, const int64_t *seq_off, const float *coords,
@@ -730,8 +723,8 @@ extern "C" int mdf_batch_upload(mdf_ctx *ctx, int n, const char *seq, const int6
     MDF_CUDA(cudaSetDevice(ctx->device));
     mdf_batch *b = new mdf_batch();
     // pooled / scores depend on the model head: allocated lazily by the first run
-    const int r = batch_build(ctx, b, true, {.n = n, .seq = seq, .seq_off = seq_off, .coords = coords, .coord_off = coord_off,
-                                             .q_aln = q_aln, .t_aln = t_aln, .aln_off = aln_off});
+    const int r = batch_build(ctx, b, {.n = n, .seq = seq, .seq_off = seq_off, .coords = coords, .coord_off = coord_off,
+                                       .q_aln = q_aln, .t_aln = t_aln, .aln_off = aln_off});
     if (r != MDF_OK) {
         mdf_batch_destroy(b);
         return r;
@@ -785,7 +778,7 @@ extern "C" int mdf_batch_upload_pairs(mdf_ctx *ctx, int n, const char *seq, cons
     nw_matrix32(matrix, A, m32);
     const PairInputs pin{&plan, (const uint8_t *)pk.at(codes), plan.pairs.data(), m32, A, gap_open, gap_extend, true};
     mdf_batch *b = new mdf_batch();
-    int r = batch_build(ctx, b, true, {.n = n, .seq = seq, .seq_off = seq_off, .coords = coords, .coord_off = coord_off, .pairs = &pin});
+    int r = batch_build(ctx, b, {.n = n, .seq = seq, .seq_off = seq_off, .coords = coords, .coord_off = coord_off, .pairs = &pin});
     if (r == MDF_OK) r = align_uploaded(ctx, b, plan);
     if (r != MDF_OK) {
         mdf_batch_destroy(b);
@@ -800,7 +793,7 @@ extern "C" int mdf_batch_fetch_alignment(mdf_batch *b, int32_t *nw_score, int32_
                                          const int64_t *ops_off, int *ops_len)
 {
     MDF_REQUIRE(b && b->ctx && nw_score && aln_len && n_match, "mdf_batch_fetch_alignment: bad arguments");
-    MDF_REQUIRE(b->pairs && b->owns_memory, "mdf_batch_fetch_alignment: needs a batch uploaded with mdf_batch_upload_pairs");
+    MDF_REQUIRE(b->pairs && !b->slot, "mdf_batch_fetch_alignment: needs a batch uploaded with mdf_batch_upload_pairs");
     MDF_REQUIRE(!ops || (ops_off && ops_len), "mdf_batch_fetch_alignment: ops_off / ops_len missing");
     const int n = b->n;
     if (n == 0) return MDF_OK;
@@ -825,7 +818,7 @@ extern "C" int mdf_batch_fetch_alignment(mdf_batch *b, int32_t *nw_score, int32_
 extern "C" int mdf_batch_destroy(mdf_batch *b)
 {
     if (!b) return MDF_OK;
-    if (b->owns_memory && b->block) {
+    if (!b->slot && b->block) {
         cudaSetDevice(b->ctx->device);
         cudaStreamSynchronize(b->ctx->stream);
         cudaFree(b->block);
@@ -843,7 +836,7 @@ extern "C" int mdf_path_run_stages(mdf_model *m, mdf_batch *b, float thr2, int g
     mdf_ctx *ctx = m->ctx;
     MDF_CUDA(cudaSetDevice(ctx->device));
     if (upto >= 2 && (b->out_G != m->G || b->out_C != m->C)) {   // (re)allocate outputs for this head
-        MDF_REQUIRE(b->owns_memory, "mdf_path_run: batch outputs do not match the model head");
+        MDF_REQUIRE(!b->slot, "mdf_path_run: batch outputs do not match the model head");
         MDF_CUDA(cudaStreamSynchronize(ctx->stream));
         if (b->out_block) MDF_CUDA(cudaFree(b->out_block));
         b->out_block = nullptr;
@@ -888,8 +881,12 @@ extern "C" int mdf_batch_fetch_scores(mdf_model *m, mdf_batch *b, float *scores)
 {
     MDF_REQUIRE(m && b && scores, "mdf_batch_fetch_scores: bad arguments");
     MDF_REQUIRE(b->out_C == m->C && b->d_scores, "mdf_batch_fetch_scores: the batch holds the scores of another head (run this head first)");
-    MDF_CUDA(cudaSetDevice(m->ctx->device));
-    return fetch_scores(m, b, scores);
+    mdf_ctx *ctx = m->ctx;
+    MDF_CUDA(cudaSetDevice(ctx->device));
+    if (b->n) MDF_CUDA(cudaMemcpyAsync(scores, b->d_scores, (size_t)b->n * m->C * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    MDF_CUDA(cudaMemcpyAsync(ctx->h_err, ctx->d_err, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    MDF_CUDA(cudaStreamSynchronize(ctx->stream));
+    return device_error("path", *ctx->h_err);
 }
 
 // The reference-layout output of the contact-map stage for a resident batch: dense int32 [Lq, Lq] per protein (what
@@ -898,7 +895,7 @@ extern "C" int mdf_batch_fetch_scores(mdf_model *m, mdf_batch *b, float *scores)
 extern "C" int mdf_batch_unpack_dense(mdf_batch *b, int32_t *dense_device, int64_t *cells_out)
 {
     MDF_REQUIRE(b && b->ctx, "mdf_batch_unpack_dense: batch is NULL");
-    MDF_REQUIRE(b->owns_memory && b->has_structure, "mdf_batch_unpack_dense: needs an uploaded batch with structures");
+    MDF_REQUIRE(!b->slot && b->has_structure, "mdf_batch_unpack_dense: needs an uploaded batch with structures");
     mdf_ctx *ctx = b->ctx;
     MDF_CUDA(cudaSetDevice(ctx->device));
     ArenaScope scope(ctx);
@@ -956,29 +953,29 @@ extern "C" int mdf_batch_fetch(mdf_model *m, mdf_batch *b, int what, void *dst, 
 // ------------------------------------------------------------------------------------------- jobs: submit / wait
 // A job = one transient batch through the whole path.  mdf_path_submit* enqueue H2D + every kernel + the D2H of the scores and
 // return; mdf_path_wait blocks until the scores are on the host.  Two jobs may be in flight per context: the inputs of job k + 1
-// are packed (pinned slot memory, host threads) and copied (copy stream, the slot's own device block) while job k computes.
-static int slot_acquire(mdf_ctx *ctx, mdf_job **out)
+// are packed (pinned slot memory, host threads) and copied (copy stream, the slot's own device block) while job k computes.  The
+// synchronous calls run the same job bodies in a third slot, which the ring never hands out, and wait.
+static int slot_acquire(mdf_ctx *ctx, mdf_job **out, bool sync = false)
 {
-    mdf_job *sl = &ctx->slots[ctx->next_slot];
+    mdf_job *sl = &ctx->slots[sync ? 2 : ctx->next_slot];
     if (sl->busy) {
         set_error("mdf_path_submit: both job slots of this context are in flight; call mdf_path_wait on the older job first");
         return MDF_EINVAL;
     }
     MDF_CUDA(cudaEventSynchronize(sl->done));        // a slot is only rewritten after its previous job has completely finished
-    ctx->next_slot ^= 1;
+    if (!sync) ctx->next_slot ^= 1;
     delete sl->batch;
     sl->batch = new mdf_batch();
     sl->h_err[0] = sl->h_err[1] = 0;
-    sl->rc = MDF_OK;
     sl->meta_top = 0;
     sl->n_pairs = 0;
     *out = sl;
     return MDF_OK;
 }
 
-// After a job has been enqueued from slot `sl`, bring the idle peer slot to the same buffer sizes while the GPU is busy with that
-// job: page-locking ~100 MB and a first cudaMalloc cost 50-75 ms of host time, which the second job of a stream of chunks would
-// otherwise pay in front of an idle GPU.
+// After a job has been enqueued from ring slot `sl`, bring the idle peer slot to the same buffer sizes while the GPU is busy with
+// that job: page-locking ~100 MB and a first cudaMalloc cost 50-75 ms of host time, which the second job of a stream of chunks
+// would otherwise pay in front of an idle GPU.
 static void slot_match_peer(mdf_ctx *ctx, mdf_job *sl)
 {
     mdf_job *peer = &ctx->slots[(sl - ctx->slots) ^ 1];
@@ -989,26 +986,27 @@ static void slot_match_peer(mdf_ctx *ctx, mdf_job *sl)
         grow_block(peer->dev, peer->dev_bytes, sl->dev_bytes, true, sl->dev_bytes);
 }
 
-// The tail of every job kind, after its kernels have been enqueued on the compute stream: the scores (and the job's error word,
-// parked in a per-slot device word because the next job resets d_err) leave on the device-to-host stream behind an event, so the
-// next job's kernels do not queue behind this job's 32 MB result copy; `more` enqueues the job's other result copies on that
-// stream.  Both therefore live in the slot's device block, never in the arena.  On success the slot is handed out as *job.
-static int job_finish(mdf_job *sl, int rc, int n, const float *d_scores, size_t score_count, float *scores,
-                      const std::function<cudaError_t(cudaStream_t)> &more, mdf_job **job)
+// A device -> host result copy of a job: from the slot's device block, or from the arena in a synchronous call, which waits first
+struct ResultCopy { void *dst; const void *src; size_t bytes; };
+
+// The tail of every job kind, after its kernels have been enqueued on the compute stream: the job's error word (parked in the
+// slot's device words because the next job resets d_err) and the result copies leave on the device-to-host stream behind an event,
+// so the next job's kernels do not queue behind this job's 32 MB result copy.  On success the slot is handed out as *job.
+static int job_finish(mdf_job *sl, int rc, int n, const std::vector<ResultCopy> &results, mdf_job **job)
 {
     mdf_ctx *ctx = sl->ctx;
     cudaStream_t out_stream = ctx->stream;
     if (rc == MDF_OK && n > 0) {
         const int slot = (int)(sl - ctx->slots);
-        cudaError_t e = cudaMemcpyAsync(ctx->d_err + 2 + slot, ctx->d_err, sizeof(int), cudaMemcpyDeviceToDevice, ctx->stream);
+        cudaError_t e = cudaMemcpyAsync(sl->d_errs, ctx->d_err, sizeof(int), cudaMemcpyDeviceToDevice, ctx->stream);
         if (e == cudaSuccess && ctx->d2h_stream) {
             e = cudaEventRecord(ctx->path_done[slot], ctx->stream);
             if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->d2h_stream, ctx->path_done[slot], 0);
             if (e == cudaSuccess) out_stream = ctx->d2h_stream;
         }
-        if (e == cudaSuccess) e = cudaMemcpyAsync(scores, d_scores, score_count * sizeof(float), cudaMemcpyDeviceToHost, out_stream);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(sl->h_err, ctx->d_err + 2 + slot, sizeof(int), cudaMemcpyDeviceToHost, out_stream);
-        if (e == cudaSuccess && more) e = more(out_stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(sl->h_err, sl->d_errs, sizeof(int), cudaMemcpyDeviceToHost, out_stream);
+        for (const ResultCopy &r : results)
+            if (e == cudaSuccess && r.bytes) e = cudaMemcpyAsync(r.dst, r.src, r.bytes, cudaMemcpyDeviceToHost, out_stream);
         if (e != cudaSuccess) { set_error("job: result copy failed: %s", cudaGetErrorString(e)); rc = MDF_ECUDA; }
     }
     if (rc != MDF_OK && ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);   // no input copy may outlive a failed call
@@ -1016,8 +1014,28 @@ static int job_finish(mdf_job *sl, int rc, int n, const float *d_scores, size_t 
     if (rc != MDF_OK) return rc;
     sl->busy = true;
     *job = sl;
-    slot_match_peer(ctx, sl);
+    if (sl != &ctx->slots[2]) slot_match_peer(ctx, sl);
     return MDF_OK;
+}
+
+// Blocks until the job in `sl` is complete, hands a pairs job's outputs to the caller and reports the job's device error words:
+// word 0 after "`where`: ", then word 1 (only ever set by mdf_gcn_forward_dense) after "forward_pass: ".
+static int job_wait(mdf_job *sl, const char *where)
+{
+    sl->busy = false;
+    MDF_CUDA(cudaEventSynchronize(sl->done));
+    if (const int n = sl->n_pairs) {
+        for (int k = 0; k < 3; ++k) memcpy(sl->out_stats[k], sl->pin_stats + (size_t)k * n, (size_t)n * 4);
+        if (sl->out_ops)
+            for (int p = 0; p < n; ++p) {
+                const int len = sl->out_stats[1][p];
+                memcpy(sl->out_ops + sl->out_ops_off[p], sl->pin_ops + sl->nw_off[p], (size_t)len);
+                sl->out_ops_len[p] = len;
+            }
+        sl->n_pairs = 0;
+    }
+    MDF_TRY(device_error(where, sl->h_err[0]));
+    return device_error("forward_pass", sl->h_err[1]);
 }
 
 // enqueue everything for flat inputs (already where they may be read asynchronously: pinned slot memory or caller buffers) and
@@ -1031,30 +1049,28 @@ static int job_enqueue(mdf_model *m, mdf_job *sl, BatchInputs in, float thr2, in
     const PairInputs *pin = in.pairs;
     static const bool timing = getenv("MDF_TIMING") != nullptr;       // host-side breakdown of one call on stderr
     const auto t0 = std::chrono::steady_clock::now();
-    // pinned staging of the small metadata; without it the copies fall back to pageable sources + a synchronise
-    grow_block(sl->meta, sl->meta_bytes, (size_t)n * 96 + (size_t)(n > 0 ? in.seq_off[n] : 0) + (2u << 20), false);
     in.G = m->G; in.C = m->C;
-    in.extra_reserve = engine_workspace(m, n, in.seq_off) + (pin ? pin->plan->scratch_bytes() + 1024 : 0);
-    int rc = batch_build(ctx, b, false, in, sl);
+    in.extra_reserve = engine_workspace(m, n, in.seq_off) + (pin ? pin->plan->scratch_bytes() + 1024 : 0) +
+                       (in.dense ? (size_t)in.seq_off[1] * in.seq_off[1] * 4 + 4096 : 0);
+    int rc = batch_build(ctx, b, in, sl);
     if (rc == MDF_OK && pin) {
         // alignment scratch (~1 byte per DP cell) from the arena, ahead of the engine stages; released in stream order
         rc = ctx->alloc_n(&b->d_nw_dir, (size_t)pin->plan->dir_words + 4);
         if (rc == MDF_OK) rc = ctx->alloc_n(&b->d_nw_bnd, (size_t)pin->plan->bnd_ints + 4);
     }
     const auto t1 = std::chrono::steady_clock::now();
-    if (rc == MDF_OK) rc = run_path(m, b, thr2, gen, 4, true);
+    if (rc == MDF_OK) rc = run_path(m, b, thr2, gen, 4, b->has_structure);
     if (timing) {
         const auto t2 = std::chrono::steady_clock::now();
         auto ms = [](auto a, auto b2) { return std::chrono::duration<double, std::milli>(b2 - a).count(); };
         fprintf(stderr, "[mdf_path_submit] n=%d: batch build + H2D %.2f ms, enqueue (host) %.2f ms\n", n, ms(t0, t1), ms(t1, t2));
     }
     sl->n_pairs = pin ? n : 0;
-    auto pair_outputs = [&](cudaStream_t s) {
-        cudaError_t e = cudaMemcpyAsync(sl->pin_stats, b->d_nw_stats, (size_t)n * 12, cudaMemcpyDeviceToHost, s);
-        if (e == cudaSuccess && pin->ops && b->h_nw_off[n]) e = cudaMemcpyAsync(sl->pin_ops, b->d_ops, (size_t)b->h_nw_off[n], cudaMemcpyDeviceToHost, s);
-        return e;
-    };
-    return job_finish(sl, rc, n, b->d_scores, (size_t)n * m->C, scores, pin ? pair_outputs : std::function<cudaError_t(cudaStream_t)>(), job);
+    std::vector<ResultCopy> results{{scores, b->d_scores, (size_t)n * m->C * sizeof(float)}};
+    if (pin) results.push_back({sl->pin_stats, b->d_nw_stats, (size_t)n * 12});
+    if (pin && pin->ops) results.push_back({sl->pin_ops, b->d_ops, (size_t)pin->plan->off[n]});
+    if (in.dense) results.push_back({sl->h_err + 1, sl->d_errs + 1, sizeof(int)});
+    return job_finish(sl, rc, n, results, job);
 }
 
 extern "C" int mdf_path_submit(mdf_model *m, int n, const char *seq, const int64_t *seq_off, const float *coords,
@@ -1149,9 +1165,35 @@ extern "C" int mdf_path_submit_pairs(mdf_model *m, int n, const char *const *que
                                .pairs = &pin}, thr2, gen, scores, job);
 }
 
+// The CNN job of batch v (sized for its n sequences) in slot `sl`.  The sequences (`seq`, v.T bytes) and the per-tile table are
+// copied on the copy stream into the slot's device block, which also holds the pooled features and the scores; the head's
+// temporaries come from the arena, in stream order.
+static int cnn_job(mdf_cnn_model *m, mdf_job *sl, CnnBatch v, const char *seq, const void *tiles, float *scores, mdf_job **job)
+{
+    mdf_ctx *ctx = m->ctx;
+    const size_t bytes = cnn_carve(m, v, nullptr);
+    if (const cudaError_t e = grow_block(sl->dev, sl->dev_bytes, bytes, true)) {
+        set_error("cudaMalloc(%zu bytes) for a job slot failed: %s", with_headroom(bytes), cudaGetErrorString(e));
+        return MDF_ENOMEM;
+    }
+    cnn_carve(m, v, sl->dev);
+    ArenaScope scope(ctx);
+    int rc = MDF_OK;
+    if (v.n > 0) {
+        // the slot's previous job has finished (slot_acquire), so its block may be overwritten while the other slot's job computes
+        cudaStream_t cs = ctx->copy_stream;
+        cudaError_t e = cudaMemcpyAsync(v.d_seq, seq, (size_t)v.T, cudaMemcpyHostToDevice, cs);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(v.d_tile_info, tiles, (size_t)v.n_tiles * sizeof(int4), cudaMemcpyHostToDevice, cs);
+        if (e == cudaSuccess) e = cudaEventRecord(ctx->copy_done, cs);
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->stream, ctx->copy_done, 0);
+        if (e != cudaSuccess) { set_error("mdf_cnn_submit_ragged: input copy failed: %s", cudaGetErrorString(e)); rc = MDF_ECUDA; }
+        if (rc == MDF_OK) rc = cnn_run(m, v);
+    }
+    return job_finish(sl, rc, v.n, {{scores, v.d_scores, (size_t)v.n * m->C * sizeof(float)}}, job);
+}
+
 // mdf_cnn_forward as a job from per-sequence pointers.  The sequences and the per-tile table are packed into the slot's pinned
-// block and copied on the copy stream into the slot's device block, which also holds the pooled features and the scores; the
-// head's temporaries come from the arena, in stream order.
+// block, then as cnn_job.
 extern "C" int mdf_cnn_submit_ragged(mdf_cnn_model *m, int n, const char *const *seq, const int *seq_len, float *scores, mdf_job **job)
 {
     MDF_REQUIRE(m && scores && job && n >= 0, "mdf_cnn_submit_ragged: bad arguments");
@@ -1175,27 +1217,8 @@ extern "C" int mdf_cnn_submit_ragged(mdf_cnn_model *m, int n, const char *const 
     MDF_TRY(pinned_block(sl->pin, sl->pin_bytes, pk.place(nullptr), " for a job slot"));
     pk.place(sl->pin);
     pk.pack(pack_threads(ctx, n));
-    int4 *tiles = reinterpret_cast<int4 *>(pk.at(TILES));
-    cnn_tiles(n, pk.off(S), tiles);
-    const size_t bytes = cnn_carve(m, v, nullptr);
-    if (const cudaError_t e = grow_block(sl->dev, sl->dev_bytes, bytes, true)) {
-        set_error("cudaMalloc(%zu bytes) for a job slot failed: %s", with_headroom(bytes), cudaGetErrorString(e));
-        return MDF_ENOMEM;
-    }
-    cnn_carve(m, v, sl->dev);
-    ArenaScope scope(ctx);
-    int rc = MDF_OK;
-    if (n > 0) {
-        // the slot's previous job has finished (slot_acquire), so its block may be overwritten while the other slot's job computes
-        cudaStream_t cs = ctx->copy_stream;
-        cudaError_t e = cudaMemcpyAsync(v.d_seq, pk.at(S), (size_t)v.T, cudaMemcpyHostToDevice, cs);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(v.d_tile_info, tiles, (size_t)v.n_tiles * sizeof(int4), cudaMemcpyHostToDevice, cs);
-        if (e == cudaSuccess) e = cudaEventRecord(ctx->copy_done, cs);
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->stream, ctx->copy_done, 0);
-        if (e != cudaSuccess) { set_error("mdf_cnn_submit_ragged: input copy failed: %s", cudaGetErrorString(e)); rc = MDF_ECUDA; }
-        if (rc == MDF_OK) rc = cnn_run(m, v);
-    }
-    return job_finish(sl, rc, n, v.d_scores, (size_t)n * m->C, scores, {}, job);
+    cnn_tiles(n, pk.off(S), reinterpret_cast<int4 *>(pk.at(TILES)));
+    return cnn_job(m, sl, v, pk.at(S), pk.at(TILES), scores, job);
 }
 
 extern "C" int mdf_path_wait(mdf_job *job)
@@ -1203,25 +1226,7 @@ extern "C" int mdf_path_wait(mdf_job *job)
     MDF_REQUIRE(job && job->ctx, "mdf_path_wait: job is NULL");
     MDF_REQUIRE(job->busy, "mdf_path_wait: this job has already been waited for");
     MDF_CUDA(cudaSetDevice(job->ctx->device));
-    job->busy = false;
-    MDF_CUDA(cudaEventSynchronize(job->done));
-    if (const int n = job->n_pairs) {
-        for (int k = 0; k < 3; ++k) memcpy(job->out_stats[k], job->pin_stats + (size_t)k * n, (size_t)n * 4);
-        if (job->out_ops)
-            for (int p = 0; p < n; ++p) {
-                const int len = job->out_stats[1][p];
-                memcpy(job->out_ops + job->out_ops_off[p], job->pin_ops + job->nw_off[p], (size_t)len);
-                job->out_ops_len[p] = len;
-            }
-        job->n_pairs = 0;
-    }
-    const int e = job->h_err[0];
-    if (e == 0) return MDF_OK;
-    set_error("path: %s", e == MDF_DERR_BAD_RESIDUE ? "Invalid character in sequence"
-                        : e == MDF_DERR_BAD_CMAP    ? "contact map holds values other than 0/1"
-                        : e == MDF_DERR_LQ_MISMATCH ? "query sequence length does not match the gap-stripped query alignment"
-                                                    : "unknown device error");
-    return MDF_EINVAL;
+    return job_wait(job, "path");
 }
 
 extern "C" int mdf_path_forward(mdf_model *m, int n, const char *seq, const int64_t *seq_off, const float *coords,
@@ -1233,14 +1238,30 @@ extern "C" int mdf_path_forward(mdf_model *m, int n, const char *seq, const int6
     return mdf_path_wait(job);
 }
 
+// ------------------------------------------------------------------------------------------- synchronous calls: one job each in the
+// context's synchronous slot, waited for before the call returns (so its inputs may be pageable and its results read the arena)
+extern "C" int mdf_cnn_forward(mdf_cnn_model *m, int n, const char *seq, const int64_t *seq_off, float *scores)
+{
+    MDF_REQUIRE(m && scores, "mdf_cnn_forward: bad arguments");
+    mdf_ctx *ctx = m->ctx;
+    MDF_CUDA(cudaSetDevice(ctx->device));
+    CnnBatch v;
+    std::vector<int4> tiles;
+    MDF_TRY(cnn_plan(n, seq, seq_off, v, tiles));
+    mdf_job *sl = nullptr, *job = nullptr;
+    MDF_TRY(slot_acquire(ctx, &sl, true));
+    grow_block(sl->meta, sl->meta_bytes, tiles.size() * sizeof(int4), false);
+    const void *staged = sl->stage(tiles.data(), tiles.size() * sizeof(int4));      // without pinned staging: `tiles` outlives the wait
+    MDF_TRY(cnn_job(m, sl, v, seq, staged ? staged : tiles.data(), scores, &job));
+    return job_wait(sl, "cnn forward");
+}
+
 extern "C" int mdf_gcn_forward_packed(mdf_model *m, int n, const char *seq, const int64_t *seq_off,
                                       const uint32_t *packed, const int64_t *packed_off, float *scores)
 {
     MDF_REQUIRE(m && scores && (n == 0 || packed), "mdf_gcn_forward_packed: bad arguments");
     mdf_ctx *ctx = m->ctx;
     MDF_CUDA(cudaSetDevice(ctx->device));
-    ArenaScope scope(ctx);
-    mdf_batch b;
     // packed_off must follow the canonical layout (contiguous, mdf_packed_row_words)
     int64_t off = 0;
     for (int p = 0; p < n; ++p) {
@@ -1248,10 +1269,10 @@ extern "C" int mdf_gcn_forward_packed(mdf_model *m, int n, const char *seq, cons
         const int64_t L = seq_off[p + 1] - seq_off[p];
         off += L * mdf_packed_row_words((int)L);
     }
-    MDF_TRY(batch_build(ctx, &b, false, {.n = n, .seq = seq, .seq_off = seq_off, .packed = packed, .G = m->G, .C = m->C,
-                                         .extra_reserve = engine_workspace(m, n, seq_off)}));
-    MDF_TRY(run_path(m, &b, 0.f, 0, 4, false));
-    return fetch_scores(m, &b, scores);
+    mdf_job *sl = nullptr, *job = nullptr;
+    MDF_TRY(slot_acquire(ctx, &sl, true));
+    MDF_TRY(job_enqueue(m, sl, {.n = n, .seq = seq, .seq_off = seq_off, .packed = packed}, 0.f, 0, scores, &job));
+    return job_wait(sl, "path");
 }
 
 extern "C" int mdf_gcn_forward_dense(mdf_model *m, const char *seq, int L, const int32_t *cmap, float *scores)
@@ -1259,27 +1280,24 @@ extern "C" int mdf_gcn_forward_dense(mdf_model *m, const char *seq, int L, const
     MDF_REQUIRE(m && scores && L >= 0 && (L == 0 || (seq && cmap)), "mdf_gcn_forward_dense: bad arguments");
     mdf_ctx *ctx = m->ctx;
     MDF_CUDA(cudaSetDevice(ctx->device));
-    ArenaScope scope(ctx);
-    mdf_batch b;
     const int64_t seq_off[2] = {0, L};
-    const size_t dense_bytes = (size_t)L * L * 4;
-    MDF_TRY(batch_build(ctx, &b, false, {.n = 1, .seq = seq, .seq_off = seq_off, .G = m->G, .C = m->C,
-                                         .extra_reserve = engine_workspace(m, 1, seq_off) + dense_bytes + 4096}));
-    int32_t *dd;
-    MDF_TRY(ctx->alloc_n(&dd, (size_t)L * L + 1));
-    if (L) MDF_CUDA(cudaMemcpyAsync(dd, cmap, dense_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    mdf_job *sl = nullptr, *job = nullptr;
+    MDF_TRY(slot_acquire(ctx, &sl, true));
+    MDF_TRY(job_enqueue(m, sl, {.n = 1, .seq = seq, .seq_off = seq_off, .dense = cmap}, 0.f, 0, scores, &job));
+    return job_wait(sl, "path");
+}
+
+// Enqueues the maps of batch b and, with dense_off, their dense int32 form in arena scratch (*dense, dense_total cells).
+static int cmap_maps(mdf_ctx *ctx, mdf_batch *b, float thr2, int gen, const int64_t *dense_off, size_t dense_total, int32_t **dense)
+{
     MDF_CUDA(cudaMemsetAsync(ctx->d_err, 0, sizeof(int), ctx->stream));
-    MDF_TRY(launch_pack_dense(ctx, L, dd, b.d_packed));
-    // run_path resets d_err, so check the pack flag through a second slot
-    MDF_CUDA(cudaMemcpyAsync(ctx->d_err + 1, ctx->d_err, sizeof(int), cudaMemcpyDeviceToDevice, ctx->stream));
-    MDF_TRY(run_path(m, &b, 0.f, 0, 4, false));
-    MDF_CUDA(cudaMemcpyAsync(ctx->h_err + 1, ctx->d_err + 1, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-    MDF_TRY(fetch_scores(m, &b, scores));
-    if (ctx->h_err[1] != 0) {
-        set_error("forward_pass: contact map holds values other than 0/1");
-        return MDF_EINVAL;
-    }
-    return MDF_OK;
+    MDF_TRY(run_cmap(ctx, b, thr2, gen));
+    if (!dense_off) return MDF_OK;
+    int64_t *doff;
+    MDF_TRY(ctx->alloc_n(dense, dense_total + 1));
+    MDF_TRY(ctx->alloc_n(&doff, (size_t)b->n + 1));
+    MDF_CUDA(cudaMemcpyAsync(doff, dense_off, (size_t)(b->n + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
+    return launch_unpack_dense(ctx, b->nwork, b->d_work, b->d_seq_off, b->d_packed, b->d_packed_off, *dense, doff);
 }
 
 extern "C" int mdf_cmap_build_transfer(mdf_ctx *ctx, int n, const float *coords, const int64_t *coord_off,
@@ -1291,53 +1309,30 @@ extern "C" int mdf_cmap_build_transfer(mdf_ctx *ctx, int n, const float *coords,
     MDF_REQUIRE((packed_out != nullptr) != (dense_out != nullptr), "mdf_cmap_build_transfer: pass exactly one of packed_out / dense_out");
     MDF_REQUIRE(!dense_out || dense_off, "mdf_cmap_build_transfer: dense_off missing");
     MDF_CUDA(cudaSetDevice(ctx->device));
+    // both output layouts must be the canonical ones
+    int64_t packed_words = 0, dense_total = 0;
+    for (int p = 0; p <= n; ++p) {
+        MDF_REQUIRE(!dense_out || p == n || dense_off[p] == dense_total, "mdf_cmap_build_transfer: dense_off[%d] is not canonical", p);
+        MDF_REQUIRE(!packed_off || packed_off[p] == packed_words, "mdf_cmap_build_transfer: packed_off[%d] is not canonical", p);
+        const int64_t L = p < n ? seq_off[p + 1] - seq_off[p] : 0;
+        packed_words += L * mdf_packed_row_words((int)L);
+        dense_total += dense_out ? L * L : 0;      // the arena room the dense output needs
+    }
+    mdf_job *sl = nullptr, *job = nullptr;
+    MDF_TRY(slot_acquire(ctx, &sl, true));
     ArenaScope scope(ctx);
-    mdf_batch b;
-    const int64_t T = seq_off[n];
-    // sequences themselves are not needed for the maps: upload a dummy residue buffer
-    std::vector<char> dummy((size_t)T, 'A');
-    size_t dense_total = 0;
-    if (dense_out) {
-        for (int p = 0; p < n; ++p) {
-            const int64_t L = seq_off[p + 1] - seq_off[p];
-            MDF_REQUIRE(dense_off[p] == (int64_t)dense_total, "mdf_cmap_build_transfer: dense_off[%d] is not canonical", p);
-            dense_total += (size_t)(L * L);
-        }
-    }
-    MDF_TRY(batch_build(ctx, &b, false, {.n = n, .seq = dummy.data(), .seq_off = seq_off, .coords = coords, .coord_off = coord_off,
-                                         .q_aln = q_aln, .t_aln = t_aln, .aln_off = aln_off, .G = 1, .C = 1,
-                                         .extra_reserve = dense_total * 4 + (size_t)(n + 1) * 8 + 8192}));
-    if (packed_off)
-        for (int p = 0; p <= n; ++p)
-            if (packed_off[p] != b.h_packed_off[p]) {
-                if (ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);
-                set_error("mdf_cmap_build_transfer: packed_off[%d] is not canonical", p);
-                return MDF_EINVAL;
-            }
-    MDF_CUDA(cudaMemsetAsync(ctx->d_err, 0, sizeof(int), ctx->stream));
-    {
-        const int rc = run_cmap(ctx, &b, thr2, gen);
-        if (rc != MDF_OK) { if (ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream); return rc; }
-    }
-    if (packed_out) {
-        if (b.h_packed_off[n])
-            MDF_CUDA(cudaMemcpyAsync(packed_out, b.d_packed, (size_t)b.h_packed_off[n] * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    } else {
-        int32_t *dd; int64_t *doff;
-        MDF_TRY(ctx->alloc_n(&dd, dense_total + 1));
-        MDF_TRY(ctx->alloc_n(&doff, (size_t)n + 1));
-        MDF_CUDA(cudaMemcpyAsync(doff, dense_off, (size_t)(n + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
-        MDF_TRY(launch_unpack_dense(ctx, b.nwork, b.d_work, b.d_seq_off, b.d_packed, b.d_packed_off, dd, doff));
-        if (dense_total)
-            MDF_CUDA(cudaMemcpyAsync(dense_out, dd, dense_total * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    }
-    MDF_CUDA(cudaMemcpyAsync(ctx->h_err, ctx->d_err, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-    MDF_CUDA(cudaStreamSynchronize(ctx->stream));
-    return ctx->check_device_error("mdf_cmap_build_transfer");
+    mdf_batch *b = sl->batch;
+    int32_t *dd = nullptr;
+    int rc = batch_build(ctx, b, {.n = n, .seq_off = seq_off, .coords = coords, .coord_off = coord_off, .q_aln = q_aln, .t_aln = t_aln,
+                                  .aln_off = aln_off, .maps_only = true, .extra_reserve = (size_t)dense_total * 4 + (size_t)(n + 1) * 8 + 8192}, sl);
+    if (rc == MDF_OK) rc = cmap_maps(ctx, b, thr2, gen, dense_out ? dense_off : nullptr, (size_t)dense_total, &dd);
+    MDF_TRY(job_finish(sl, rc, n, {packed_out ? ResultCopy{packed_out, b->d_packed, (size_t)packed_words * 4}
+                                              : ResultCopy{dense_out, dd, (size_t)dense_total * 4}}, &job));
+    return job_wait(sl, "mdf_cmap_build_transfer");
 }
 
-// n alignments as arrays of per-alignment pointers: count the query lengths, pack into pinned staging (host threads), then the flat
-// entry point above.  packed_out == nullptr: offsets only.
+// n alignments as arrays of per-alignment pointers: count the query lengths, pack into the synchronous slot's pinned block (host
+// threads), then the flat entry point above.  packed_out == nullptr: offsets only.
 extern "C" int mdf_cmap_build_transfer_ragged(mdf_ctx *ctx, int n, const float *const *coords, const int *coord_rows,
                                               const char *const *q_aln, const char *const *t_aln, const int *aln_len, float thr2, int gen,
                                               uint32_t *packed_out, size_t packed_capacity_words, int64_t *packed_off_out,
@@ -1370,10 +1365,11 @@ extern "C" int mdf_cmap_build_transfer_ragged(mdf_ctx *ctx, int n, const float *
         MDF_REQUIRE(coord_rows[p] >= 0 && (coords[p] || coord_rows[p] == 0), "mdf_cmap_build_transfer_ragged: alignment %d has no coordinates", p);
         MDF_REQUIRE(t_aln[p] || aln_len[p] == 0, "mdf_cmap_build_transfer_ragged: alignment %d has no target string", p);
     }
+    mdf_job *sl = &ctx->slots[2];       // idle between synchronous calls: its pinned block takes the inputs of the flat call below
     RaggedPack pk(n);
     const int R = pk.column(coord_rows, 12, coords), Q = pk.column(aln_len, 1, q_aln), T = pk.column(aln_len, 1, t_aln);
-    MDF_TRY(pinned_block(ctx->rag_pin, ctx->rag_pin_bytes, pk.place(nullptr), ""));
-    pk.place(ctx->rag_pin);
+    MDF_TRY(pinned_block(sl->pin, sl->pin_bytes, pk.place(nullptr), ""));
+    pk.place(sl->pin);
     pk.pack(nt);
     return mdf_cmap_build_transfer(ctx, n, (const float *)pk.at(R), pk.off(R), pk.at(Q), pk.at(T), pk.off(Q), seq_off_out, thr2, gen,
                                    packed_out, packed_off_out, nullptr, nullptr);

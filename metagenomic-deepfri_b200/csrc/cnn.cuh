@@ -1,5 +1,5 @@
 // Sequence-only DeepCNN branch (cnn_tc.cu): the model and the device view of one batch, shared by the resident form
-// (mdf_cnn_upload / mdf_cnn_run) and the asynchronous job (mdf_cnn_submit_ragged, api.cu).
+// (mdf_cnn_upload / mdf_cnn_run) and the jobs (mdf_cnn_submit_ragged, mdf_cnn_forward, api.cu).
 #pragma once
 #include "mdf_common.cuh"
 
@@ -36,6 +36,8 @@ struct mdf_cnn_model {
 
 namespace mdf {
 
+// Checks n sequences at CSR offsets seq_off (the messages name mdf_cnn_upload), sizes v (n, T, n_tiles) and writes their tiles.
+int cnn_plan(int n, const char *seq, const int64_t *seq_off, CnnBatch &v, std::vector<int4> &tiles);
 // Tiles of n sequences (offsets seq_off); with `tiles` != nullptr also writes the table.  Returns the tile count.
 int cnn_tiles(int n, const int64_t *seq_off, int4 *tiles);
 // Lays v's device buffers out from `base` for v.n, v.T, v.n_tiles (base == nullptr: only measures); returns the block's bytes.

@@ -504,23 +504,33 @@ extern "C" int mdf_cnn_model_create(mdf_ctx *ctx, const mdf_cnn_desc *d, mdf_cnn
     return MDF_OK;
 }
 
-extern "C" int mdf_cnn_upload(mdf_cnn_model *m, int n, const char *seq, const int64_t *seq_off)
+int mdf::cnn_plan(int n, const char *seq, const int64_t *seq_off, CnnBatch &v, std::vector<int4> &tiles)
 {
-    MDF_REQUIRE(m && n >= 0 && (n == 0 || (seq && seq_off)), "mdf_cnn_upload: bad arguments");
-    mdf_ctx *ctx = m->ctx;
-    MDF_CUDA(cudaSetDevice(ctx->device));
-    MDF_CUDA(cudaStreamSynchronize(ctx->stream));
-    m->batch = CnnBatch();
+    MDF_REQUIRE(n >= 0 && (n == 0 || (seq && seq_off)), "mdf_cnn_upload: bad arguments");
+    v = CnnBatch();
     if (n == 0) return MDF_OK;
     MDF_REQUIRE(seq_off[0] == 0, "mdf_cnn_upload: seq_off[0] must be 0");
     const int64_t T = seq_off[n];
     MDF_REQUIRE(T < (int64_t)1 << 31, "mdf_cnn_upload: more than 2^31 residues in one batch");
     for (int p = 0; p < n; ++p)          // ReduceMax over an empty residue axis is an error in the reference graph as well
         MDF_REQUIRE(seq_off[p + 1] - seq_off[p] >= 1, "mdf_cnn_upload: sequence %d is empty (the max-pool over residues needs at least one)", p);
-    std::vector<int4> tiles(cnn_tiles(n, seq_off, nullptr));
+    v.n = n; v.T = T; v.n_tiles = cnn_tiles(n, seq_off, nullptr);
+    tiles.resize((size_t)v.n_tiles);
     cnn_tiles(n, seq_off, tiles.data());
+    return MDF_OK;
+}
+
+extern "C" int mdf_cnn_upload(mdf_cnn_model *m, int n, const char *seq, const int64_t *seq_off)
+{
+    MDF_REQUIRE(m, "mdf_cnn_upload: bad arguments");
+    mdf_ctx *ctx = m->ctx;
+    MDF_CUDA(cudaSetDevice(ctx->device));
+    MDF_CUDA(cudaStreamSynchronize(ctx->stream));
+    m->batch = CnnBatch();
     CnnBatch v;
-    v.n = n; v.T = T; v.n_tiles = (int)tiles.size();
+    std::vector<int4> tiles;
+    MDF_TRY(cnn_plan(n, seq, seq_off, v, tiles));
+    if (n == 0) return MDF_OK;
     const size_t need = cnn_carve(m, v, nullptr);
     if (need > m->block_bytes) {            // the resident block only grows: back-to-back batches reuse it
         cnn_free_batch(m);
@@ -531,7 +541,7 @@ extern "C" int mdf_cnn_upload(mdf_cnn_model *m, int n, const char *seq, const in
     }
     cnn_carve(m, v, static_cast<char *>(m->block));
     m->batch = v;
-    MDF_CUDA(cudaMemcpyAsync(v.d_seq, seq, (size_t)T, cudaMemcpyHostToDevice, ctx->stream));
+    MDF_CUDA(cudaMemcpyAsync(v.d_seq, seq, (size_t)v.T, cudaMemcpyHostToDevice, ctx->stream));
     MDF_CUDA(cudaMemcpyAsync(v.d_tile_info, tiles.data(), tiles.size() * sizeof(int4), cudaMemcpyHostToDevice, ctx->stream));
     MDF_CUDA(cudaStreamSynchronize(ctx->stream));      // `tiles` is a local
     return MDF_OK;
@@ -557,13 +567,5 @@ extern "C" int mdf_cnn_fetch(mdf_cnn_model *m, float *scores, float *pooled)
         MDF_CUDA(cudaMemcpyAsync(pooled, v.d_pooled, (size_t)v.n * m->Ctot * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     MDF_CUDA(cudaMemcpyAsync(ctx->h_err, ctx->d_err, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
     MDF_CUDA(cudaStreamSynchronize(ctx->stream));
-    return ctx->check_device_error("cnn forward");
-}
-
-extern "C" int mdf_cnn_forward(mdf_cnn_model *m, int n, const char *seq, const int64_t *seq_off, float *scores)
-{
-    MDF_REQUIRE(m && scores, "mdf_cnn_forward: bad arguments");
-    MDF_TRY(mdf_cnn_upload(m, n, seq, seq_off));
-    MDF_TRY(mdf_cnn_run(m));
-    return mdf_cnn_fetch(m, scores, nullptr);
+    return device_error("cnn forward", *ctx->h_err);
 }

@@ -31,8 +31,7 @@ struct mdf_batch {
     int nwork = 0;          // 32-row blocks over all proteins
     bool has_structure = false;
     bool copy_pending = false;   // structure inputs are still in flight on ctx->copy_stream (wait for ctx->copy_done before reading them)
-    bool owns_memory = false;
-    mdf_job *slot = nullptr;     // transient batch of an asynchronous job: its metadata is staged through the slot's pinned memory
+    mdf_job *slot = nullptr;     // the job slot whose memory holds this batch; nullptr: a resident batch with its own cudaMalloc block
     void *block = nullptr;  // one allocation holding everything below
     void *out_block = nullptr;  // pooled + scores of persistent batches (sized by the model head)
     int out_G = 0, out_C = 0;

@@ -13,6 +13,7 @@
 namespace mdf {
 
 void set_error(const char *fmt, ...);
+int device_error(const char *where, int code);   // MDF_DERR_* code -> MDF_EINVAL and "`where`: <text>"; 0 -> MDF_OK
 
 #define MDF_CUDA(call)                                                                         \
     do {                                                                                       \
@@ -57,20 +58,20 @@ struct Carver {   // sub-allocates one block; first pass (base == nullptr) only 
 
 }  // namespace mdf
 
-// One of the two job slots of a context (mdf_path_submit* / mdf_path_wait): the device block that holds a transient batch's inputs,
-// contact maps and scores, and the pinned host block its inputs are packed into.  While job k computes out of slot k & 1, job
-// k + 1 is packed and copied into the other slot; the engine workspace (arena) is shared in stream order.
+// One of the three job slots of a context: the device block that holds a transient batch's inputs, contact maps and scores, and
+// the pinned host block its inputs are packed into.  Slots 0 and 1 are the ring of mdf_path_submit*: while job k computes out of
+// slot k & 1, job k + 1 is packed and copied into the other; slot 2 serves the synchronous calls.  The arena is shared in stream order.
 struct mdf_batch;
 struct mdf_model;
 struct mdf_job {
     struct mdf_ctx *ctx = nullptr;
     char *dev = nullptr;  size_t dev_bytes = 0;     // cudaMalloc
     char *pin = nullptr;  size_t pin_bytes = 0;     // cudaHostAlloc
-    int *h_err = nullptr;                           // pinned [2]: device error flag of this job
+    int *d_errs = nullptr;      // device [2]: [0] first device error of the job's kernels, [1] map check of mdf_gcn_forward_dense
+    int *h_err = nullptr;       // pinned [2]: their copies (d_errs keeps them as the next job resets ctx->d_err)
     cudaEvent_t done = nullptr;                     // recorded after the scores have reached the host
     bool busy = false;                              // submitted, not yet waited for
     mdf_batch *batch = nullptr;
-    int rc = 0;                                     // deferred submit status
     // pinned staging for the small per-batch metadata (work lists, offsets, tile tables): copied from here the H2D copies are
     // truly asynchronous, so a submit never blocks on the previous job and the GPU does not idle between jobs
     char *meta = nullptr; size_t meta_bytes = 0, meta_top = 0;
@@ -115,14 +116,13 @@ struct mdf_ctx {
     // device-side error flag (invalid residue, non-0/1 cmap, Lq mismatch ...)
     int *d_err = nullptr;
     int *h_err = nullptr;  // pinned
-    // second stream for the structure inputs of mdf_path_forward: their host->device copy runs beside the LSTM language model,
-    // which only needs the sequences; the contact-map stage waits for `copy_done`
+    // second stream for the structure inputs of jobs: their host->device copy runs beside the LSTM language model, which only
+    // needs the sequences; the contact-map stage waits for `copy_done`
     cudaStream_t copy_stream = nullptr;
-    char *rag_pin = nullptr; size_t rag_pin_bytes = 0;   // pinned staging of the synchronous ragged entry points (grow-only)
     cudaStream_t d2h_stream = nullptr;       // scores of asynchronous jobs leave on their own stream: the next job's kernels start at once
-    cudaEvent_t path_done[2] = {nullptr, nullptr};   // per job slot: kernels of the job finished (compute stream)
+    cudaEvent_t path_done[3] = {nullptr, nullptr, nullptr};   // per job slot: kernels of the job finished (compute stream)
     cudaEvent_t copy_done = nullptr;
-    mdf_job slots[2];
+    mdf_job slots[3];                        // 0, 1: the ring of asynchronous jobs; 2: the synchronous calls
     int next_slot = 0;
     int host_threads = 4;     // packing threads of mdf_path_submit_ragged (MDF_HOST_THREADS)
 
@@ -136,7 +136,6 @@ struct mdf_ctx {
     template <typename T>
     int alloc_n(T **out, size_t count) { return alloc((void **)out, count * sizeof(T)); }
     int reserve(size_t bytes);            // make sure `bytes` are available above arena_top
-    int check_device_error(const char *where);
 };
 
 struct ArenaScope {

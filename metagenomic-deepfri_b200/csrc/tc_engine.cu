@@ -599,7 +599,7 @@ static int build_meta(mdf_ctx *ctx, mdf_batch *b, TcBatchMeta &meta, bool want_e
     const size_t bytes = align_up((size_t)Tp * 4, 256) + align_up(tile_info.size() * 16, 256) +
                          align_up(exp_tiles.size() * 16 + 16, 256) + align_up((size_t)(n + 1) * 8, 256);
     char *base = nullptr;
-    if (b->owns_memory) {
+    if (!b->slot) {
         MDF_CUDA(cudaMalloc((void **)&base, bytes));
         meta.persistent = true;
     } else {
@@ -611,7 +611,7 @@ static int build_meta(mdf_ctx *ctx, mdf_batch *b, TcBatchMeta &meta, bool want_e
     meta.exp_tiles = (int4 *)base; base += align_up(exp_tiles.size() * 16 + 16, 256);
     meta.seg_off = (int64_t *)base;
     cudaStream_t s = ctx->stream;
-    // asynchronous jobs stage these tables through the slot's pinned memory: the copies then never block the submitting thread
+    // jobs stage these tables through the slot's pinned memory: the copies then never block the submitting thread
     bool staged = b->slot != nullptr;
     auto src_of = [&](const void *p, size_t bytes) { return mdf_job::src_of(b->slot, p, bytes, &staged); };
     // the [Tp] row map (24 MB for a 16k-protein batch) is filled on the device; only the per-tile / per-protein arrays travel
@@ -680,7 +680,7 @@ int tc_forward(mdf_model *m, mdf_batch *b, int upto, const std::function<int()> 
     const bool want_compact = tm->compact && tm->adj_expand && tm->adj_sparse && tm->pool_fused;
     TcBatchMeta local_meta;
     TcBatchMeta *meta = &local_meta;
-    if (b->owns_memory) {
+    if (!b->slot) {
         if (!b->tc_meta) {
             TcBatchMeta *pm = new TcBatchMeta();
             int r = build_meta(ctx, b, *pm, !tm->adj_expand, want_compact);
@@ -717,7 +717,7 @@ int tc_forward(mdf_model *m, mdf_batch *b, int upto, const std::function<int()> 
     // ---- LSTM language model.  A persistent batch keeps the last layer's output image: another head with the same LM
     // (the MF / BP / CC / EC models share it) skips the recurrence altogether.
     bool lm_cached = false;
-    if (b->owns_memory && b->reuse && !ctx->debug_taps) {
+    if (!b->slot && b->reuse && !ctx->debug_taps) {
         const size_t need = (size_t)Tp * m->H * sizeof(__half);
         if (b->lm_cache && b->lm_cache_bytes == need && b->lm_hash == tm->lm_hash) {
             lm_cached = true;
@@ -737,7 +737,7 @@ int tc_forward(mdf_model *m, mdf_batch *b, int upto, const std::function<int()> 
                                   b->d_seq_off, row_off, ctx->debug_taps ? Hlimg[0] : nullptr, Hlimg[1], scratch, b->h_order.data(),
                                   b->h_seq_off.data()));
     }
-    if (b->owns_memory && b->reuse && !ctx->debug_taps) b->lm_hash = tm->lm_hash;
+    if (!b->slot && b->reuse && !ctx->debug_taps) b->lm_hash = tm->lm_hash;
     if (ctx->debug_taps) {                                // fp32 copies of the LSTM outputs over packed residues
         for (int l = 0; l < m->n_lstm; ++l) {
             float *tap = nullptr;
